@@ -10,7 +10,9 @@ Workload: BASELINE.json configs[2] -- 2^20 envs sharded over 8 GPUs, i.e. 131072
 weak scaling (per-GPU work fixed), random initial orbits, i.i.d. uniform actions, auto-reset so the
 batch stays in steady state.  Side measurements in the same line: "batch4096" (configs[1]: the split organisation of the
 kernel, with the one-thread organisation beside it), "stress" (configs[4]: J2 + four wheels + dumping, FP64 and mixed precision) and "opnav" (configs[3]).
-`e2e` goes through bskenv_step_host with host buffers (zero-copy page-locked memory).  Prints ONE JSON line (rank 0)."""
+`e2e` goes through bskenv_step_host with host buffers (zero-copy page-locked memory).  Prints ONE JSON line (rank 0).
+`--dump-outputs DIR` also writes what the last timed step of the headline returned, so that two builds can be compared on the
+same seeded inputs."""
 import argparse
 import json
 import os
@@ -23,6 +25,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark writes nothing into the tree (it may run from a read-only checkout)
 
 METRIC = "env decision-steps/sec"
 UNIT = "env-steps/s"
@@ -50,7 +53,16 @@ def parse():
     ap.add_argument("--opnav-envs", type=int, default=113664,
                     help="opNav batch: two resident sets of the step kernel's three-block organisation (148 SMs x 3 blocks x 128 "
                          "threads = 56832 envs each) = three sets of its two-block organisation")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step of the headline returned (obs, reward, done and "
+                         "the info arrays) as DIR/<name>.npy, float64, at most 64 MB (a fixed sample of envs beyond that; "
+                         "env_index.npy names them); rank 0's envs under --gpus N > 1")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "native" or args.workload != "leo"):
+        ap.error("--dump-outputs applies to the headline (--impl native --workload leo)")
+    return args
 
 
 class ClockSampler:
@@ -80,6 +92,8 @@ class ClockSampler:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         time.sleep(0.15)
         self.proc.terminate()
+        self.proc.wait()              # reap it: no defunct nvidia-smi left behind
+        self.thread.join()
         sm, mx, pw, reasons = [], [], [], set()
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
         rows = [r for t, r in self.rows if t0 - 0.05 <= t <= t1 + 0.15] or [r for _, r in self.rows]
@@ -176,7 +190,8 @@ def workload_name(envs_per_gpu):
 
 
 def time_device_steps(env, actions_dev, steps, warmup, torch, dist, world):
-    """K launches on the current stream between CUDA events; per-launch events give the kernel duration."""
+    """K launches on the current stream between CUDA events; per-launch events give the kernel duration.  Also returns what
+    the last timed env.step returned (the env's own buffers: valid until its next step)."""
     for t in range(warmup):
         env.step(actions_dev[t % len(actions_dev)])
     torch.cuda.synchronize()
@@ -186,14 +201,39 @@ def time_device_steps(env, actions_dev, steps, warmup, torch, dist, world):
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(steps + 1)]
     ev[0].record()
     for t in range(steps):
-        env.step(actions_dev[(warmup + t) % len(actions_dev)])
+        last = env.step(actions_dev[(warmup + t) % len(actions_dev)])
         ev[t + 1].record()
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
     total_ms = ev[0].elapsed_time(ev[steps])
     per = [ev[t].elapsed_time(ev[t + 1]) for t in range(steps)]
-    return total_ms, per
+    return total_ms, per, last
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def snapshot_outputs(obs, reward, done, info):
+    """Device copies of what one LeoPowerAttVecEnv.step returned, as float64 arrays [N] or [N, 5].  terminal_obs is defined
+    only for the envs that finished in that step (the library leaves the other rows as they were): those rows are zeroed."""
+    fin = done.bool()
+    return {"obs": obs.double().clone(), "reward": reward.double().clone(), "done": done.double(),
+            "done_reason": info["done_reason"].double(), "terminal_obs": info["terminal_obs"].double() * fin[:, None],
+            "episode_r": info["episode_r"].double().clone(), "episode_l": info["episode_l"].double()}
+
+
+def dump_outputs(outdir, arrays):
+    """Writes each array as outdir/<name>.npy.  Beyond DUMP_LIMIT_BYTES in all, a fixed seeded sample of envs (rows) is
+    written; env_index.npy holds the env indices of the rows either way."""
+    n = len(arrays["obs"])
+    per_env = 8 * (1 + sum(int(np.prod(a.shape[1:])) for a in arrays.values()))
+    m = min(n, DUMP_LIMIT_BYTES // per_env)
+    idx = np.arange(n) if m == n else np.sort(np.random.RandomState(0).choice(n, m, replace=False))
+    os.makedirs(outdir, exist_ok=True)
+    np.save(os.path.join(outdir, "env_index.npy"), idx.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, f"{name}.npy"), a.cpu().numpy()[idx])
 
 
 def main():
@@ -246,7 +286,8 @@ def main():
     sampler = ClockSampler(local_rank) if rank == 0 else None
     l0 = env.launch_count()
     t_mark0 = time.perf_counter()
-    total_ms, per_ms = time_device_steps(env, actions_dev, K, W, torch, dist, world)
+    total_ms, per_ms, last = time_device_steps(env, actions_dev, K, W, torch, dist, world)
+    dumped = snapshot_outputs(*last) if args.dump_outputs and rank == 0 else None   # before the steps below overwrite them
     # ---- end to end through the host-buffer C-ABI entry point (bskenv_step_host) ----
     for t in range(min(W, 3)):
         act_pinned[:] = actions_host[t]
@@ -331,6 +372,8 @@ def main():
         else:
             line["cpu_baseline"] = None
         print(json.dumps(line), flush=True)
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped)
     env.close()
     if world > 1:
         dist.barrier()
@@ -349,7 +392,7 @@ def side_batch(n, torch, dev, peak_tf):
     for org in ("auto", "thread"):
         env = LeoPowerAttVecEnv(n, device=dev.index, seed=5, auto_reset=True, organisation=org)
         env.reset()
-        total_ms, per = time_device_steps(env, acts, 10, 3, torch, None, 1)
+        total_ms, per, _ = time_device_steps(env, acts, 10, 3, torch, None, 1)
         flops, name = env.flops_per_step(), env.kernel_name()
         ms = total_ms / 10
         tf = flops * n / (ms * 1e-3) / 1e12
@@ -387,7 +430,7 @@ def side_stress(n, torch, dev, peak_tf, steps=5, warmup=3):
     for prec, key in ((0, "fp64"), (1, "mixed")):
         env = LeoPowerAttVecEnv(n, device=dev.index, seed=17, use_j2=1, rw_set=1, precision=prec)
         env.reset()
-        total_ms, per = time_device_steps(env, acts, steps, warmup, torch, None, 1)
+        total_ms, per, _ = time_device_steps(env, acts, steps, warmup, torch, None, 1)
         ms = float(np.mean(per))
         flops = env.flops_per_step()
         tf = flops * n / (ms * 1e-3) / 1e12
@@ -403,7 +446,7 @@ def side_stress(n, torch, dev, peak_tf, steps=5, warmup=3):
     env = LeoPowerAttVecEnv(n, device=dev.index, seed=17, use_j2=1, rw_set=1, auto_reset=True)
     env.reset()
     acts2 = torch.randint(0, 3, (13, n), dtype=torch.int32, device=dev, generator=g)
-    total_ms, per = time_device_steps(env, acts2, steps, 8, torch, None, 1)
+    total_ms, per, _ = time_device_steps(env, acts2, steps, 8, torch, None, 1)
     ms = float(np.mean(per))
     tf = env.flops_per_step() * n / (ms * 1e-3) / 1e12
     out["fp64_steady_state"] = {"value": n * steps / (total_ms * 1e-3), "unit": UNIT, "ms_per_step": total_ms / steps, "kernel": env.kernel_name(),
@@ -478,7 +521,7 @@ def side_opnav(n, torch, dev, peak_tf, steps=3, warmup=3, cpu_seconds=4.0):
     acts = torch.randint(0, 2, (steps + warmup, n), dtype=torch.int32, device=dev)
     acts_host = acts.cpu().numpy()
     l0 = env.launch_count()
-    total_ms, per = time_device_steps(env, acts, steps, warmup, torch, None, 1)
+    total_ms, per, _ = time_device_steps(env, acts, steps, warmup, torch, None, 1)
     act_pinned, outs = env.host_buffers()             # page-locked, device-mapped: the kernels read / write them in place
     act_pinned[:] = acts_host[0]
     env.step_host(act_pinned, outs)
@@ -519,7 +562,7 @@ def side_opnav(n, torch, dev, peak_tf, steps=3, warmup=3, cpu_seconds=4.0):
         env = OpNavVecEnv(n, device=dev.index, seed=5, auto_reset=True, sample_orbit=1, camera_reenable=1)
         env.reset()
         l0 = env.launch_count()
-        t_ms, per3 = time_device_steps(env, acts, steps, warmup, torch, None, 1)
+        t_ms, per3, _ = time_device_steps(env, acts, steps, warmup, torch, None, 1)
         k3 = (env.launch_count() - l0) // (warmup + steps)
         out["three_kernel_interval"] = {"value": n * steps / (t_ms * 1e-3), "unit": UNIT, "ms_per_step": t_ms / steps, "kernels_per_step": int(k3),
                                         "noise_buffer_bytes": 15 * 8 * 3001 * ((n + 31) // 32 * 32) if k3 == 3 else 0,

@@ -53,22 +53,28 @@ def build(force=False):
 
 def build_fast():
     """The same sources as an optimised host build (-O3 -march=native, contraction allowed): bench.py's second CPU
-    baseline.  -march=native ties the binary to the CPU it was compiled on, so it is built where it runs, into
-    oracle/_fast/ under a name derived from that CPU's model and flags (the GPU box is not this container)."""
+    baseline.  -march=native ties the binary to the CPU it was compiled on, so it is built where it runs.  It goes to a
+    per-user temporary directory, not into the tree (the benchmark may run from a read-only checkout), under a name
+    derived from that CPU's model and flags and from the sources."""
     import hashlib
+    import tempfile
     try:
         info = open("/proc/cpuinfo").read()
         key = "".join(l for l in info.splitlines()[:40] if l.startswith(("model name", "flags")))
     except OSError:
         key = "unknown"
-    tag = hashlib.sha1(key.encode()).hexdigest()[:10]
-    d = os.path.join(_HERE, "_fast")
-    os.makedirs(d, exist_ok=True)
-    so = os.path.join(d, f"libbsk_oracle_fast_{tag}.so")
-    srcs = [os.path.join(_HERE, f) for f in ("bsk_oracle.c", "bsk_oracle.h", "opnav_oracle.c", "opnav_oracle.h")]
-    if not os.path.exists(so) or any(os.path.getmtime(so) < os.path.getmtime(f) for f in srcs):
-        subprocess.check_call(["gcc", "-O3", "-march=native", "-fPIC", "-fopenmp", "-std=c99", "-shared", "-o", so,
+    h = hashlib.sha1(key.encode())
+    for f in ("bsk_oracle.c", "bsk_oracle.h", "opnav_oracle.c", "opnav_oracle.h"):
+        with open(os.path.join(_HERE, f), "rb") as fh:
+            h.update(fh.read())
+    d = os.path.join(tempfile.gettempdir(), f"bskenv_oracle_fast_{os.getuid()}")
+    os.makedirs(d, mode=0o700, exist_ok=True)
+    so = os.path.join(d, f"libbsk_oracle_fast_{h.hexdigest()[:16]}.so")
+    if not os.path.exists(so):
+        tmp = f"{so}.{os.getpid()}.tmp"
+        subprocess.check_call(["gcc", "-O3", "-march=native", "-fPIC", "-fopenmp", "-std=c99", "-shared", "-o", tmp,
                                os.path.join(_HERE, "bsk_oracle.c"), os.path.join(_HERE, "opnav_oracle.c"), "-lm"])
+        os.replace(tmp, so)
     return so
 
 
