@@ -51,7 +51,7 @@ EXPORTS = ["bskenv_abi_version", "bskenv_default_config", "bskenv_create", "bske
            "bskenv_state_field", "bskenv_episode_stats", "bskenv_launch_count", "bskenv_fp64_peak",
            "bskenv_flops_per_step", "bskenv_set_ephemeris", "bskenv_set_gravity_degree2", "bskenv_step_info",
            "bskenv_step_host_async", "bskenv_step_host_wait", "bskenv_alloc_host", "bskenv_free_host", "bskenv_kernel_name",
-           "bskenv_set_organisation"]
+           "bskenv_set_organisation", "bskenv_set_param_pool", "bskenv_get_env_params"]
 
 
 def lib_path():
@@ -97,6 +97,8 @@ def lib():
     L.bskenv_kernel_name.restype = C.c_char_p
     L.bskenv_kernel_name.argtypes = [vp]
     L.bskenv_set_organisation.argtypes = [vp, C.c_int]
+    L.bskenv_set_param_pool.argtypes = [vp, C.c_int, vp, C.c_int]
+    L.bskenv_get_env_params.argtypes = [vp, vp, vp, vp]
     L.bskenv_fp64_peak.argtypes = [C.c_int, C.c_double, C.POINTER(C.c_double)]
     L.bskenv_flops_per_step.restype = C.c_double
     L.bskenv_flops_per_step.argtypes = [vp]

@@ -15,6 +15,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/bskenv.h"
@@ -37,6 +38,11 @@
                                 // B200 with one / two / four groups per block: 4096 envs 3.34 -> 2.39 ms, 8192 3.42 -> 2.49, 16384 3.76 -> 3.00
 #endif
 #define LEO_BUS_BYTES_PFIX ((size_t)leo::LEO_NM_PFIX * LEO_BLOCK * sizeof(double))   // ... of the planet-fixed gravity variant
+#ifdef LEO_PENV_GLOBAL
+#define LEO_BUS_BYTES_PENV LEO_BUS_BYTES                                               // ... of the per-env parameter kernel
+#else
+#define LEO_BUS_BYTES_PENV ((size_t)leo::LEO_NM_PENV * LEO_BLOCK * sizeof(double))
+#endif
 
 namespace {
 
@@ -124,11 +130,13 @@ __device__ __forceinline__ int chunk_peek(const int *p)
 
 // What follows the last chunk of a decision interval: results, per-env episode record, in-kernel auto-reset, episode statistics
 // (warp-shuffle reduction, one atomic per warp and statistic).  Called by all 32 lanes of the warp that stepped the group.
+// PA = ParEnv: the auto-reset also assigns the env's pool row for the new episode.
+template <class PA = leo::ParBatch>
 __device__ __forceinline__ void step_finish(const LeoParams &P, double *__restrict__ S, int64_t *__restrict__ I, double *__restrict__ ics,
                                             int64_t stride, int64_t e, bool valid, int lane, leo::StepOut &o, double *__restrict__ obs,
                                             double *__restrict__ reward, uint8_t *__restrict__ done, uint8_t *__restrict__ reason,
                                             double *__restrict__ term_obs, double *__restrict__ stats, double *__restrict__ ep_return,
-                                            int64_t *__restrict__ ep_length)
+                                            int64_t *__restrict__ ep_length, const LeoPool &pool = LeoPool{})
 {
     double ep_ret = 0., ep_len = 0.;
     if (valid) {
@@ -153,7 +161,9 @@ __device__ __forceinline__ void step_finish(const LeoParams &P, double *__restri
                 double ic[19];
                 leo::sample_ic(P, P.first_env_index + e, ep, ic);
                 for (int k = 0; k < 19; k++) ics[(int64_t)k * stride + e] = ic[k];
-                leo::leo_reset_env(P, S, I, stride, e, ic, o.ob);
+                if (!std::is_same<PA, leo::ParBatch>::value)
+                    leo::pool_assign(pool, S, stride, e, leo::pool_row(pool, P.seed, P.first_env_index + e, ep));
+                leo::leo_reset_env<PA>(P, S, I, stride, e, ic, o.ob);
             }
         }
         for (int k = 0; k < 5; k++) obs[e * 5 + k] = o.ob[k];
@@ -236,6 +246,64 @@ leo_step_kernel(const __grid_constant__ LeoParams P, const __grid_constant__ Leo
     }
 }
 
+// The same organisation with per-env spacecraft parameters (bskenv_set_param_pool): leo_step_env<..., ParEnv> reads each
+// env's derived values from the parameter block behind its state (stage-rate values through its bus column, which is
+// LEO_NM_PENV fields long), and the auto-reset assigns the pool row of the new episode.  Built for the reference
+// configuration only (three wheels, DIAG, FP64).  A kernel of its own rather than a template argument of leo_step_kernel,
+// so that the batch-global kernels stay exactly as they are.
+template <int NRW, int J2, bool DIAG, int MINB>
+__global__ void LEO_STEP_BOUNDS(MINB)
+leo_step_penv_kernel(const __grid_constant__ LeoParams P, const LeoPool pool, double *__restrict__ S, int64_t *__restrict__ I,
+                     double *__restrict__ ics, int64_t stride, int64_t n, const int32_t *__restrict__ actions,
+                     double *__restrict__ obs, double *__restrict__ reward, uint8_t *__restrict__ done, uint8_t *__restrict__ reason,
+                     double *__restrict__ term_obs, double *__restrict__ stats, const LeoSched sc, double *__restrict__ ep_return,
+                     int64_t *__restrict__ ep_length)
+{
+    static_assert(NRW == 3 && DIAG && J2 != 2, "per-env parameters are built for the reference configuration");
+    extern __shared__ double bus_smem[];          // [LEO_NM_PENV][LEO_BLOCK]
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    leo::MBus bus;
+    bus.p = nullptr;
+    bus.a = (uint32_t)__cvta_generic_to_shared(bus_smem) + threadIdx.x * (uint32_t)sizeof(double);
+    for (bool more = true; more; more = sc.dynamic != 0) {
+        int g, c_first = 0, c_end = sc.n_chunks;
+        if (sc.dynamic) {
+            g = 0;
+            if (lane == 0) g = atomicAdd(&sc.sched[0], 1);
+            g = __shfl_sync(0xffffffffu, g, 0);
+            if (g >= sc.n_groups * sc.n_chunks) break;
+            c_first = g / sc.n_groups; c_end = c_first + 1;
+            g -= c_first * sc.n_groups;
+            if (c_first > 0) {
+                if (lane == 0)
+                    while (chunk_peek(sc.progress + g) < c_first) __nanosleep(200);
+                __syncwarp();
+            }
+        } else {
+            g = blockIdx.x * (LEO_BLOCK / 32) + warp;
+        }
+        const int64_t slot = (int64_t)g * LEO_LANES + lane;
+        const bool valid = lane < LEO_LANES && slot < n;
+        const int64_t e = (valid && sc.perm) ? (int64_t)sc.perm[slot] : slot;
+        leo::StepOut o;
+        o.done = 0; o.reason = 0; o.reward = 0.;
+        for (int c = c_first; c < c_end; c++) {
+            if (valid) leo::leo_step_env<NRW, J2, DIAG, false, leo::ParEnv>(P, S, I, stride, e, bus, actions[e], o, LeoParamsF(), c, sc.n_chunks);
+            if (c + 1 < sc.n_chunks) {
+                if (sc.dynamic) {
+                    __threadfence();
+                    __syncwarp();
+                    if (lane == 0) chunk_publish(sc.progress + g, c + 1);
+                }
+                continue;
+            }
+            step_finish<leo::ParEnv>(P, S, I, ics, stride, e, valid, lane, o, obs, reward, done, reason, term_obs, stats, ep_return,
+                                     ep_length, pool);
+        }
+        __syncwarp();
+    }
+}
+
 // Ragged batches in the split organisation: the lanes of the last group that have no env step a DUPLICATE of the last env
 // (its state copied into the padding columns [n, stride) of the state blocks before every launch, the same action), so that
 // every lane of a group takes the same barriers through the same code; nothing they compute leaves the padding columns.
@@ -295,11 +363,12 @@ leo_split_kernel(const __grid_constant__ LeoParams P, double *__restrict__ S, in
 #endif
 }
 
-// mode 0: explicit ICs (row-major [n][19]); 1: stored ICs (reset_init); 2: device-sampled ICs
+// mode 0: explicit ICs (row-major [n][19]); 1: stored ICs (reset_init); 2: device-sampled ICs.
+// With a parameter pool (pool.n_rows > 0) modes 0 and 2 assign the env's pool row; mode 1 keeps it.
 __global__ void __launch_bounds__(256)
 leo_reset_kernel(const __grid_constant__ LeoParams P, double *__restrict__ S, int64_t *__restrict__ I, double *__restrict__ ics,
                  int64_t stride, int64_t n, int mode, const double *__restrict__ ics_in, const uint8_t *__restrict__ mask,
-                 double *__restrict__ obs)
+                 double *__restrict__ obs, const LeoPool pool)
 {
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n) return;
@@ -316,9 +385,26 @@ leo_reset_kernel(const __grid_constant__ LeoParams P, double *__restrict__ S, in
     }
     for (int k = 0; k < 19; k++) ics[(int64_t)k * stride + e] = ic[k];
     double ob[5];
-    leo::leo_reset_env(P, S, I, stride, e, ic, ob);
+    if (pool.n_rows > 0) {
+        if (mode != 1) leo::pool_assign(pool, S, stride, e, leo::pool_row(pool, P.seed, P.first_env_index + e, I[(int64_t)I_EPISODE * stride + e]));
+        leo::leo_reset_env<leo::ParEnv>(P, S, I, stride, e, ic, ob);
+    } else {
+        leo::leo_reset_env(P, S, I, stride, e, ic, ob);
+    }
     if (obs)
         for (int k = 0; k < 5; k++) obs[e * 5 + k] = ob[k];
+}
+
+// bskenv_get_env_params: the reference values and the pool row of every env (the batch configuration, row -1, when the
+// parameter block is not in use)
+struct ParamRow { double v[BSKENV_PARAM_DIM]; };
+__global__ void gather_params_kernel(const double *__restrict__ S, int64_t stride, int64_t n, int live, const ParamRow batch,
+                                     double *__restrict__ out, int32_t *__restrict__ row)
+{
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    for (int k = 0; k < BSKENV_PARAM_DIM; k++) out[e * BSKENV_PARAM_DIM + k] = live ? S[(int64_t)(LEO_ND + PE_RAW + k) * stride + e] : batch.v[k];
+    if (row) row[e] = live ? (int32_t)S[(int64_t)(LEO_ND + PE_ROW) * stride + e] : -1;
 }
 
 __global__ void gather_ics_kernel(const double *__restrict__ ics, int64_t stride, int64_t n, double *__restrict__ out)
@@ -376,6 +462,8 @@ struct bskenv_handle {
     int64_t launches;
     const char *kernel_name;    // the step-kernel instantiation of the last launch
     int organisation;           // BSKENV_ORG_*: 0 auto, 1 one thread per env, 2 two warps per env group (small batches)
+    LeoPool pool;               // loaded parameter pool (n_rows = 0: none); rows in device memory
+    int s_fields;               // double fields allocated per env in S: LEO_ND, or LEO_ND + LEO_NPD once a pool was loaded
     std::string err;
 };
 
@@ -420,7 +508,8 @@ static int launch_step(bskenv_handle *h, const int32_t *act, double *obs, double
         CU_TRY(h, cudaMemsetAsync(h->sched, 0, sizeof(int) * (size_t)(4 + groups), st));    // queue head + chunk progress per group
     }
     // two warps per env group: whole groups only, the two configurations the small-batch kernels are built for
-    const bool split_cfg = !h->P.grav_pfix && !h->P.mixed && ((h->P.nrw == 3 && !h->cfg.use_j2 && h->P.diag) || (h->P.nrw == 4 && h->cfg.use_j2));
+    const bool penv = h->pool.n_rows > 0;                      // per-env parameters: one thread per env at every batch size
+    const bool split_cfg = !penv && !h->P.grav_pfix && !h->P.mixed && ((h->P.nrw == 3 && !h->cfg.use_j2 && h->P.diag) || (h->P.nrw == 4 && h->cfg.use_j2));
     const bool split_fit = split_cfg && groups <= (int64_t)h->sm_count * LEO_SPLIT_MAX_G;
     if (h->organisation == BSKENV_ORG_SPLIT && !split_fit) {
         h->err = "bskenv_step: the split organisation takes at most 128 * SM-count envs, FP64, and the reference or the stress configuration";
@@ -476,8 +565,20 @@ static int launch_step(bskenv_handle *h, const int32_t *act, double *obs, double
                                                                                  rew, done, reason, term_obs, h->stats, sc, ep_return, ep_length); \
     } while (0)
 #define LEO_LAUNCH(NRW, J2, DIAG, F32) LEO_LAUNCH_B(NRW, J2, DIAG, F32, LEO_MIN_BLOCKS)
+#define LEO_LAUNCH_PENV(J2)                                                                                    \
+    do {                                                                                                       \
+        static bool attr_set[64] = {false};                                                                    \
+        if (!attr_set[h->device & 63]) {                                                                       \
+            CU_TRY(h, cudaFuncSetAttribute(leo_step_penv_kernel<3, J2, true, LEO_MIN_BLOCKS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LEO_BUS_BYTES_PENV)); \
+            attr_set[h->device & 63] = true;                                                                   \
+        }                                                                                                      \
+        h->kernel_name = "leo_step_penv_kernel<3," #J2 ",true," LEO_STR(LEO_MIN_BLOCKS) ">";                    \
+        leo_step_penv_kernel<3, J2, true, LEO_MIN_BLOCKS><<<grid, LEO_BLOCK, LEO_BUS_BYTES_PENV, st>>>(h->P, h->pool, h->S, h->I, h->ics, \
+            h->stride, h->n, act, obs, rew, done, reason, term_obs, h->stats, sc, ep_return, ep_length);        \
+    } while (0)
+    if (penv) { if (h->cfg.use_j2) LEO_LAUNCH_PENV(1); else LEO_LAUNCH_PENV(0); }    // (bskenv_set_param_pool checks the configuration)
     // small-batch organisation: built for the reference configuration and for the stress configuration
-    if (small && !h->P.grav_pfix && !h->P.mixed && h->P.nrw == 3 && !h->cfg.use_j2 && h->P.diag) LEO_LAUNCH_B(3, 0, true, false, 1);
+    else if (small &&!h->P.grav_pfix && !h->P.mixed && h->P.nrw == 3 && !h->cfg.use_j2 && h->P.diag) LEO_LAUNCH_B(3, 0, true, false, 1);
     else if (small && !h->P.grav_pfix && !h->P.mixed && h->P.nrw == 4 && h->cfg.use_j2) LEO_LAUNCH_B(4, 1, false, false, 1);
     else
     if (h->P.grav_pfix) {     // SURVEY 8(f)-4: degree-2 field in the planet-fixed frame (general EOM path)
@@ -494,6 +595,7 @@ static int launch_step(bskenv_handle *h, const int32_t *act, double *obs, double
     else                    { if (h->P.diag) LEO_LAUNCH(3, 0, true, false); else LEO_LAUNCH(3, 0, false, false); }
 #undef LEO_LAUNCH
 #undef LEO_LAUNCH_B
+#undef LEO_LAUNCH_PENV
     CU_TRY(h, cudaGetLastError());
     h->launches++;
     if (st != h->own_stream || !st) CU_TRY(h, note_launch(h, st));
@@ -514,6 +616,7 @@ int bskenv_set_organisation(bskenv_handle *h, int organisation)
 {
     if (!h) return BSKENV_EINVAL;
     if (organisation < BSKENV_ORG_AUTO || organisation > BSKENV_ORG_THREAD_INDEX) { h->err = "bskenv_set_organisation: unknown organisation"; return BSKENV_EINVAL; }
+    if (organisation == BSKENV_ORG_SPLIT && h->pool.n_rows > 0) { h->err = "bskenv_set_organisation: the split organisation has no per-env parameters (a parameter pool is loaded)"; return BSKENV_EINVAL; }
     h->organisation = organisation;
     return BSKENV_OK;
 }
@@ -541,6 +644,7 @@ int bskenv_create(const bskenv_config *cfg, int device, int64_t n_envs, int64_t 
     h->device = device; h->n = n_envs; h->stride = (n_envs + 31) / 32 * 32; h->launches = 0; h->kernel_name = nullptr; h->organisation = BSKENV_ORG_AUTO;
     h->S = h->ics = h->stats = nullptr; h->I = nullptr; h->sched = nullptr; h->perm = nullptr; h->bucket = nullptr;
     h->d_eph[0] = h->d_eph[1] = nullptr;
+    h->pool.rows = nullptr; h->pool.n_rows = 0; h->pool.assign = 0; h->s_fields = LEO_ND;
     for (int k = 0; k < 8; k++) { h->h_stage[k] = nullptr; h->pend_user[k] = nullptr; h->pend_bytes[k] = 0; }
     h->host_pending = 0; h->own_stream = nullptr; h->ev_last = nullptr; h->ev_valid = 0;
     cudaError_t e = cudaSetDevice(device);
@@ -571,7 +675,7 @@ int bskenv_destroy(bskenv_handle *h)
     if (!h) return BSKENV_OK;
     cudaSetDevice(h->device);
     cudaFree(h->S); cudaFree(h->I); cudaFree(h->ics); cudaFree(h->stats); cudaFree(h->sched); cudaFree(h->perm); cudaFree(h->bucket);
-    cudaFree(h->d_eph[0]); cudaFree(h->d_eph[1]);
+    cudaFree(h->d_eph[0]); cudaFree(h->d_eph[1]); cudaFree((void *)h->pool.rows);
     if (h->own_stream) { cudaStreamSynchronize(h->own_stream); cudaStreamDestroy(h->own_stream); }
     for (int k = 0; k < 8; k++) cudaFreeHost(h->h_stage[k]);
     if (h->ev_last) cudaEventDestroy(h->ev_last);
@@ -584,6 +688,7 @@ int bskenv_set_gravity_degree2(bskenv_handle *h, int enable, const double *cbar)
     if (!h) return BSKENV_EINVAL;
     if (!enable) { h->P.grav_pfix = 0; return BSKENV_OK; }
     if (h->P.mixed) { h->err = "bskenv_set_gravity_degree2: not built for precision = 1"; return BSKENV_EINVAL; }
+    if (h->pool.n_rows > 0) { h->err = "bskenv_set_gravity_degree2: not built with per-env parameters (a parameter pool is loaded)"; return BSKENV_EINVAL; }
     leo_host::set_degree2(h->P, cbar);
     return BSKENV_OK;
 }
@@ -611,13 +716,73 @@ int bskenv_set_ephemeris(bskenv_handle *h, int kind, double t0, double seg_len, 
     return BSKENV_OK;
 }
 
+int bskenv_set_param_pool(bskenv_handle *h, int n_rows, const double *rows_host, int assign)
+{
+    if (!h) return BSKENV_EINVAL;
+    NO_HOST_PENDING(h, "bskenv_set_param_pool");
+    if (n_rows < 0 || (n_rows > 0 && !rows_host)) { h->err = "bskenv_set_param_pool: bad row count or null rows"; return BSKENV_EINVAL; }
+    if (n_rows > 0) {
+        if (assign != BSKENV_PARAMS_BY_INDEX && assign != BSKENV_PARAMS_PER_EPISODE) { h->err = "bskenv_set_param_pool: unknown assignment mode"; return BSKENV_EINVAL; }
+        if (h->P.nrw != 3 || !h->P.diag) { h->err = "bskenv_set_param_pool: per-env parameters are built for the three-wheel reference spacecraft (rw_set = 0)"; return BSKENV_EINVAL; }
+        if (h->P.mixed) { h->err = "bskenv_set_param_pool: per-env parameters are not built for precision = 1"; return BSKENV_EINVAL; }
+        if (h->P.grav_pfix) { h->err = "bskenv_set_param_pool: per-env parameters are not built for the degree-2 field"; return BSKENV_EINVAL; }
+        if (h->organisation == BSKENV_ORG_SPLIT) { h->err = "bskenv_set_param_pool: the split organisation has no per-env parameters"; return BSKENV_EINVAL; }
+    }
+    std::vector<double> rows((size_t)LEO_NPD * n_rows), one(LEO_NPD);
+    for (int r = 0; r < n_rows; r++) {
+        const std::string err = leo_host::param_row_build(h->cfg, rows_host + (size_t)r * BSKENV_PARAM_DIM, (double)r, one.data());
+        if (!err.empty()) { h->err = "bskenv_set_param_pool: row " + std::to_string(r) + ": " + err; return BSKENV_EINVAL; }
+        for (int f = 0; f < LEO_NPD; f++) rows[(size_t)f * n_rows + r] = one[f];
+    }
+    CU_TRY(h, cudaSetDevice(h->device));
+    CU_TRY(h, cudaDeviceSynchronize());                         // a launch in flight may still read the old pool or the state block
+    cudaFree((void *)h->pool.rows);
+    h->pool.rows = nullptr;
+    const bool was_loaded = h->pool.n_rows > 0;
+    h->pool.n_rows = 0;
+    if (n_rows == 0) return BSKENV_OK;                          // unloaded: the batch configuration, the batch-global kernels
+    if (h->s_fields < LEO_ND + LEO_NPD) {                       // first pool of this handle: room for the parameter block
+        double *S2 = nullptr;
+        CU_TRY(h, cudaMalloc(&S2, sizeof(double) * (LEO_ND + LEO_NPD) * h->stride));
+        CU_TRY(h, cudaMemcpy(S2, h->S, sizeof(double) * LEO_ND * h->stride, cudaMemcpyDeviceToDevice));
+        cudaFree(h->S);
+        h->S = S2; h->s_fields = LEO_ND + LEO_NPD;
+    }
+    if (!was_loaded) {                                          // running envs keep the batch values until their next reset
+        double raw[BSKENV_PARAM_DIM];
+        leo_host::param_row_get(h->cfg, raw);
+        leo_host::param_row_derive(h->P, raw, -1.0, one.data());
+        std::vector<double> blk((size_t)LEO_NPD * h->stride);
+        for (int f = 0; f < LEO_NPD; f++)
+            for (int64_t e = 0; e < h->stride; e++) blk[(size_t)f * h->stride + e] = one[f];
+        CU_TRY(h, cudaMemcpy(h->S + (size_t)LEO_ND * h->stride, blk.data(), sizeof(double) * blk.size(), cudaMemcpyHostToDevice));
+    }
+    double *d_rows = nullptr;
+    CU_TRY(h, cudaMalloc(&d_rows, sizeof(double) * rows.size()));
+    CU_TRY(h, cudaMemcpy(d_rows, rows.data(), sizeof(double) * rows.size(), cudaMemcpyHostToDevice));
+    h->pool.rows = d_rows; h->pool.n_rows = n_rows; h->pool.assign = assign;
+    return BSKENV_OK;
+}
+
+int bskenv_get_env_params(bskenv_handle *h, double *params_dev, int32_t *row_dev, void *stream)
+{
+    if (!h || !params_dev) { if (h) h->err = "bskenv_get_env_params: null params"; return BSKENV_EINVAL; }
+    CU_TRY(h, cudaSetDevice(h->device));
+    ParamRow batch;
+    leo_host::param_row_get(h->cfg, batch.v);
+    gather_params_kernel<<<(int)((h->n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->S, h->stride, h->n, h->pool.n_rows > 0 ? 1 : 0,
+                                                                                      batch, params_dev, row_dev);
+    CU_TRY(h, cudaGetLastError());
+    return BSKENV_OK;
+}
+
 static int do_reset(bskenv_handle *h, int mode, const double *ics_in, const uint8_t *mask, double *obs, void *stream)
 {
     if (!h) return BSKENV_EINVAL;
     NO_HOST_PENDING(h, "bskenv_reset");
     CU_TRY(h, cudaSetDevice(h->device));
     const int grid = (int)((h->n + 255) / 256);
-    leo_reset_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, mode, ics_in, mask, obs);
+    leo_reset_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, mode, ics_in, mask, obs, h->pool);
     CU_TRY(h, cudaGetLastError());
     CU_TRY(h, note_launch(h, (cudaStream_t)stream));
     return BSKENV_OK;

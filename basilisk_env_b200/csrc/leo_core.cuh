@@ -29,6 +29,13 @@
 
 namespace leo {
 
+// Where the functions below read the per-spacecraft parameters (bskenv_set_param_pool): a policy template parameter.
+// ParBatch, the default of every batch-global kernel, returns the field of the parameter block (a constant-bank operand);
+// ParEnv reads the env's own derived values.  PAt locates them.  Both are defined with the message bus (MBus) below.
+struct ParBatch;
+struct ParEnv;
+struct PAt;
+
 // ------------------------------------------------------------------------------------------------
 // small vector algebra
 // ------------------------------------------------------------------------------------------------
@@ -384,12 +391,15 @@ LEO_HD AttGuid att_tracking_error(V3 sigma_BN, V3 omega_BN_B, const AttRef &ref)
     g.domega_RN_B = rot_BN(BN, sigma_BN, ref.domega_RN_N);
     return g;
 }
-LEO_HD V3 mrp_feedback(const LeoParams &P, const AttGuid &g)
+template <class PA = ParBatch>
+LEO_HD V3 mrp_feedback(const LeoParams &P, const AttGuid &g, const double *S, int64_t stride, int64_t e)
 { // MRP_Feedback with Ki < 0 (integral off) and no wheel feed-forward wired (SIM:440-449)
+    double buf[9];
+    const double *Ifsw = PA::I_fsw(P, S, stride, e, buf);
     V3 w = g.omega_BR_B + g.omega_RN_B;
-    V3 Lr = g.omega_BR_B * P.P + g.sigma_BR * P.K;
-    Lr = Lr - cross(g.omega_RN_B, mv9(P.I_fsw, w));
-    Lr = Lr - mv9(P.I_fsw, g.domega_RN_B - cross(w, g.omega_RN_B));
+    V3 Lr = g.omega_BR_B * PA::Pgain(P, S, stride, e) + g.sigma_BR * PA::K(P, S, stride, e);
+    Lr = Lr - cross(g.omega_RN_B, mv9(Ifsw, w));
+    Lr = Lr - mv9(Ifsw, g.domega_RN_B - cross(w, g.omega_RN_B));
     return -Lr;
 }
 
@@ -430,7 +440,7 @@ LEO_HD_NOINLINE void thr_force_mapping(const LeoParams &P, V3 Lr, double (&F)[LE
 // Returns 1 when the dumping block ran and left nothing to do: no on-time remaining on any thruster and a zero
 // command (the chain is then "quiet": until the next Reset every pass only advances the rest counter and the
 // time tag, see fsw_pass).
-template <int NRW>
+template <int NRW, class PA = ParBatch>
 LEO_HD_NOINLINE int fsw_desat(const LeoParams &P, double *S, int64_t *I, int64_t stride, int64_t e, int64_t now_ns,
                               const double (&ws)[NRW])
 {
@@ -441,7 +451,8 @@ LEO_HD_NOINLINE int fsw_desat(const LeoParams &P, double *S, int64_t *I, int64_t
         V3 hs = mk(0., 0., 0.);
         for (int i = 0; i < NRW; i++) hs = hs + arr(P.gs[i]) * (P.Js[i] * ws[i]);
         double hm = norm(hs);
-        V3 dH = (hm < P.hs_min) ? mk(0., 0., 0.) : hs * (-(hm - P.hs_min) / hm);
+        const double hs_min = PA::hs_min(P, S, stride, e);
+        V3 dH = (hm < hs_min) ? mk(0., 0., 0.) : hs * (-(hm - hs_min) / hm);
         SD(F_DELTAH) = dH.x; SD(F_DELTAH + 1) = dH.y; SD(F_DELTAH + 2) = dH.z;
         SI(I_DHTIME) = now_ns;
         SI(I_INITREQ) = 0;
@@ -765,6 +776,7 @@ LEO_HD_NOINLINE void sample_ic(const LeoParams &P, int64_t global_env, int64_t e
 // reset: LEOPowerAttitudeSimulator.__init__ (SIM:67-117) + InitializeSimulationAndDiscover, and the
 // initial observation of leoPowerAttEnv.reset (ENV:188-190)
 // ------------------------------------------------------------------------------------------------
+template <class PA = ParBatch>
 LEO_HD void leo_reset_env(const LeoParams &P, double *S, int64_t *I, int64_t stride, int64_t e, const double (&ic)[19],
                           double *obs /* 5, may be null */)
 {
@@ -775,7 +787,8 @@ LEO_HD void leo_reset_env(const LeoParams &P, double *S, int64_t *I, int64_t str
     for (int f = 0; f < LEO_NI; f++) SI(f) = 0;
     SI(I_EPISODE) = episode;
     for (int k = 0; k < 12; k++) SD(F_R + k) = ic[k];
-    for (int k = 0; k < 3; k++) SD(F_LDIST + k) = P.dist_mag * ic[12 + k];             // SIM:295 (quirk Q4: raw vector)
+    const double dist_mag = PA::dist_mag(P, S, stride, e);
+    for (int k = 0; k < 3; k++) SD(F_LDIST + k) = dist_mag * ic[12 + k];               // SIM:295 (quirk Q4: raw vector)
     for (int k = 0; k < 3; k++) SD(F_WHL + k) = ic[15 + k] * P.wheel_rpm2rad;       // SIM:303-305
     const double w4 = (ic[15] + ic[16] + ic[17]) / 3.0;                              // rw_set 1: fourth wheel at the mean speed
     if (P.nrw == 4) SD(F_WHL + 3) = w4 * P.wheel_rpm2rad;
@@ -821,7 +834,10 @@ enum LeoMField : int {
     // only allocated by the planet-fixed gravity variant (J2 == 2):
     M_PFIX = 54,     // J20002Pfix of the last SPICE message (9, row-major)
     M_PFIXD = 63,    // J20002Pfix_dot (9)
-    LEO_NM_PFIX = 72
+    LEO_NM_PFIX = 72,
+    // only allocated by the per-env parameter kernel (ParEnv): the stage-rate parameters PE_INV_MASS..PE_DRAGKA+2
+    M_PE = 54,
+    LEO_NM_PENV = 64
 };
 #define LEO_M_MIRROR 28          // number of leading bus fields that mirror state fields starting at F_GUID
 struct MBus {
@@ -848,6 +864,84 @@ LEO_HD void mst(MBus m, int f, double v)
 }
 LEO_HD V3 mld3(MBus m, int f) { return mk(mld(m, f), mld(m, f + 1), mld(m, f + 2)); }
 LEO_HD void mst3(MBus m, int f, V3 v) { mst(m, f, v.x); mst(m, f + 1, v.y); mst(m, f + 2, v.z); }
+
+// ------------------------------------------------------------------------------------------------
+// per-spacecraft parameters (see ParBatch above)
+// ------------------------------------------------------------------------------------------------
+struct PAt { MBus m; const double *S; int64_t stride, e; };   // an env's bus column and state column
+struct ParBatch {
+    // read at every RK stage
+    LEO_HD static void load_bus(const LeoParams &, const PAt &) {}
+    LEO_HD static double inv_mass(const LeoParams &P, const PAt &) { return P.inv_mass; }
+    LEO_HD static double D(const LeoParams &P, const PAt &, int k) { return P.D[4 * k]; }          // diagonal (DIAG path)
+    LEO_HD static double Dinv(const LeoParams &P, const PAt &, int k) { return P.Dinv[4 * k]; }
+    LEO_HD static double dragKa(const LeoParams &P, const PAt &, int k) { return P.dragKa[k]; }
+    // read once per dynamics tick, per flight-software pass or per reset
+    LEO_HD static double rho0(const LeoParams &P, const double *, int64_t, int64_t) { return P.rho0; }
+    LEO_HD static double inv_H(const LeoParams &P, const double *, int64_t, int64_t) { return P.inv_H; }
+    LEO_HD static double panel_coef(const LeoParams &P, const double *, int64_t, int64_t) { return P.panel_coef; }
+    LEO_HD static double sink_power(const LeoParams &P, const double *, int64_t, int64_t) { return P.sink_power; }
+    LEO_HD static double capacity(const LeoParams &P, const double *, int64_t, int64_t) { return P.capacity; }
+    LEO_HD static double K(const LeoParams &P, const double *, int64_t, int64_t) { return P.K; }
+    LEO_HD static double Pgain(const LeoParams &P, const double *, int64_t, int64_t) { return P.P; }
+    LEO_HD static const double *I_fsw(const LeoParams &P, const double *, int64_t, int64_t, double *) { return P.I_fsw; }
+    LEO_HD static double hs_min(const LeoParams &P, const double *, int64_t, int64_t) { return P.hs_min; }
+    LEO_HD static double dist_mag(const LeoParams &P, const double *, int64_t, int64_t) { return P.dist_mag; }
+};
+// The env's own values: the LEO_NPD block behind the state fields (leo_params.h: LeoPField).  The stage-rate values are
+// copied into this thread's bus column once per call of leo_step_env (load_bus) and read from shared memory at every
+// stage; the others are read from global memory where they are used.  LEO_PENV_GLOBAL (measurement builds, DESIGN.md
+// section 12) reads the stage-rate values from global memory as well.  Only the DIAG path reads D / Dinv through here.
+struct ParEnv {
+    LEO_HD static double g(const double *S, int64_t stride, int64_t e, int f) { return S[(int64_t)(LEO_ND + f) * stride + e]; }
+#ifdef LEO_PENV_GLOBAL
+    LEO_HD static void load_bus(const LeoParams &, const PAt &) {}
+    LEO_HD static double st(const PAt &at, int f) { return g(at.S, at.stride, at.e, f); }
+#else
+    LEO_HD static void load_bus(const LeoParams &, const PAt &at)
+    {
+#pragma unroll
+        for (int f = PE_INV_MASS; f <= PE_DRAGKA + 2; f++) mst(at.m, M_PE + f, g(at.S, at.stride, at.e, f));
+    }
+    LEO_HD static double st(const PAt &at, int f) { return mld(at.m, M_PE + f); }
+#endif
+    LEO_HD static double inv_mass(const LeoParams &, const PAt &at) { return st(at, PE_INV_MASS); }
+    LEO_HD static double D(const LeoParams &, const PAt &at, int k) { return st(at, PE_D + k); }
+    LEO_HD static double Dinv(const LeoParams &, const PAt &at, int k) { return st(at, PE_DINV + k); }
+    LEO_HD static double dragKa(const LeoParams &, const PAt &at, int k) { return st(at, PE_DRAGKA + k); }
+    LEO_HD static double rho0(const LeoParams &, const double *S, int64_t s, int64_t e) { return g(S, s, e, PE_RHO0); }
+    LEO_HD static double inv_H(const LeoParams &, const double *S, int64_t s, int64_t e) { return g(S, s, e, PE_INV_H); }
+    LEO_HD static double panel_coef(const LeoParams &, const double *S, int64_t s, int64_t e) { return g(S, s, e, PE_PANEL); }
+    LEO_HD static double sink_power(const LeoParams &, const double *S, int64_t s, int64_t e) { return g(S, s, e, PE_SINK); }
+    LEO_HD static double capacity(const LeoParams &, const double *S, int64_t s, int64_t e) { return g(S, s, e, PE_CAP); }
+    LEO_HD static double K(const LeoParams &, const double *S, int64_t s, int64_t e) { return g(S, s, e, PE_K); }
+    LEO_HD static double Pgain(const LeoParams &, const double *S, int64_t s, int64_t e) { return g(S, s, e, PE_P); }
+    LEO_HD static const double *I_fsw(const LeoParams &, const double *S, int64_t s, int64_t e, double *buf)
+    { // the same 3x3 product as the batch path (its off-diagonal zeros included): identical arithmetic for a default row
+        for (int k = 0; k < 9; k++) buf[k] = 0.0;
+        for (int k = 0; k < 3; k++) buf[4 * k] = g(S, s, e, PE_IFSW + k);
+        return buf;
+    }
+    LEO_HD static double hs_min(const LeoParams &, const double *S, int64_t s, int64_t e) { return g(S, s, e, PE_HSMIN); }
+    LEO_HD static double dist_mag(const LeoParams &, const double *S, int64_t s, int64_t e) { return g(S, s, e, PE_DIST); }
+};
+
+// Pool row of an env at a reset.  BY_INDEX: global env index mod n_rows.  PER_EPISODE: one Philox4x32-10 block keyed like
+// the IC stream, (seed, global env, episode), at counter word 0xFFFFFFFF, which the IC sampler (blocks 0, 1, ...) never
+// reaches: the IC draws are those of a run without a pool, and neither depends on the sharding.
+LEO_HD int64_t pool_row(const LeoPool &pool, uint64_t seed, int64_t global_env, int64_t episode)
+{
+    if (pool.assign == LEO_POOL_BY_INDEX) return global_env % pool.n_rows;
+    uint32_t o[4];
+    philox4x32((uint32_t)global_env, (uint32_t)((uint64_t)global_env >> 32), (uint32_t)episode, 0xFFFFFFFFu, (uint32_t)seed,
+               (uint32_t)(seed >> 32), o);
+    return (int64_t)((((uint64_t)o[1] << 32) | o[0]) % (uint64_t)pool.n_rows);
+}
+// Copy a derived pool row into the env's parameter block
+LEO_HD void pool_assign(const LeoPool &pool, double *S, int64_t stride, int64_t e, int64_t row)
+{
+    for (int f = 0; f < LEO_NPD; f++) S[(int64_t)(LEO_ND + f) * stride + e] = pool.rows[(int64_t)f * pool.n_rows + row];
+}
 
 LEO_HD_NOINLINE void sun_latch_to_bus(const LeoParams &P, MBus m, int64_t msg_ns)
 {
@@ -893,7 +987,7 @@ LEO_HD_NOINLINE void pfix_latch_to_bus(const LeoParams &P, MBus m, int64_t msg_n
 // Returns the state of the desat chain: 0 did not run; 1 full pass; 3 full pass that left the chain quiet (to be
 // confirmed by the thruster latch); 4 quiet pass (all on-times and commands are zero and stay zero: only
 // thrMomentumDumping's rest counter and time tag advance).
-template <int NRW>
+template <int NRW, class PA = ParBatch>
 LEO_HD_NOINLINE int fsw_pass(const LeoParams &P, double *S, int64_t *I, int64_t stride, int64_t e, MBus m, int mask,
                              int64_t n, int64_t now_ns, Dyn x, const double (&W)[NRW], int64_t sun_ns, int desat_quiet)
 {
@@ -929,7 +1023,7 @@ LEO_HD_NOINLINE int fsw_pass(const LeoParams &P, double *S, int64_t *I, int64_t 
             I[(int64_t)I_DUMPPRIOR * stride + e] = now_ns;
             desat_ran = 4;
         } else {
-            desat_ran = 1 | (fsw_desat<NRW>(P, S, I, stride, e, now_ns, ws) << 1);
+            desat_ran = 1 | (fsw_desat<NRW, PA>(P, S, I, stride, e, now_ns, ws) << 1);
         }
     }
     if (mask & LEO_TASK_MRP) {
@@ -937,7 +1031,7 @@ LEO_HD_NOINLINE int fsw_pass(const LeoParams &P, double *S, int64_t *I, int64_t 
         AttGuid g;
         g.sigma_BR = mld3(m, M_GUID); g.omega_BR_B = mld3(m, M_GUID + 3);
         g.omega_RN_B = mld3(m, M_GUID + 6); g.domega_RN_B = mld3(m, M_GUID + 9);
-        V3 Lr = mrp_feedback(P, g);
+        V3 Lr = mrp_feedback<PA>(P, g, S, stride, e);
         mst3(m, M_LR, Lr);
         g = att_tracking_error(ns, nw, ref);
         mst3(m, M_GUID, g.sigma_BR); mst3(m, M_GUID + 3, g.omega_BR_B);
@@ -996,9 +1090,11 @@ struct StageIn {
 //   DIAG   fast path of the reference configuration: diagonal hub inertia, three wheels along the body axes
 //          (AP:20-37) and drag facets located on their own normal axis (SIM:274-281) -- the same arithmetic
 //          with the structural zeros dropped
-template <int J2, bool DIAG>
-LEO_HD void eom(const LeoParams &P, const Dyn &x, Dyn &k, const StageIn &a, double ct, bool thr_on, MBus m)
+template <int J2, bool DIAG, class PA = ParBatch>
+LEO_HD void eom(const LeoParams &P, const Dyn &x, Dyn &k, const StageIn &a, double ct, bool thr_on, MBus m,
+                const double *S = nullptr, int64_t stride = 0, int64_t e = 0)
 {
+    const PAt at = {m, S, stride, e};
     // gravity: central point mass (+J2) + Sun third body (gravityEffector)
     V3 g;
     {
@@ -1035,7 +1131,7 @@ LEO_HD void eom(const LeoParams &P, const Dyn &x, Dyn &k, const StageIn &a, doub
     {
         double ax = fabs(vB.x), ay = fabs(vB.y), az = fabs(vB.z);
         // DIAG also means equal + / - facet areas on every axis (SIM:274-281: 0.06 / 0.06, 2.02 / 2.02, 0.03 / 0.03): Kd = 0
-        Sp = P.dragKa[0] * ax + P.dragKa[1] * ay + P.dragKa[2] * az;
+        Sp = PA::dragKa(P, at, 0) * ax + PA::dragKa(P, at, 1) * ay + PA::dragKa(P, at, 2) * az;
         if (!DIAG) Sp += P.dragKd[0] * vB.x + P.dragKd[1] * vB.y + P.dragKd[2] * vB.z;
         if (DIAG) {
             Mp = mk(P.dragMa[0][0] * ax + P.dragMd[0][0] * vB.x, P.dragMa[1][1] * ay + P.dragMd[1][1] * vB.y,
@@ -1054,9 +1150,9 @@ LEO_HD void eom(const LeoParams &P, const Dyn &x, Dyn &k, const StageIn &a, doub
     V3 rot = add_cross(a.Lc, Mp * mrho, vB);
     const V3 hw = a.HB + a.tau_u * ct;
     if (DIAG) {
-        V3 h = mk(fmad(P.D[0], x.w.x, hw.x), fmad(P.D[4], x.w.y, hw.y), fmad(P.D[8], x.w.z, hw.z));
+        V3 h = mk(fmad(PA::D(P, at, 0), x.w.x, hw.x), fmad(PA::D(P, at, 1), x.w.y, hw.y), fmad(PA::D(P, at, 2), x.w.z, hw.z));
         rot = sub_cross(rot, x.w, h);
-        k.w = mk(rot.x * P.Dinv[0], rot.y * P.Dinv[4], rot.z * P.Dinv[8]);
+        k.w = mk(rot.x * PA::Dinv(P, at, 0), rot.y * PA::Dinv(P, at, 1), rot.z * PA::Dinv(P, at, 2));
     } else {
         V3 h = mv9(P.D, x.w) + hw;
         rot = sub_cross(rot, x.w, h);
@@ -1077,8 +1173,9 @@ LEO_HD void eom(const LeoParams &P, const Dyn &x, Dyn &k, const StageIn &a, doub
 // The Sun's third-body acceleration is held (evaluated by the caller once per flight-software period at the period's mid
 // time and predicted mid position, see sun_window()); the thrust is constant over the step.  Steps in which a thruster may
 // switch, and the step whose Sun clock wraps, go through rk4_general().
-template <int J2, bool DIAG>
-LEO_HD Dyn rk4_step(const LeoParams &P, const Dyn &x, const StageIn &a, bool thr_on, MBus m)
+template <int J2, bool DIAG, class PA = ParBatch>
+LEO_HD Dyn rk4_step(const LeoParams &P, const Dyn &x, const StageIn &a, bool thr_on, MBus m,
+                    const double *S = nullptr, int64_t stride = 0, int64_t e = 0)
 {
     const double h = a.h, hh = 0.5 * h, h6 = h * (1.0 / 6.0), h3 = h * (1.0 / 3.0);
     Dyn k, acc;
@@ -1094,7 +1191,7 @@ LEO_HD Dyn rk4_step(const LeoParams &P, const Dyn &x, const StageIn &a, bool thr
     for (int st = 0; st < 4; st++) {
         Dyn xs;
         xs.r = x.r + k.r * c; xs.v = x.v + k.v * c; xs.s = x.s + k.s * c; xs.w = x.w + k.w * c;
-        eom<J2, DIAG>(P, xs, k, a, c, thr_on, m);
+        eom<J2, DIAG, PA>(P, xs, k, a, c, thr_on, m, S, stride, e);
         const double wo = (st == 0 || st == 3) ? h6 : h3;
         acc.r = acc.r + k.r * wo; acc.v = acc.v + k.v * wo; acc.s = acc.s + k.s * wo; acc.w = acc.w + k.w * wo;
         c = (st == 2) ? h : hh;
@@ -1112,7 +1209,7 @@ LEO_HD Dyn rk4_step(const LeoParams &P, const Dyn &x, const StageIn &a, bool thr
 // accumulation order.
 struct SunDt { double d0, dm, d1; };
 struct ThrEventOut { Dyn x; int factor, active; };
-template <int J2, bool DIAG>
+template <int J2, bool DIAG, class PA = ParBatch>
 LEO_HD_NOINLINE ThrEventOut rk4_general(const LeoParams &P, const double *S, int64_t stride, int64_t e, MBus m, Dyn x,
                                         StageIn a, SunDt dts, double tBefore, double tauPrev, int thr_factor, int thr_active)
 {
@@ -1133,12 +1230,12 @@ LEO_HD_NOINLINE ThrEventOut rk4_general(const LeoParams &P, const double *S, int
             const double tau = t_add(tBefore, (st == 0) ? 0.0 : (st == 3 ? h : t_mul(h, 0.5)));
             ThrOut to = thr_stage(P, tc, tau, t_sub(tau, tauPrev), thr_factor);
             thr_factor = to.factor; thr_active = to.active;
-            Fm = to.F * P.inv_mass; Lx = Lx + to.L;
+            Fm = to.F * PA::inv_mass(P, PAt{m, S, stride, e}); Lx = Lx + to.L;
             tauPrev = tau;
         }
         a.Lc = Lx - a.tau_u;
         mst3(m, M_FM, Fm);
-        eom<J2, DIAG>(P, xs, k, a, ct, thr_on, m);
+        eom<J2, DIAG, PA>(P, xs, k, a, ct, thr_on, m, S, stride, e);
         const double wo = (st == 0 || st == 3) ? h6 : h3;
         const double cn = (st == 2) ? h : hh;
         xo.r = xo.r + k.r * wo; xo.v = xo.v + k.v * wo; xo.s = xo.s + k.s * wo; xo.w = xo.w + k.w * wo;
@@ -1154,6 +1251,7 @@ LEO_HD_NOINLINE ThrEventOut rk4_general(const LeoParams &P, const double *S, int
 // time and the commanded on-times only change at the next command latch).  Publishes the held thrust on the
 // bus and rebuilds the held body torque.
 struct ThrRefresh { V3 Lc, L_thr; double t_next; };
+template <class PA = ParBatch>
 LEO_HD_NOINLINE ThrRefresh thr_refresh(const LeoParams &P, const double *S, int64_t stride, int64_t e, MBus m, int factor, V3 tau_u)
 {
     ThrRefresh o;
@@ -1168,7 +1266,7 @@ LEO_HD_NOINLINE ThrRefresh thr_refresh(const LeoParams &P, const double *S, int6
         double t_off = t_add(S[(int64_t)(F_THRON + k) * stride + e], start);
         if (t_off < o.t_next) o.t_next = t_off;
     }
-    mst3(m, M_FM, F * P.inv_mass);
+    mst3(m, M_FM, F * PA::inv_mass(P, PAt{m, S, stride, e}));
     o.Lc = (mld3(m, M_LEXT) + o.L_thr) - tau_u;
     return o;
 }
@@ -1289,7 +1387,8 @@ LEO_HD double exp_bounded(double x)
 namespace leo {
 
 // F32 = false: the FP64 kernel (the reference's arithmetic; every parity claim).  F32 = true: mixed precision, see leo_f32.cuh.
-template <int NRW, int J2, bool DIAG, bool F32 = false>
+// PA = ParEnv: the env's own spacecraft parameters (bskenv_set_param_pool; DIAG, FP64 only).
+template <int NRW, int J2, bool DIAG, bool F32 = false, class PA = ParBatch>
 // `chunk` / `n_chunks`: the decision interval may be executed as n_chunks consecutive calls of ticks/n_chunks dynamics
 // ticks each (chunk 0 applies the mode switch, the last chunk samples the observation and does the gym bookkeeping); the
 // persistent state carries everything across a chunk boundary exactly as it does across a decision boundary, and the
@@ -1307,6 +1406,7 @@ LEO_HD void leo_step_env(const LeoParams &P, double *__restrict__ S, int64_t *__
     x.v = mk(SD(F_V), SD(F_V + 1), SD(F_V + 2));
     x.s = mk(SD(F_SIG), SD(F_SIG + 1), SD(F_SIG + 2));
     x.w = mk(SD(F_OMG), SD(F_OMG + 1), SD(F_OMG + 2));
+    PA::load_bus(P, PAt{m, S, stride, e});
     double C[NRW], uJ[NRW];                                     // wheel invariants / motor torque over Js (general path)
     a.tau_u = mk(0., 0., 0.); a.HB = mk(0., 0., 0.);
 #pragma unroll
@@ -1398,7 +1498,7 @@ LEO_HD void leo_step_env(const LeoParams &P, double *__restrict__ S, int64_t *__
             double W[NRW];
             wheel_speeds<NRW, DIAG>(P, a.HB, C, x.w, W);
 #ifndef LEO_EXP_NOFSW       // (LEO_EXP_*: measurement switches -- compile a block out to read its cost off the clock, DESIGN.md 5b / 6)
-            desat_ran = fsw_pass<NRW>(P, S, I, stride, e, m, mask, n, n * P.dyn_ns, x, W, (int64_t)sun_d, desat_quiet);
+            desat_ran = fsw_pass<NRW, PA>(P, S, I, stride, e, m, mask, n, n * P.dyn_ns, x, W, (int64_t)sun_d, desat_quiet);
             rw_sat |= 2;
 #endif    // a (possibly) new wheel command: re-latch after this tick's integration
             // SpiceTask was queued for this time long before DynTask -> runs first (scheduler FIFO rule); the
@@ -1431,9 +1531,9 @@ LEO_HD void leo_step_env(const LeoParams &P, double *__restrict__ S, int64_t *__
                 const double ph = t_sub(prevTime, ppT);
                 tauPrev = t_add(t_sub(prevTime, ph), ph);
             }
-            ThrEventOut o = rk4_general<J2, DIAG>(P, S, stride, e, m, x, a, dts, tBefore, tauPrev, thr_factor, thr_active);
+            ThrEventOut o = rk4_general<J2, DIAG, PA>(P, S, stride, e, m, x, a, dts, tBefore, tauPrev, thr_factor, thr_active);
             x = o.x; thr_factor = o.factor; thr_active = o.active;
-            ThrRefresh th = thr_refresh(P, S, stride, e, m, thr_active ? thr_factor : 0, a.tau_u);
+            ThrRefresh th = thr_refresh<PA>(P, S, stride, e, m, thr_active ? thr_factor : 0, a.tau_u);
             a.Lc = th.Lc; mst3(m, M_LTHR, th.L_thr); mst(m, M_TNEXT, th.t_next);
         } else if (F32) {
             StageInF af;
@@ -1444,7 +1544,7 @@ LEO_HD void leo_step_env(const LeoParams &P, double *__restrict__ S, int64_t *__
             x = rk4_step_mixed<(J2 != 0), DIAG>(PF, x, af, thr_on, thr_on ? tof(mld3(m, M_FM)) : mkf(0.f, 0.f, 0.f));
         } else {
             if (J2 == 2) a.dtp = dtsm;     // orientation held at the step's mid time, like the Sun
-            x = rk4_step<J2, DIAG>(P, x, a, thr_active != 0, m);
+            x = rk4_step<J2, DIAG, PA>(P, x, a, thr_active != 0, m, S, stride, e);
         }
         // ================= everything else that runs every tick: one straight-line block =================
         // the wheel invariant advances with the motor torque held over the step
@@ -1485,7 +1585,7 @@ LEO_HD void leo_step_env(const LeoParams &P, double *__restrict__ S, int64_t *__
         } else {
             r2 = dot(x.r, x.r); ir = rsq(r2);
             // exponentialAtmosphere (density latched for the NEXT step, zero-order hold)
-            a.rho = P.rho0 * exp_bounded(-(r2 * ir - P.Rp_atmo) * P.inv_H);
+            a.rho = PA::rho0(P, S, stride, e) * exp_bounded(-(r2 * ir - P.Rp_atmo) * PA::inv_H(P, S, stride, e));
         }
         // wheel-limit flags (the latch itself is a rare event, below)
         double W[NRW];
@@ -1507,7 +1607,7 @@ LEO_HD void leo_step_env(const LeoParams &P, double *__restrict__ S, int64_t *__
             V3 n_N = rot_NB(R, x.s, arr(P.nHat_B));            // panel normal in the inertial frame
             double proj = dot(n_N, r_SB) * id;                 // sHat_B . nHat_B
             if (proj < 0.) proj = 0.;
-            pgeo = P.panel_coef * proj * (id * id);
+            pgeo = PA::panel_coef(P, S, stride, e) * proj * (id * id);
         }
 #endif
         // clock of the NEXT tick
@@ -1552,8 +1652,9 @@ LEO_HD void leo_step_env(const LeoParams &P, double *__restrict__ S, int64_t *__
         // ================= battery (quirk Q2: the sink message does not exist at tick 0) =================
         {
             const double panel = F32 ? (double)(panel_f * shf) : pgeo * shadow;
-            double E = charge + (panel + P.sink_power) * h_this;
-            if (E > P.capacity) E = P.capacity;
+            const double capacity = PA::capacity(P, S, stride, e);
+            double E = charge + (panel + PA::sink_power(P, S, stride, e)) * h_this;
+            if (E > capacity) E = capacity;
             if (E < 0.) E = 0.;
             charge = j >= 0 ? E : charge;
         }

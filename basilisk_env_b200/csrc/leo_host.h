@@ -176,6 +176,49 @@ static inline std::string build_params(const bskenv_config &c, LeoParams &p)
     return "";
 }
 
+// ---- per-env parameter pools (bskenv_set_param_pool): BSKENV_PARAM_DIM reference values per row ----
+static inline void param_row_get(const bskenv_config &c, double r[BSKENV_PARAM_DIM])
+{
+    const double v[BSKENV_PARAM_DIM] = {c.mass, c.width, c.depth, c.height, c.baseDensity, c.scaleHeight, c.disturbance_magnitude,
+                                        c.panelArea, c.panelEfficiency, c.powerDraw, c.storageCapacity, c.K, c.P, c.hs_min};
+    memcpy(r, v, sizeof(v));
+}
+static inline void param_row_set(bskenv_config &c, const double r[BSKENV_PARAM_DIM])
+{
+    c.mass = r[0]; c.width = r[1]; c.depth = r[2]; c.height = r[3]; c.baseDensity = r[4]; c.scaleHeight = r[5];
+    c.disturbance_magnitude = r[6]; c.panelArea = r[7]; c.panelEfficiency = r[8]; c.powerDraw = r[9]; c.storageCapacity = r[10];
+    c.K = r[11]; c.P = r[12]; c.hs_min = r[13];
+}
+// The values a row puts into an env's parameter block (leo_params.h: LeoPField), taken from the parameter block that
+// build_params derived for the configuration with the row's values: the device never re-derives them.
+static inline void param_row_derive(const LeoParams &p, const double raw[BSKENV_PARAM_DIM], double row, double out[LEO_NPD])
+{
+    out[PE_INV_MASS] = p.inv_mass;
+    for (int k = 0; k < 3; k++) {
+        out[PE_D + k] = p.D[4 * k]; out[PE_DINV + k] = p.Dinv[4 * k]; out[PE_DRAGKA + k] = p.dragKa[k]; out[PE_IFSW + k] = p.I_fsw[4 * k];
+    }
+    out[PE_RHO0] = p.rho0; out[PE_INV_H] = p.inv_H; out[PE_PANEL] = p.panel_coef; out[PE_SINK] = p.sink_power;
+    out[PE_CAP] = p.capacity; out[PE_K] = p.K; out[PE_P] = p.P; out[PE_HSMIN] = p.hs_min; out[PE_DIST] = p.dist_mag;
+    out[PE_ROW] = row;
+    for (int k = 0; k < BSKENV_PARAM_DIM; k++) out[PE_RAW + k] = raw[k];
+}
+// Checks a row against the configuration it is applied to and derives it; returns "" or an error message.
+static inline std::string param_row_build(const bskenv_config &base, const double raw[BSKENV_PARAM_DIM], double row, double out[LEO_NPD])
+{
+    for (int k = 0; k < BSKENV_PARAM_DIM; k++)
+        if (!isfinite(raw[k])) return "non-finite value";
+    if (!(raw[0] > 0) || !(raw[1] > 0) || !(raw[2] > 0) || !(raw[3] > 0)) return "mass, width, depth and height must be positive";
+    if (!(raw[5] > 0)) return "scaleHeight must be positive";
+    if (!(raw[10] > 0)) return "storageCapacity must be positive";
+    bskenv_config c = base;
+    param_row_set(c, raw);
+    LeoParams p;
+    const std::string err = build_params(c, p);
+    if (!err.empty()) return err;
+    param_row_derive(p, raw, row, out);
+    return "";
+}
+
 // SURVEY 8(f)-4: normalised degree-2 coefficients (C20, C21, S21, C22, S22; the form gravity-model files carry and
 // Basilisk's loadGravFromFile reads) -> mu Req^2 [M] of the closed-form gradient used by the kernel.
 // Un-normalisation: C_nm = Cbar_nm sqrt((2 - delta_0m)(2n + 1)(n - m)!/(n + m)!).

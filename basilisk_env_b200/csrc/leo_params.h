@@ -139,6 +139,34 @@ enum LeoIField : int {
     LEO_NI = 22
 };
 
+// ---- per-env spacecraft parameters (bskenv_set_param_pool): derived values of the env's pool row ----
+// Field-major [LEO_NPD][stride] block that follows the LEO_ND double state fields in the same allocation, so that every
+// function that addresses an env's state (S, stride, e) also reaches its parameters.  Values come from
+// leo_host::build_params on the host; the device never re-derives them.
+enum LeoPField : int {
+    PE_INV_MASS = 0, // 1 / mass
+    PE_D = 1,        // diagonal of D (3)
+    PE_DINV = 4,     // diagonal of Dinv (3)
+    PE_DRAGKA = 7,   // dragKa (3), carries 1 / mass
+    PE_RHO0 = 10,
+    PE_INV_H = 11,
+    PE_PANEL = 12,   // panel_coef
+    PE_SINK = 13,    // sink_power
+    PE_CAP = 14,     // capacity
+    PE_K = 15,
+    PE_P = 16,
+    PE_IFSW = 17,    // diagonal of I_fsw (3)
+    PE_HSMIN = 20,
+    PE_DIST = 21,    // dist_mag
+    PE_ROW = 22,     // pool row of the env, -1 = the batch configuration
+    PE_RAW = 23,     // the row itself: BSKENV_PARAM_DIM reference values (bskenv_get_env_params; the kernels never read them)
+    LEO_NPD = 37
+};
+// Loaded pool: derived rows field-major [LEO_NPD][n_rows] (PE_ROW holds the row index); assign = LEO_POOL_*
+#define LEO_POOL_BY_INDEX 0      // row = global env index mod n_rows           (BSKENV_PARAMS_BY_INDEX)
+#define LEO_POOL_PER_EPISODE 1   // row drawn per (seed, global env, episode)   (BSKENV_PARAMS_PER_EPISODE)
+struct LeoPool { const double *rows; int32_t n_rows, assign; };
+
 #define LEO_TASK_SUN 1
 #define LEO_TASK_NADIR 2
 #define LEO_TASK_MRP 4

@@ -142,6 +142,12 @@ CONFIG_KEYS = ("mass", "width", "depth", "height", "planetRadius", "baseDensity"
                "maxCounterValue", "thrMinFireTime")
 
 
+# keys of the initial_conditions dict that may differ from env to env through a parameter pool
+# (LeoPowerAttVecEnv.set_param_pool, include/bskenv.h bskenv_set_param_pool), in the C ABI's row order (BSKENV_PARAM_DIM)
+PARAM_KEYS = ("mass", "width", "depth", "height", "baseDensity", "scaleHeight", "disturbance_magnitude", "panelArea",
+              "panelEfficiency", "powerDraw", "storageCapacity", "K", "P", "hs_min")
+
+
 def config_overrides(ic):
     """bskenv_config overrides carried by an `initial_conditions` dict."""
     out = {}

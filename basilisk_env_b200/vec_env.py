@@ -11,6 +11,7 @@ import torch
 
 from . import _native
 from . import spaces
+from .initial_conditions import PARAM_KEYS
 
 DONE_MAXLEN, DONE_WHEEL, DONE_POWER, DONE_DECAY = 1, 2, 4, 8
 OBS_DIM, IC_DIM = 5, 19
@@ -136,6 +137,43 @@ class LeoPowerAttVecEnv:
             assert cbar.shape == (5,)
             ptr = cbar.ctypes.data
         self._check(self._L.bskenv_set_gravity_degree2(self._h, int(bool(enable)), ptr), "set_gravity_degree2")
+
+    def set_param_pool(self, pool, assign="per_episode"):
+        """Load a pool of spacecraft parameter sets (Monte Carlo dispersions / domain randomisation): each env runs one row
+        for a whole episode, picked at its next reset (include/bskenv.h: bskenv_set_param_pool).
+        pool : dict of `initial_conditions.PARAM_KEYS` -> arrays [K] (missing keys take the configuration's value), or an
+            array [K, 14] in PARAM_KEYS order; None unloads the pool.
+        assign : "per_episode" (row drawn per (seed, global env index, episode)) or "by_index" (row = global env index
+            mod K: with K = the global env count, an explicit per-env table)."""
+        if pool is None:
+            self._check(self._L.bskenv_set_param_pool(self._h, 0, None, 0), "bskenv_set_param_pool")
+            return
+        if isinstance(pool, dict):
+            unknown = set(pool) - set(PARAM_KEYS)
+            if unknown:
+                raise KeyError(f"not per-env parameters: {sorted(unknown)} (see initial_conditions.PARAM_KEYS)")
+            cols = {k: np.ravel(np.asarray(v, dtype=np.float64)) for k, v in pool.items()}
+            sizes = {len(v) for v in cols.values()}
+            if len(sizes) != 1:
+                raise ValueError("every pool column needs the same length")
+            k = sizes.pop()
+            rows = np.stack([cols[key] if key in cols else np.full(k, float(getattr(self.cfg, key))) for key in PARAM_KEYS], axis=1)
+        else:
+            rows = np.asarray(pool.cpu().numpy() if torch.is_tensor(pool) else pool, dtype=np.float64)
+        rows = np.ascontiguousarray(rows, dtype=np.float64)
+        if rows.ndim != 2 or rows.shape[1] != len(PARAM_KEYS) or rows.shape[0] == 0:
+            raise ValueError(f"pool must have shape (K, {len(PARAM_KEYS)}) with K > 0")
+        self._check(self._L.bskenv_set_param_pool(self._h, rows.shape[0], rows.ctypes.data, PARAM_ASSIGN[assign]),
+                    "bskenv_set_param_pool")
+
+    def env_params(self):
+        """The spacecraft parameters every env runs with: (dict of PARAM_KEYS -> [N] f64 tensors, pool row [N] int32,
+        -1 = the batch configuration)."""
+        p = torch.empty((self.num_envs, len(PARAM_KEYS)), dtype=torch.float64, device=self.device)
+        row = torch.empty(self.num_envs, dtype=torch.int32, device=self.device)
+        self._check(self._L.bskenv_get_env_params(self._h, C.c_void_p(p.data_ptr()), C.c_void_p(row.data_ptr()), self._stream()),
+                    "bskenv_get_env_params")
+        return {k: p[:, j] for j, k in enumerate(PARAM_KEYS)}, row
 
     def reset(self, seed=None, mask=None):
         """Sample fresh initial conditions on the device and return the initial observation [N,5]."""
@@ -289,6 +327,7 @@ class LeoPowerAttVecEnv:
 
 
 ORGANISATIONS = {"auto": 0, "thread": 1, "split": 2, "thread_index": 3}
+PARAM_ASSIGN = {"by_index": 0, "per_episode": 1}
 _FIELD_WIDTH = {"r_BN_N": 3, "v_BN_N": 3, "sigma_BN": 3, "omega_BN_B": 3, "Omega": 4, "u_current": 4,
                 "extTorquePntB_B": 3, "att_guidance": 12, "att_reference": 9, "commandedControlTorque": 3,
                 "rwTorqueCommand": 4, "wheelDeltaH": 3, "ThrustOnCmd": 8, "thrOnTimeRemaining": 8, "OnTimeRequest": 8,

@@ -116,6 +116,33 @@ int64_t bskenv_num_envs(const bskenv_handle *h);
 int bskenv_set_ephemeris(bskenv_handle *h, int kind, double t0, double seg_len, int n_seg, int n_coef, const double *coef);
 int bskenv_set_gravity_degree2(bskenv_handle *h, int enable, const double *cbar /* [5] or NULL */);
 
+/* Per-env spacecraft parameters (Monte Carlo dispersions, domain randomisation): in the reference every
+ * LEOPowerAttitudeSimulator is built from its own `initial_conditions` dict (simulators/leoPowerAttitudeSimulator.py:127-191);
+ * here a POOL of n_rows parameter sets is loaded into the handle and each env runs one row for a whole episode.  A row is
+ * BSKENV_PARAM_DIM doubles, the reference's keys and units in this order:
+ *   mass, width, depth, height, baseDensity, scaleHeight, disturbance_magnitude, panelArea, panelEfficiency, powerDraw,
+ *   storageCapacity, K, P, hs_min
+ * Everything else stays batch-global (bskenv_config).  The row is picked at reset -- bskenv_reset_seeded, bskenv_reset_ics
+ * and the in-kernel auto-reset; bskenv_reset_init keeps the env's row, as the reference rebuilds from the same dict:
+ *   BSKENV_PARAMS_BY_INDEX     row = (first_env_index + e) % n_rows  (n_rows = global env count: an explicit per-env table)
+ *   BSKENV_PARAMS_PER_EPISODE  row drawn from a counter-based stream keyed by (seed, global env index, episode), separate
+ *                              from the IC stream: the initial conditions are those of a run without a pool, and neither
+ *                              depends on the sharding.  `episode` is the env's episode counter after the reset.
+ * Loading a pool does not touch running envs until their next reset (envs that have not been reset under a pool run the
+ * batch configuration, row -1).  n_rows = 0 unloads the pool: new resets use the batch configuration and bskenv_step*
+ * returns to the batch-global kernels.  Each row is derived on the host exactly as bskenv_create derives the batch
+ * configuration.  BSKENV_EINVAL for a non-positive mass, dimension, scaleHeight or storageCapacity, a non-finite value, an
+ * unknown mode, and for configurations the per-env kernel is not built for: rw_set = 1, precision = 1, the degree-2 field
+ * (bskenv_set_gravity_degree2) and BSKENV_ORG_SPLIT (which bskenv_set_organisation refuses while a pool is loaded).  With
+ * a pool loaded, BSKENV_ORG_AUTO runs one thread per env at every batch size (kernel leo_step_penv_kernel). */
+#define BSKENV_PARAM_DIM 14
+#define BSKENV_PARAMS_BY_INDEX 0
+#define BSKENV_PARAMS_PER_EPISODE 1
+int bskenv_set_param_pool(bskenv_handle *h, int n_rows, const double *rows_host /* [n_rows][14] */, int assign);
+/* The parameters every env runs with, double[n][BSKENV_PARAM_DIM] row-major, and its pool row (int32[n], may be NULL;
+ * -1 = the batch configuration). */
+int bskenv_get_env_params(bskenv_handle *h, double *params_dev /* [n][14] */, int32_t *row_dev /* [n] or NULL */, void *stream);
+
 /* reset(): sample fresh initial conditions on the device (distributions and clipping of
  * initial_conditions/leo_orbit.py:25-39, sc_attitudes.py:3-13, simulators/...Simulator.py:152-167).
  * `mask_dev` (uint8[n], may be NULL = all) selects the envs to reset.  `obs_dev` (double[n*5], may be
