@@ -43,7 +43,7 @@ OPNAV_EXPORTS = ["bskenv_opnav_default_config", "bskenv_opnav_create", "bskenv_o
                  "bskenv_opnav_get_ics", "bskenv_opnav_step", "bskenv_opnav_step_host", "bskenv_opnav_state_dims",
                  "bskenv_opnav_get_state", "bskenv_opnav_set_state", "bskenv_opnav_state_field",
                  "bskenv_opnav_episode_stats", "bskenv_opnav_launch_count", "bskenv_opnav_flops_per_step",
-                 "bskenv_opnav_set_ephemeris", "bskenv_opnav_step_info"]
+                 "bskenv_opnav_set_ephemeris", "bskenv_opnav_step_info", "bskenv_opnav_set_ic_pool", "bskenv_opnav_get_ic_rows"]
 
 EXPORTS = ["bskenv_abi_version", "bskenv_default_config", "bskenv_create", "bskenv_destroy", "bskenv_last_error",
            "bskenv_num_envs", "bskenv_reset_seeded", "bskenv_reset_ics", "bskenv_reset_init", "bskenv_get_ics",
@@ -51,7 +51,8 @@ EXPORTS = ["bskenv_abi_version", "bskenv_default_config", "bskenv_create", "bske
            "bskenv_state_field", "bskenv_episode_stats", "bskenv_launch_count", "bskenv_fp64_peak",
            "bskenv_flops_per_step", "bskenv_set_ephemeris", "bskenv_set_gravity_degree2", "bskenv_step_info",
            "bskenv_step_host_async", "bskenv_step_host_wait", "bskenv_alloc_host", "bskenv_free_host", "bskenv_kernel_name",
-           "bskenv_set_organisation", "bskenv_set_param_pool", "bskenv_get_env_params"]
+           "bskenv_set_organisation", "bskenv_set_param_pool", "bskenv_get_env_params", "bskenv_set_ic_pool",
+           "bskenv_get_ic_rows"]
 
 
 def lib_path():
@@ -99,6 +100,8 @@ def lib():
     L.bskenv_set_organisation.argtypes = [vp, C.c_int]
     L.bskenv_set_param_pool.argtypes = [vp, C.c_int, vp, C.c_int]
     L.bskenv_get_env_params.argtypes = [vp, vp, vp, vp]
+    L.bskenv_set_ic_pool.argtypes = [vp, C.c_int, vp, C.c_int]
+    L.bskenv_get_ic_rows.argtypes = [vp, vp, vp]
     L.bskenv_fp64_peak.argtypes = [C.c_int, C.c_double, C.POINTER(C.c_double)]
     L.bskenv_flops_per_step.restype = C.c_double
     L.bskenv_flops_per_step.argtypes = [vp]
@@ -128,6 +131,8 @@ def lib():
     L.bskenv_opnav_flops_per_step.restype = C.c_double
     L.bskenv_opnav_flops_per_step.argtypes = [vp]
     L.bskenv_opnav_set_ephemeris.argtypes = [vp, C.c_double, C.c_double, C.c_int, C.c_int, vp]
+    L.bskenv_opnav_set_ic_pool.argtypes = [vp, C.c_int, vp, C.c_int]
+    L.bskenv_opnav_get_ic_rows.argtypes = [vp, vp, vp]
     if L.bskenv_abi_version() != 1:
         raise RuntimeError("libbskenv.so ABI version mismatch")
     _LIB = L

@@ -363,30 +363,40 @@ leo_split_kernel(const __grid_constant__ LeoParams P, double *__restrict__ S, in
 #endif
 }
 
-// mode 0: explicit ICs (row-major [n][19]); 1: stored ICs (reset_init); 2: device-sampled ICs.
-// With a parameter pool (pool.n_rows > 0) modes 0 and 2 assign the env's pool row; mode 1 keeps it.
+// mode 0: explicit ICs (row-major [n][19]); 1: stored ICs (reset_init); 2: device-sampled ICs, or a row of the IC pool.
+// With a parameter pool (pool.n_rows > 0) modes 0 and 2 assign the env's pool row; mode 1 keeps it.  Mode 2 is also the
+// auto-reset of a handle with an IC pool (launch_step: the step kernel runs without its in-kernel reset, then this kernel
+// with mask = done): the same sequence as step_finish -- episode + 1, ICs, parameter row, leo_reset_env, observation.
+// The parameter row is picked before the IC row, which BSKENV_ICS_PARAM_ROW takes from it.
 __global__ void __launch_bounds__(256)
 leo_reset_kernel(const __grid_constant__ LeoParams P, double *__restrict__ S, int64_t *__restrict__ I, double *__restrict__ ics,
                  int64_t stride, int64_t n, int mode, const double *__restrict__ ics_in, const uint8_t *__restrict__ mask,
-                 double *__restrict__ obs, const LeoPool pool)
+                 double *__restrict__ obs, const LeoPool pool, const IcPool icp)
 {
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n) return;
     if (mask && !mask[e]) return;
+    const int64_t ge = P.first_env_index + e;
+    int64_t ep = I[(int64_t)I_EPISODE * stride + e];
+    if (mode == 2) I[(int64_t)I_EPISODE * stride + e] = ++ep;
+    const int64_t prow = (pool.n_rows > 0 && mode != 1) ? leo::pool_row(pool, P.seed, ge, ep) : -1;
     double ic[19];
     if (mode == 0) {
         for (int k = 0; k < 19; k++) ic[k] = ics_in[e * 19 + k];
     } else if (mode == 1) {
         for (int k = 0; k < 19; k++) ic[k] = ics[(int64_t)k * stride + e];
+    } else if (icp.n_rows > 0) {
+        const int64_t r = leo::ic_pool_row(icp, P.seed, ge, ep, prow);
+        for (int k = 0; k < 19; k++) ic[k] = icp.rows[r * 19 + k];
+        icp.row_of[e] = (int32_t)r; icp.row_ep[e] = ep;
     } else {
-        int64_t ep = I[(int64_t)I_EPISODE * stride + e] + 1;
-        I[(int64_t)I_EPISODE * stride + e] = ep;
-        leo::sample_ic(P, P.first_env_index + e, ep, ic);
+        leo::sample_ic(P, ge, ep, ic);
     }
+    if (icp.row_of && mode != 1 && !(mode == 2 && icp.n_rows > 0)) { icp.row_of[e] = -1; icp.row_ep[e] = ep; }
     for (int k = 0; k < 19; k++) ics[(int64_t)k * stride + e] = ic[k];
     double ob[5];
     if (pool.n_rows > 0) {
-        if (mode != 1) leo::pool_assign(pool, S, stride, e, leo::pool_row(pool, P.seed, P.first_env_index + e, I[(int64_t)I_EPISODE * stride + e]));
+        if (mode != 1) leo::pool_assign(pool, S, stride, e, prow);
         leo::leo_reset_env<leo::ParEnv>(P, S, I, stride, e, ic, ob);
     } else {
         leo::leo_reset_env(P, S, I, stride, e, ic, ob);
@@ -412,6 +422,15 @@ __global__ void gather_ics_kernel(const double *__restrict__ ics, int64_t stride
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n) return;
     for (int k = 0; k < 19; k++) out[e * 19 + k] = ics[(int64_t)k * stride + e];
+}
+// bskenv_get_ic_rows: the recorded row where it belongs to the env's current episode (an in-kernel reset after an unload
+// advances the episode counter without touching the record)
+__global__ void gather_ic_rows_kernel(const int32_t *__restrict__ row_of, const int64_t *__restrict__ row_ep, const int64_t *__restrict__ ep,
+                                      int64_t n, int32_t *__restrict__ out)
+{
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    out[e] = row_ep[e] == ep[e] ? row_of[e] : -1;
 }
 // dense [fields][n] <-> padded [fields][stride]
 template <typename T>
@@ -464,6 +483,7 @@ struct bskenv_handle {
     int organisation;           // BSKENV_ORG_*: 0 auto, 1 one thread per env, 2 two warps per env group (small batches)
     LeoPool pool;               // loaded parameter pool (n_rows = 0: none); rows in device memory
     int s_fields;               // double fields allocated per env in S: LEO_ND, or LEO_ND + LEO_NPD once a pool was loaded
+    IcPool icp;                 // loaded initial-condition pool (n_rows = 0: none); rows and per-env record in device memory
     std::string err;
 };
 
@@ -488,9 +508,29 @@ static cudaError_t note_launch(bskenv_handle *h, cudaStream_t st)
         if ((h)->host_pending) { (h)->err = what ": a host-buffer step is in flight (call bskenv_step_host_wait first)"; return BSKENV_EINVAL; } \
     } while (0)
 
+// Auto-reset of a handle with an IC pool: after the step kernel (which ran without its in-kernel reset), the reset kernel in
+// its sampling mode over the envs the step finished -- mask = the step's `done`, obs = the step's `obs` (the terminal
+// observation there is replaced by the first one of the new episode; term_obs, the episode record and the statistics were
+// written by the step kernel before, exactly as before an in-kernel reset).  On the host-buffer paths both are the buffers
+// the step kernel wrote: mapped caller memory or the staging blocks, which are copied back after this launch.
+static int launch_follow_reset(bskenv_handle *h, const uint8_t *done, double *obs, cudaStream_t st)
+{
+    leo_reset_kernel<<<(int)((h->n + 255) / 256), 256, 0, st>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, 2, nullptr, done, obs,
+                                                                h->pool, h->icp);
+    CU_TRY(h, cudaGetLastError());
+    h->launches++;
+    return BSKENV_OK;
+}
+
 static int launch_step(bskenv_handle *h, const int32_t *act, double *obs, double *rew, uint8_t *done, uint8_t *reason,
                        double *term_obs, cudaStream_t st, double *ep_return = nullptr, int64_t *ep_length = nullptr)
 {
+    // With an IC pool the step kernels run on a copy of the parameter block without auto_reset (read only by step_finish) and
+    // launch_follow_reset does the reset: every organisation and configuration, the step kernels as they are.
+    const bool follow = h->icp.n_rows > 0 && h->P.auto_reset;
+    LeoParams P_nr;
+    if (follow) { P_nr = h->P; P_nr.auto_reset = 0; }
+    const LeoParams &PK = follow ? P_nr : h->P;
     const int wpb = LEO_BLOCK / 32;
     const int64_t groups = (h->n + LEO_LANES - 1) / LEO_LANES;
     const int resident = h->sm_count * LEO_MIN_BLOCKS;          // blocks of one full resident set
@@ -530,15 +570,16 @@ static int launch_step(bskenv_handle *h, const int32_t *act, double *obs, double
         }
         if (which == 0) {
             h->kernel_name = "leo_split_kernel<3,0,true>";
-            leo_split_kernel<3, 0, true><<<dgrid, 64 * G, smem, st>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, act, obs, rew, done, reason, term_obs,
+            leo_split_kernel<3, 0, true><<<dgrid, 64 * G, smem, st>>>(PK, h->S, h->I, h->ics, h->stride, h->n, act, obs, rew, done, reason, term_obs,
                                                                  h->stats, (int)groups, sc.n_chunks, ep_return, ep_length);
         } else {
             h->kernel_name = "leo_split_kernel<4,1,false>";
-            leo_split_kernel<4, 1, false><<<dgrid, 64 * G, smem, st>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, act, obs, rew, done, reason, term_obs,
+            leo_split_kernel<4, 1, false><<<dgrid, 64 * G, smem, st>>>(PK, h->S, h->I, h->ics, h->stride, h->n, act, obs, rew, done, reason, term_obs,
                                                                   h->stats, (int)groups, sc.n_chunks, ep_return, ep_length);
         }
         CU_TRY(h, cudaGetLastError());
         h->launches++;
+        if (follow) { const int rc = launch_follow_reset(h, done, obs, st); if (rc) return rc; }
         if (st != h->own_stream || !st) CU_TRY(h, note_launch(h, st));
         return BSKENV_OK;
     }
@@ -561,7 +602,7 @@ static int launch_step(bskenv_handle *h, const int32_t *act, double *obs, double
             attr_set[h->device & 63] = true;                                                                   \
         }                                                                                                      \
         h->kernel_name = "leo_step_kernel<" #NRW "," #J2 "," #DIAG "," #F32 "," LEO_STR(MINB) ">";              \
-        leo_step_kernel<NRW, J2, DIAG, F32, MINB><<<grid, LEO_BLOCK, bus_bytes, st>>>(h->P, h->PF, h->S, h->I, h->ics, h->stride, h->n, act, obs, \
+        leo_step_kernel<NRW, J2, DIAG, F32, MINB><<<grid, LEO_BLOCK, bus_bytes, st>>>(PK, h->PF, h->S, h->I, h->ics, h->stride, h->n, act, obs, \
                                                                                  rew, done, reason, term_obs, h->stats, sc, ep_return, ep_length); \
     } while (0)
 #define LEO_LAUNCH(NRW, J2, DIAG, F32) LEO_LAUNCH_B(NRW, J2, DIAG, F32, LEO_MIN_BLOCKS)
@@ -573,7 +614,7 @@ static int launch_step(bskenv_handle *h, const int32_t *act, double *obs, double
             attr_set[h->device & 63] = true;                                                                   \
         }                                                                                                      \
         h->kernel_name = "leo_step_penv_kernel<3," #J2 ",true," LEO_STR(LEO_MIN_BLOCKS) ">";                    \
-        leo_step_penv_kernel<3, J2, true, LEO_MIN_BLOCKS><<<grid, LEO_BLOCK, LEO_BUS_BYTES_PENV, st>>>(h->P, h->pool, h->S, h->I, h->ics, \
+        leo_step_penv_kernel<3, J2, true, LEO_MIN_BLOCKS><<<grid, LEO_BLOCK, LEO_BUS_BYTES_PENV, st>>>(PK, h->pool, h->S, h->I, h->ics, \
             h->stride, h->n, act, obs, rew, done, reason, term_obs, h->stats, sc, ep_return, ep_length);        \
     } while (0)
     if (penv) { if (h->cfg.use_j2) LEO_LAUNCH_PENV(1); else LEO_LAUNCH_PENV(0); }    // (bskenv_set_param_pool checks the configuration)
@@ -598,6 +639,7 @@ static int launch_step(bskenv_handle *h, const int32_t *act, double *obs, double
 #undef LEO_LAUNCH_PENV
     CU_TRY(h, cudaGetLastError());
     h->launches++;
+    if (follow) { const int rc = launch_follow_reset(h, done, obs, st); if (rc) return rc; }
     if (st != h->own_stream || !st) CU_TRY(h, note_launch(h, st));
     return BSKENV_OK;
 }
@@ -645,6 +687,7 @@ int bskenv_create(const bskenv_config *cfg, int device, int64_t n_envs, int64_t 
     h->S = h->ics = h->stats = nullptr; h->I = nullptr; h->sched = nullptr; h->perm = nullptr; h->bucket = nullptr;
     h->d_eph[0] = h->d_eph[1] = nullptr;
     h->pool.rows = nullptr; h->pool.n_rows = 0; h->pool.assign = 0; h->s_fields = LEO_ND;
+    h->icp.rows = nullptr; h->icp.row_of = nullptr; h->icp.row_ep = nullptr; h->icp.n_rows = 0; h->icp.assign = 0;
     for (int k = 0; k < 8; k++) { h->h_stage[k] = nullptr; h->pend_user[k] = nullptr; h->pend_bytes[k] = 0; }
     h->host_pending = 0; h->own_stream = nullptr; h->ev_last = nullptr; h->ev_valid = 0;
     cudaError_t e = cudaSetDevice(device);
@@ -676,6 +719,7 @@ int bskenv_destroy(bskenv_handle *h)
     cudaSetDevice(h->device);
     cudaFree(h->S); cudaFree(h->I); cudaFree(h->ics); cudaFree(h->stats); cudaFree(h->sched); cudaFree(h->perm); cudaFree(h->bucket);
     cudaFree(h->d_eph[0]); cudaFree(h->d_eph[1]); cudaFree((void *)h->pool.rows);
+    cudaFree((void *)h->icp.rows); cudaFree(h->icp.row_of); cudaFree(h->icp.row_ep);
     if (h->own_stream) { cudaStreamSynchronize(h->own_stream); cudaStreamDestroy(h->own_stream); }
     for (int k = 0; k < 8; k++) cudaFreeHost(h->h_stage[k]);
     if (h->ev_last) cudaEventDestroy(h->ev_last);
@@ -721,6 +765,11 @@ int bskenv_set_param_pool(bskenv_handle *h, int n_rows, const double *rows_host,
     if (!h) return BSKENV_EINVAL;
     NO_HOST_PENDING(h, "bskenv_set_param_pool");
     if (n_rows < 0 || (n_rows > 0 && !rows_host)) { h->err = "bskenv_set_param_pool: bad row count or null rows"; return BSKENV_EINVAL; }
+    if (h->icp.n_rows > 0 && h->icp.assign == BSKENV_ICS_PARAM_ROW && n_rows != h->icp.n_rows) {
+        h->err = "bskenv_set_param_pool: an IC pool of " + std::to_string(h->icp.n_rows) +
+                 " rows is paired with the parameter pool (BSKENV_ICS_PARAM_ROW): unload it before changing the row count or unloading";
+        return BSKENV_EINVAL;
+    }
     if (n_rows > 0) {
         if (assign != BSKENV_PARAMS_BY_INDEX && assign != BSKENV_PARAMS_PER_EPISODE) { h->err = "bskenv_set_param_pool: unknown assignment mode"; return BSKENV_EINVAL; }
         if (h->P.nrw != 3 || !h->P.diag) { h->err = "bskenv_set_param_pool: per-env parameters are built for the three-wheel reference spacecraft (rw_set = 0)"; return BSKENV_EINVAL; }
@@ -776,13 +825,62 @@ int bskenv_get_env_params(bskenv_handle *h, double *params_dev, int32_t *row_dev
     return BSKENV_OK;
 }
 
+int bskenv_set_ic_pool(bskenv_handle *h, int n_rows, const double *ics_host, int assign)
+{
+    if (!h) return BSKENV_EINVAL;
+    NO_HOST_PENDING(h, "bskenv_set_ic_pool");
+    if (n_rows < 0 || (n_rows > 0 && !ics_host)) { h->err = "bskenv_set_ic_pool: bad row count or null rows"; return BSKENV_EINVAL; }
+    if (n_rows > 0) {
+        if (assign != BSKENV_ICS_BY_INDEX && assign != BSKENV_ICS_PER_EPISODE && assign != BSKENV_ICS_PARAM_ROW) {
+            h->err = "bskenv_set_ic_pool: unknown assignment mode"; return BSKENV_EINVAL;
+        }
+        if (assign == BSKENV_ICS_PARAM_ROW && h->pool.n_rows != n_rows) {
+            h->err = "bskenv_set_ic_pool: BSKENV_ICS_PARAM_ROW needs a loaded parameter pool of the same row count (" +
+                     std::to_string(n_rows) + " IC rows, " + std::to_string(h->pool.n_rows) + " parameter rows)";
+            return BSKENV_EINVAL;
+        }
+        for (int r = 0; r < n_rows; r++) {
+            const std::string err = leo_host::ic_row_check(ics_host + (size_t)r * BSKENV_IC_DIM, BSKENV_IC_DIM);
+            if (!err.empty()) { h->err = "bskenv_set_ic_pool: row " + std::to_string(r) + ": " + err; return BSKENV_EINVAL; }
+        }
+    }
+    CU_TRY(h, cudaSetDevice(h->device));
+    CU_TRY(h, cudaDeviceSynchronize());                         // a launch in flight may still read the old pool
+    cudaFree((void *)h->icp.rows);
+    h->icp.rows = nullptr; h->icp.n_rows = 0;
+    if (n_rows == 0) return BSKENV_OK;                          // unloaded: resets sample again, the in-kernel auto-reset
+    if (!h->icp.row_of) {                                       // first pool of this handle: the per-env record, all -1
+        CU_TRY(h, cudaMalloc(&h->icp.row_of, sizeof(int32_t) * h->stride));
+        CU_TRY(h, cudaMalloc(&h->icp.row_ep, sizeof(int64_t) * h->stride));
+        CU_TRY(h, cudaMemset(h->icp.row_of, 0xFF, sizeof(int32_t) * h->stride));
+        CU_TRY(h, cudaMemset(h->icp.row_ep, 0, sizeof(int64_t) * h->stride));
+    }
+    double *d_rows = nullptr;
+    const size_t bytes = sizeof(double) * (size_t)n_rows * BSKENV_IC_DIM;
+    CU_TRY(h, cudaMalloc(&d_rows, bytes));
+    CU_TRY(h, cudaMemcpy(d_rows, ics_host, bytes, cudaMemcpyHostToDevice));
+    h->icp.rows = d_rows; h->icp.n_rows = n_rows; h->icp.assign = assign;
+    return BSKENV_OK;
+}
+
+int bskenv_get_ic_rows(bskenv_handle *h, int32_t *rows_dev, void *stream)
+{
+    if (!h || !rows_dev) { if (h) h->err = "bskenv_get_ic_rows: null rows"; return BSKENV_EINVAL; }
+    CU_TRY(h, cudaSetDevice(h->device));
+    if (!h->icp.row_of) CU_TRY(h, cudaMemsetAsync(rows_dev, 0xFF, sizeof(int32_t) * h->n, (cudaStream_t)stream));
+    else gather_ic_rows_kernel<<<(int)((h->n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->icp.row_of, h->icp.row_ep,
+                                                                                             h->I + (size_t)I_EPISODE * h->stride, h->n, rows_dev);
+    CU_TRY(h, cudaGetLastError());
+    return BSKENV_OK;
+}
+
 static int do_reset(bskenv_handle *h, int mode, const double *ics_in, const uint8_t *mask, double *obs, void *stream)
 {
     if (!h) return BSKENV_EINVAL;
     NO_HOST_PENDING(h, "bskenv_reset");
     CU_TRY(h, cudaSetDevice(h->device));
     const int grid = (int)((h->n + 255) / 256);
-    leo_reset_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, mode, ics_in, mask, obs, h->pool);
+    leo_reset_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, mode, ics_in, mask, obs, h->pool, h->icp);
     CU_TRY(h, cudaGetLastError());
     CU_TRY(h, note_launch(h, (cudaStream_t)stream));
     return BSKENV_OK;

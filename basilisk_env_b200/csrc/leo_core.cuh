@@ -943,6 +943,23 @@ LEO_HD void pool_assign(const LeoPool &pool, double *S, int64_t stride, int64_t 
     for (int f = 0; f < LEO_NPD; f++) S[(int64_t)(LEO_ND + f) * stride + e] = pool.rows[(int64_t)f * pool.n_rows + row];
 }
 
+// Initial-condition pool row of an env at a reset (LEO and opNav).  BY_INDEX: global env index mod n_rows.  PARAM_ROW: the
+// env's parameter-pool row of the same reset.  PER_EPISODE: one Philox4x32-10 block keyed like the IC stream, (seed, global
+// env, episode), at counter word 0xFFFFFFFE.  No other stream reaches that word: the IC samplers use blocks 0, 1, ... (a few
+// dozen at most), the parameter pool 0xFFFFFFFF, and the opNav noise streams (stream << 16 | block) with stream 1 or 2 and
+// block < 4 -- those run under the key seed_hi ^ episode, which is the IC key at episode 0, so only the counter word keeps
+// them apart, and it does.  The ICs a run samples, its parameter rows and its noise are therefore those of a run without an
+// IC pool, and none of them depends on the sharding.
+LEO_HD int64_t ic_pool_row(const IcPool &pool, uint64_t seed, int64_t global_env, int64_t episode, int64_t param_row)
+{
+    if (pool.assign == IC_POOL_BY_INDEX) return global_env % pool.n_rows;
+    if (pool.assign == IC_POOL_PARAM_ROW) return param_row;
+    uint32_t o[4];
+    philox4x32((uint32_t)global_env, (uint32_t)((uint64_t)global_env >> 32), (uint32_t)episode, 0xFFFFFFFEu, (uint32_t)seed,
+               (uint32_t)(seed >> 32), o);
+    return (int64_t)((((uint64_t)o[1] << 32) | o[0]) % (uint64_t)pool.n_rows);
+}
+
 LEO_HD_NOINLINE void sun_latch_to_bus(const LeoParams &P, MBus m, int64_t msg_ns)
 {
     SunLatch s = sun_latch(P, msg_ns);

@@ -219,6 +219,16 @@ static inline std::string param_row_build(const bskenv_config &base, const doubl
     return "";
 }
 
+// Checks one initial-condition pool row of `dim` doubles whose first three are the position rN (LEO: BSKENV_IC_DIM, opNav:
+// BSKENV_OPNAV_IC_DIM); returns "" or an error message.
+static inline std::string ic_row_check(const double *row, int dim)
+{
+    for (int k = 0; k < dim; k++)
+        if (!isfinite(row[k])) return "non-finite value in column " + std::to_string(k);
+    if (row[0] == 0.0 && row[1] == 0.0 && row[2] == 0.0) return "zero position vector rN";
+    return "";
+}
+
 // SURVEY 8(f)-4: normalised degree-2 coefficients (C20, C21, S21, C22, S22; the form gravity-model files carry and
 // Basilisk's loadGravFromFile reads) -> mu Req^2 [M] of the closed-form gradient used by the kernel.
 // Un-normalisation: C_nm = Cbar_nm sqrt((2 - delta_0m)(2n + 1)(n - m)!/(n + m)!).

@@ -166,6 +166,13 @@ enum LeoPField : int {
 #define LEO_POOL_BY_INDEX 0      // row = global env index mod n_rows           (BSKENV_PARAMS_BY_INDEX)
 #define LEO_POOL_PER_EPISODE 1   // row drawn per (seed, global env, episode)   (BSKENV_PARAMS_PER_EPISODE)
 struct LeoPool { const double *rows; int32_t n_rows, assign; };
+// Loaded initial-condition pool (LEO and opNav): rows row-major [n_rows][dim]; row_of[e] = the row env e's current episode
+// started from (-1: sampled or explicit ICs) and row_ep[e] the episode counter it was recorded at (the in-kernel reset of a
+// handle without a pool does not touch either); both allocated at the first load and kept after an unload.
+#define IC_POOL_BY_INDEX 0       // row = global env index mod n_rows           (BSKENV_ICS_BY_INDEX)
+#define IC_POOL_PER_EPISODE 1    // row drawn per (seed, global env, episode)   (BSKENV_ICS_PER_EPISODE)
+#define IC_POOL_PARAM_ROW 2      // row = the env's parameter-pool row          (BSKENV_ICS_PARAM_ROW)
+struct IcPool { const double *rows; int32_t *row_of; int64_t *row_ep; int32_t n_rows, assign; };
 
 #define LEO_TASK_SUN 1
 #define LEO_TASK_NADIR 2

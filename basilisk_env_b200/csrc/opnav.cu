@@ -265,30 +265,46 @@ opnav_pass2_kernel(const __grid_constant__ OpNavParams P, double *__restrict__ S
     }
 }
 
-// mode 0: explicit ICs (row-major [n][12]); 1: stored ICs; 2: device-sampled ICs
+// mode 0: explicit ICs (row-major [n][12]); 1: stored ICs; 2: device-sampled ICs, or a row of the IC pool.  Mode 2 is also
+// the auto-reset of a handle with an IC pool (opnav_launch_step: after the last kernel of the interval, mask = done), the
+// same sequence as the in-kernel reset of opnav_pass2_kernel.
 __global__ void __launch_bounds__(256)
 opnav_reset_kernel(const __grid_constant__ OpNavParams P, double *__restrict__ S, int64_t *__restrict__ I, double *__restrict__ ics,
                    int64_t stride, int64_t n, int mode, const double *__restrict__ ics_in, const uint8_t *__restrict__ mask,
-                   double *__restrict__ obs)
+                   double *__restrict__ obs, const IcPool icp)
 {
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n) return;
     if (mask && !mask[e]) return;
+    int64_t ep = I[(int64_t)OI_EPISODE * stride + e];
     double ic[OPNAV_IC_DIM];
     if (mode == 0) {
         for (int k = 0; k < OPNAV_IC_DIM; k++) ic[k] = ics_in[e * OPNAV_IC_DIM + k];
     } else if (mode == 1) {
         for (int k = 0; k < OPNAV_IC_DIM; k++) ic[k] = ics[(int64_t)k * stride + e];
     } else {
-        int64_t ep = I[(int64_t)OI_EPISODE * stride + e] + 1;
-        I[(int64_t)OI_EPISODE * stride + e] = ep;
-        opnav::sample_ic(P, P.first_env_index + e, ep, ic);
+        I[(int64_t)OI_EPISODE * stride + e] = ++ep;
+        if (icp.n_rows > 0) {
+            const int64_t r = leo::ic_pool_row(icp, P.seed, P.first_env_index + e, ep, -1);
+            for (int k = 0; k < OPNAV_IC_DIM; k++) ic[k] = icp.rows[r * OPNAV_IC_DIM + k];
+            icp.row_of[e] = (int32_t)r; icp.row_ep[e] = ep;
+        } else {
+            opnav::sample_ic(P, P.first_env_index + e, ep, ic);
+        }
     }
+    if (icp.row_of && mode != 1 && !(mode == 2 && icp.n_rows > 0)) { icp.row_of[e] = -1; icp.row_ep[e] = ep; }
     for (int k = 0; k < OPNAV_IC_DIM; k++) ics[(int64_t)k * stride + e] = ic[k];
     double ob[4];
     opnav::opnav_reset_env(P, S, I, stride, e, ic, ob);
     if (obs)
         for (int k = 0; k < 4; k++) obs[e * 4 + k] = ob[k];
+}
+__global__ void opnav_gather_ic_rows_kernel(const int32_t *__restrict__ row_of, const int64_t *__restrict__ row_ep,
+                                            const int64_t *__restrict__ ep, int64_t n, int32_t *__restrict__ out)
+{
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    out[e] = row_ep[e] == ep[e] ? row_of[e] : -1;      // as bskenv.cu: gather_ic_rows_kernel
 }
 __global__ void opnav_gather_ics_kernel(const double *__restrict__ ics, int64_t stride, int64_t n, double *__restrict__ out)
 {
@@ -328,6 +344,7 @@ struct bskenv_opnav_handle {
     cudaEvent_t ev_last;        // recorded after every launch queued through the device-buffer entry points
     int ev_valid;
     int64_t launches;
+    IcPool icp;                 // loaded initial-condition pool (n_rows = 0: none), as in the LEO handle
     std::string err;
 };
 
@@ -344,6 +361,12 @@ static int opnav_launch_step(bskenv_opnav_handle *h, const int32_t *act, double 
                              uint8_t *reason, double *debug, double *term_obs, cudaStream_t st, double *ep_return = nullptr,
                              int64_t *ep_length = nullptr)
 {
+    // With an IC pool the second pass runs without its in-kernel reset (auto_reset is read nowhere else) and the reset kernel
+    // follows the interval, as in bskenv.cu: launch_follow_reset.
+    const bool follow = h->icp.n_rows > 0 && h->P.auto_reset;
+    OpNavParams P_nr;
+    if (follow) { P_nr = h->P; P_nr.auto_reset = 0; }
+    const OpNavParams &PK = follow ? P_nr : h->P;
     const int wpb = ON_BLOCK / 32;
     const int64_t groups = (h->n + 31) / 32;
     // First pass (noise + dynamics): 255 registers / two blocks per SM or 168 registers (with spills) / three; measured per full
@@ -413,13 +436,18 @@ static int opnav_launch_step(bskenv_opnav_handle *h, const int32_t *act, double 
     else if (minb1 == 3) opnav_pass1_kernel<3><<<grid1, ON_BLOCK, smem_a, st>>>(h->P, h->S, h->I, h->stride, h->n, act, s1, h->perm, h->mbuf);
     else opnav_pass1_kernel<2><<<grid1, ON_BLOCK, smem_a, st>>>(h->P, h->S, h->I, h->stride, h->n, act, s1, h->perm, h->mbuf);
     if (minb2 == 3)
-        opnav_pass2_kernel<3><<<grid2, ON_BLOCK, smem_b, st>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, act, obs, rew, done, reason, debug,
+        opnav_pass2_kernel<3><<<grid2, ON_BLOCK, smem_b, st>>>(PK, h->S, h->I, h->ics, h->stride, h->n, act, obs, rew, done, reason, debug,
                                                           term_obs, h->stats, s2, h->perm, ep_return, ep_length, h->mbuf);
     else
-        opnav_pass2_kernel<2><<<grid2, ON_BLOCK, smem_b, st>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, act, obs, rew, done, reason, debug,
+        opnav_pass2_kernel<2><<<grid2, ON_BLOCK, smem_b, st>>>(PK, h->S, h->I, h->ics, h->stride, h->n, act, obs, rew, done, reason, debug,
                                                           term_obs, h->stats, s2, h->perm, ep_return, ep_length, h->mbuf);
     ON_TRY(h, cudaGetLastError());
     h->launches += 2;
+    if (follow) {           // obs / done: the buffers the second pass wrote (device, mapped host or staging memory)
+        opnav_reset_kernel<<<(int)((h->n + 255) / 256), 256, 0, st>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, 2, nullptr, done, obs, h->icp);
+        ON_TRY(h, cudaGetLastError());
+        h->launches++;
+    }
     if (st != h->own_stream || !st) { h->ev_valid = 1; ON_TRY(h, cudaEventRecord(h->ev_last, st)); }
     return BSKENV_OK;
 }
@@ -451,6 +479,7 @@ int bskenv_opnav_create(const bskenv_opnav_config *cfg, int device, int64_t n_en
     h->device = device; h->n = n_envs; h->stride = (n_envs + 31) / 32 * 32; h->launches = 0;
     h->S = h->ics = h->stats = nullptr; h->I = nullptr; h->sched = nullptr; h->perm = nullptr; h->d_eph = nullptr; h->mbuf = nullptr; h->nzbuf = nullptr; h->noise_split = -1;
     for (int k = 0; k < 6; k++) h->h_stage[k] = nullptr;
+    h->icp.rows = nullptr; h->icp.row_of = nullptr; h->icp.row_ep = nullptr; h->icp.n_rows = 0; h->icp.assign = 0;
     h->own_stream = nullptr; h->ev_last = nullptr; h->ev_valid = 0;
     cudaError_t e = cudaSetDevice(device);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->ev_last, cudaEventDisableTiming);
@@ -484,6 +513,7 @@ int bskenv_opnav_destroy(bskenv_opnav_handle *h)
     if (!h) return BSKENV_OK;
     cudaSetDevice(h->device);
     cudaFree(h->S); cudaFree(h->I); cudaFree(h->ics); cudaFree(h->stats); cudaFree(h->sched); cudaFree(h->perm); cudaFree(h->d_eph); cudaFree(h->mbuf); cudaFree(h->nzbuf);
+    cudaFree((void *)h->icp.rows); cudaFree(h->icp.row_of); cudaFree(h->icp.row_ep);
     if (h->own_stream) { cudaStreamSynchronize(h->own_stream); cudaStreamDestroy(h->own_stream); }
     for (int k = 0; k < 6; k++) cudaFreeHost(h->h_stage[k]);
     if (h->ev_last) cudaEventDestroy(h->ev_last);
@@ -518,7 +548,7 @@ static int opnav_do_reset(bskenv_opnav_handle *h, int mode, const double *ics_in
     if (!h) return BSKENV_EINVAL;
     ON_TRY(h, cudaSetDevice(h->device));
     const int grid = (int)((h->n + 255) / 256);
-    opnav_reset_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, mode, ics_in, mask, obs);
+    opnav_reset_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, mode, ics_in, mask, obs, h->icp);
     ON_TRY(h, cudaGetLastError());
     h->ev_valid = 1; ON_TRY(h, cudaEventRecord(h->ev_last, (cudaStream_t)stream));
     return BSKENV_OK;
@@ -543,6 +573,50 @@ int bskenv_opnav_get_ics(bskenv_opnav_handle *h, double *ics_dev, void *stream)
     if (!h || !ics_dev) return BSKENV_EINVAL;
     ON_TRY(h, cudaSetDevice(h->device));
     opnav_gather_ics_kernel<<<(int)((h->n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->ics, h->stride, h->n, ics_dev);
+    ON_TRY(h, cudaGetLastError());
+    return BSKENV_OK;
+}
+
+int bskenv_opnav_set_ic_pool(bskenv_opnav_handle *h, int n_rows, const double *ics_host, int assign)
+{
+    if (!h) return BSKENV_EINVAL;
+    if (n_rows < 0 || (n_rows > 0 && !ics_host)) { h->err = "bskenv_opnav_set_ic_pool: bad row count or null rows"; return BSKENV_EINVAL; }
+    if (n_rows > 0) {
+        if (assign != BSKENV_ICS_BY_INDEX && assign != BSKENV_ICS_PER_EPISODE) {
+            h->err = "bskenv_opnav_set_ic_pool: unknown assignment mode (the opNav batch has no parameter pool to pair with)";
+            return BSKENV_EINVAL;
+        }
+        for (int r = 0; r < n_rows; r++) {
+            const std::string err = leo_host::ic_row_check(ics_host + (size_t)r * BSKENV_OPNAV_IC_DIM, BSKENV_OPNAV_IC_DIM);
+            if (!err.empty()) { h->err = "bskenv_opnav_set_ic_pool: row " + std::to_string(r) + ": " + err; return BSKENV_EINVAL; }
+        }
+    }
+    ON_TRY(h, cudaSetDevice(h->device));
+    ON_TRY(h, cudaDeviceSynchronize());                         // a launch in flight may still read the old pool
+    cudaFree((void *)h->icp.rows);
+    h->icp.rows = nullptr; h->icp.n_rows = 0;
+    if (n_rows == 0) return BSKENV_OK;
+    if (!h->icp.row_of) {
+        ON_TRY(h, cudaMalloc(&h->icp.row_of, sizeof(int32_t) * h->stride));
+        ON_TRY(h, cudaMalloc(&h->icp.row_ep, sizeof(int64_t) * h->stride));
+        ON_TRY(h, cudaMemset(h->icp.row_of, 0xFF, sizeof(int32_t) * h->stride));
+        ON_TRY(h, cudaMemset(h->icp.row_ep, 0, sizeof(int64_t) * h->stride));
+    }
+    double *d_rows = nullptr;
+    const size_t bytes = sizeof(double) * (size_t)n_rows * BSKENV_OPNAV_IC_DIM;
+    ON_TRY(h, cudaMalloc(&d_rows, bytes));
+    ON_TRY(h, cudaMemcpy(d_rows, ics_host, bytes, cudaMemcpyHostToDevice));
+    h->icp.rows = d_rows; h->icp.n_rows = n_rows; h->icp.assign = assign;
+    return BSKENV_OK;
+}
+
+int bskenv_opnav_get_ic_rows(bskenv_opnav_handle *h, int32_t *rows_dev, void *stream)
+{
+    if (!h || !rows_dev) { if (h) h->err = "bskenv_opnav_get_ic_rows: null rows"; return BSKENV_EINVAL; }
+    ON_TRY(h, cudaSetDevice(h->device));
+    if (!h->icp.row_of) ON_TRY(h, cudaMemsetAsync(rows_dev, 0xFF, sizeof(int32_t) * h->n, (cudaStream_t)stream));
+    else opnav_gather_ic_rows_kernel<<<(int)((h->n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->icp.row_of, h->icp.row_ep,
+                                                                                                  h->I + (size_t)OI_EPISODE * h->stride, h->n, rows_dev);
     ON_TRY(h, cudaGetLastError());
     return BSKENV_OK;
 }

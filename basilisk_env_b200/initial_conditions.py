@@ -148,6 +148,33 @@ PARAM_KEYS = ("mass", "width", "depth", "height", "baseDensity", "scaleHeight", 
               "panelEfficiency", "powerDraw", "storageCapacity", "K", "P", "hs_min")
 
 
+def scenario_rows(scenarios, config):
+    """A scenario table from full reference `initial_conditions` dicts (the shape `set_ICs()` returns): (IC rows [K, 19],
+    parameter rows [K, 14] in PARAM_KEYS order) for `LeoPowerAttVecEnv.set_scenario_pool`.
+    config : the batch's configuration, a mapping of CONFIG_KEYS -> value; a PARAM_KEYS entry a dict leaves out takes its
+        value from here.  A batch-global key (CONFIG_KEYS minus PARAM_KEYS) must equal it: ValueError names the key and the
+        scenario index otherwise."""
+    scenarios = list(scenarios)
+    if not scenarios:
+        raise ValueError("a scenario pool needs at least one scenario")
+    ics, params = [], []
+    for j, ic in enumerate(scenarios):
+        for k in CONFIG_KEYS:
+            if k in PARAM_KEYS or ic.get(k) is None:
+                continue
+            want = np.ravel(np.asarray(config[k], dtype=np.float64))
+            got = np.ravel(np.asarray(ic[k], dtype=np.float64))
+            if got.shape != want.shape or not np.array_equal(got, want):
+                raise ValueError(f"scenario {j}: {k!r} = {got.tolist()} differs from the batch configuration {want.tolist()} "
+                                 "(only the parameter-pool keys initial_conditions.PARAM_KEYS may differ per env)")
+        axes = ic.get("controlAxes_B")
+        if axes is not None and list(np.ravel(axes)) != [1, 0, 0, 0, 1, 0, 0, 0, 1]:
+            raise ValueError(f"scenario {j}: controlAxes_B other than the identity is not on the reference path")
+        ics.append(ic_row(ic))
+        params.append([float(ic[k]) if ic.get(k) is not None else float(config[k]) for k in PARAM_KEYS])
+    return np.stack(ics), np.asarray(params, dtype=np.float64)
+
+
 def config_overrides(ic):
     """bskenv_config overrides carried by an `initial_conditions` dict."""
     out = {}

@@ -131,6 +131,27 @@ class OpNavVecEnv:
         self._check(self._L.bskenv_opnav_set_ephemeris(self._h, float(table.t0), float(table.seg_len), coef.shape[0],
                                                        coef.shape[2], coef.ctypes.data), "set_ephemeris")
 
+    def set_ic_pool(self, ics, assign="per_episode"):
+        """Load a pool of initial conditions [K, 12] (rN vN rError vError) that `reset()` and the auto-reset of `step` draw
+        from instead of the built-in sampler (include/bskenv.h: bskenv_opnav_set_ic_pool); None unloads it.
+        assign : "per_episode" (row drawn per (seed, global env index, episode)) or "by_index" (global env index mod K)."""
+        if ics is None:
+            self._check(self._L.bskenv_opnav_set_ic_pool(self._h, 0, None, 0), "bskenv_opnav_set_ic_pool")
+            return
+        rows = ics.detach().cpu().numpy() if torch.is_tensor(ics) else ics
+        rows = np.ascontiguousarray(rows, dtype=np.float64)
+        if rows.ndim != 2 or rows.shape[1] != IC_DIM or rows.shape[0] == 0:
+            raise ValueError(f"ics must have shape (K, {IC_DIM}) with K > 0")
+        self._check(self._L.bskenv_opnav_set_ic_pool(self._h, rows.shape[0], rows.ctypes.data, IC_ASSIGN[assign]),
+                    "bskenv_opnav_set_ic_pool")
+
+    def ic_rows(self):
+        """The IC-pool row each env's current episode started from (int32 [N]; -1 = sampled or explicit ICs)."""
+        row = torch.empty(self.num_envs, dtype=torch.int32, device=self.device)
+        self._check(self._L.bskenv_opnav_get_ic_rows(self._h, C.c_void_p(row.data_ptr()), self._stream()),
+                    "bskenv_opnav_get_ic_rows")
+        return row
+
     def reset(self, seed=None, mask=None):
         """Sample fresh initial conditions on the device; returns the initial observation [N,4] (zeros)."""
         if seed is not None:
@@ -245,6 +266,7 @@ class OpNavVecEnv:
         return float(self._L.bskenv_opnav_flops_per_step(self._h))
 
 
+IC_ASSIGN = {"by_index": 0, "per_episode": 1}
 _FIELD_WIDTH = {"r_BN_N": 3, "v_BN_N": 3, "sigma_BN": 3, "omega_BN_B": 3, "Omega": 4, "reactionwheel_cmds": 4,
                 "navErrors": 15, "sun_point_data": 3, "filter_state": 6, "filter_sBar": 21, "sim_obs": 4, "sim_states": 12}
 

@@ -11,7 +11,7 @@ import torch
 
 from . import _native
 from . import spaces
-from .initial_conditions import PARAM_KEYS
+from .initial_conditions import CONFIG_KEYS, PARAM_KEYS, ic_row, scenario_rows
 
 DONE_MAXLEN, DONE_WHEEL, DONE_POWER, DONE_DECAY = 1, 2, 4, 8
 OBS_DIM, IC_DIM = 5, 19
@@ -175,6 +175,48 @@ class LeoPowerAttVecEnv:
                     "bskenv_get_env_params")
         return {k: p[:, j] for j, k in enumerate(PARAM_KEYS)}, row
 
+    def set_ic_pool(self, ics, assign="per_episode"):
+        """Load a pool of initial conditions that resets draw from instead of the built-in sampler -- `reset()` and the
+        auto-reset of `step` alike (include/bskenv.h: bskenv_set_ic_pool).
+        ics : array or tensor [K, 19] (see initial_conditions.ic_row), a sequence of reference `initial_conditions` dicts, or
+            None to unload the pool.
+        assign : "per_episode" (row drawn per (seed, global env index, episode)), "by_index" (row = global env index mod K)
+            or "param_row" (row = the env's parameter-pool row: a scenario table, see `set_scenario_pool`)."""
+        if ics is None:
+            self._check(self._L.bskenv_set_ic_pool(self._h, 0, None, 0), "bskenv_set_ic_pool")
+            return
+        if torch.is_tensor(ics):
+            rows = ics.detach().cpu().numpy()
+        elif len(ics) and isinstance(ics[0], dict):
+            rows = np.stack([ic_row(ic) for ic in ics])
+        else:
+            rows = ics
+        rows = np.ascontiguousarray(rows, dtype=np.float64)
+        if rows.ndim != 2 or rows.shape[1] != IC_DIM or rows.shape[0] == 0:
+            raise ValueError(f"ics must have shape (K, {IC_DIM}) with K > 0")
+        self._check(self._L.bskenv_set_ic_pool(self._h, rows.shape[0], rows.ctypes.data, IC_ASSIGN[assign]), "bskenv_set_ic_pool")
+
+    def ic_rows(self):
+        """The IC-pool row each env's current episode started from (int32 [N]; -1 = sampled or explicit ICs)."""
+        row = torch.empty(self.num_envs, dtype=torch.int32, device=self.device)
+        self._check(self._L.bskenv_get_ic_rows(self._h, C.c_void_p(row.data_ptr()), self._stream()), "bskenv_get_ic_rows")
+        return row
+
+    def set_scenario_pool(self, scenarios, assign="per_episode"):
+        """Load K full reference `initial_conditions` dicts (the shape `initial_conditions.set_ICs()` returns) as a scenario
+        table: their PARAM_KEYS become the parameter pool (assigned by `assign`), their initial conditions an IC pool paired
+        with it ("param_row"), so that every episode runs one (initial conditions, parameters) pair -- the batched form of
+        K reference simulators, each built from its own dict.  A batch-global key that differs from this handle's
+        configuration raises ValueError.  None unloads both pools."""
+        self.set_ic_pool(None)
+        if scenarios is None:
+            self.set_param_pool(None)
+            return
+        config = {k: list(getattr(self.cfg, k)) if k in ("nHat_B", "sigma_R0N") else getattr(self.cfg, k) for k in CONFIG_KEYS}
+        ics, params = scenario_rows(scenarios, config)
+        self.set_param_pool(params, assign=assign)
+        self.set_ic_pool(ics, assign="param_row")
+
     def reset(self, seed=None, mask=None):
         """Sample fresh initial conditions on the device and return the initial observation [N,5]."""
         if seed is not None:
@@ -328,6 +370,7 @@ class LeoPowerAttVecEnv:
 
 ORGANISATIONS = {"auto": 0, "thread": 1, "split": 2, "thread_index": 3}
 PARAM_ASSIGN = {"by_index": 0, "per_episode": 1}
+IC_ASSIGN = {"by_index": 0, "per_episode": 1, "param_row": 2}
 _FIELD_WIDTH = {"r_BN_N": 3, "v_BN_N": 3, "sigma_BN": 3, "omega_BN_B": 3, "Omega": 4, "u_current": 4,
                 "extTorquePntB_B": 3, "att_guidance": 12, "att_reference": 9, "commandedControlTorque": 3,
                 "rwTorqueCommand": 4, "wheelDeltaH": 3, "ThrustOnCmd": 8, "thrOnTimeRemaining": 8, "OnTimeRequest": 8,

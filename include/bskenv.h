@@ -143,6 +143,35 @@ int bskenv_set_param_pool(bskenv_handle *h, int n_rows, const double *rows_host 
  * -1 = the batch configuration). */
 int bskenv_get_env_params(bskenv_handle *h, double *params_dev /* [n][14] */, int32_t *row_dev /* [n] or NULL */, void *stream);
 
+/* Per-episode initial conditions from a pool (Monte Carlo campaigns over dispersed start states, curricula, replayed failure
+ * cases, fixed evaluation sets): the second half of the reference's `initial_conditions` dict, the state an episode starts
+ * from.  n_rows rows of BSKENV_IC_DIM doubles, the layout of bskenv_reset_ics, are loaded into the handle (device memory);
+ * resets that sample -- bskenv_reset_seeded and the auto-reset of bskenv_step* -- take a pool row instead of the built-in
+ * sampler.  The row of each reset:
+ *   BSKENV_ICS_BY_INDEX     row = (first_env_index + e) % n_rows
+ *   BSKENV_ICS_PER_EPISODE  row drawn from a counter-based stream keyed by (seed, global env index, episode), separate from the
+ *                           IC sampler, the parameter pool and the opNav noise streams: those are the draws of a run without
+ *                           an IC pool, and nothing depends on the sharding.  `episode` is the counter after the reset.
+ *   BSKENV_ICS_PARAM_ROW    row = the env's parameter-pool row of the same reset (LEO only): with a parameter pool of the same
+ *                           n_rows the two pools are one scenario table of (initial conditions, parameters) pairs.
+ * bskenv_reset_ics uses its explicit rows and records row -1; bskenv_reset_init replays the stored ICs and keeps the row;
+ * bskenv_get_ics reports the pool values an env started from.  Loading a pool does not touch running envs until their next
+ * reset; n_rows = 0 unloads it (new resets sample again and bskenv_step* returns to the in-kernel auto-reset).  With a pool and
+ * auto_reset, bskenv_step* launches the step kernel without its in-kernel reset and then the reset kernel over the envs that
+ * finished (mask = done): one more launch per step (bskenv_launch_count; bskenv_kernel_name still names the step kernel),
+ * every organisation and configuration, the same results as bskenv_reset_seeded with mask = done after a step without
+ * auto_reset.  BSKENV_EINVAL for a non-finite value or a zero position vector (the message names the row), an unknown mode,
+ * BSKENV_ICS_PARAM_ROW without a loaded parameter pool of the same n_rows, and -- while such a paired pool is loaded --
+ * bskenv_set_param_pool with another row count or an unload.  Refused while a host-buffer step is in flight.
+ * bskenv_get_ic_rows: the pool row each env's current episode started from (int32[n], device memory); -1 = sampled or
+ * explicit ICs, or a reset before the pool was loaded.  The row is not part of the state (bskenv_state_dims, get_state /
+ * set_state): a checkpoint does not carry it. */
+#define BSKENV_ICS_BY_INDEX 0
+#define BSKENV_ICS_PER_EPISODE 1
+#define BSKENV_ICS_PARAM_ROW 2
+int bskenv_set_ic_pool(bskenv_handle *h, int n_rows, const double *ics_host /* [n_rows][19] */, int assign);
+int bskenv_get_ic_rows(bskenv_handle *h, int32_t *rows_dev /* [n] */, void *stream);
+
 /* reset(): sample fresh initial conditions on the device (distributions and clipping of
  * initial_conditions/leo_orbit.py:25-39, sc_attitudes.py:3-13, simulators/...Simulator.py:152-167).
  * `mask_dev` (uint8[n], may be NULL = all) selects the envs to reset.  `obs_dev` (double[n*5], may be
@@ -299,6 +328,11 @@ int bskenv_opnav_reset_ics(bskenv_opnav_handle *h, const double *ics_dev /* [n*1
                            double *obs_dev, void *stream);
 int bskenv_opnav_reset_init(bskenv_opnav_handle *h, const uint8_t *mask_dev, double *obs_dev, void *stream);
 int bskenv_opnav_get_ics(bskenv_opnav_handle *h, double *ics_dev, void *stream);
+/* Initial-condition pool of the opNav batch: rows of BSKENV_OPNAV_IC_DIM doubles (rN vN rError vError), BSKENV_ICS_BY_INDEX or
+ * BSKENV_ICS_PER_EPISODE; semantics, refusals and the extra launch of the step as bskenv_set_ic_pool / bskenv_get_ic_rows
+ * (the auto-reset runs after the last kernel of the interval, in the two-kernel and the three-kernel form). */
+int bskenv_opnav_set_ic_pool(bskenv_opnav_handle *h, int n_rows, const double *ics_host /* [n_rows][12] */, int assign);
+int bskenv_opnav_get_ic_rows(bskenv_opnav_handle *h, int32_t *rows_dev /* [n] */, void *stream);
 /* step(): ONE call = one decision interval for every env (two kernels: noise walk + dynamics / flight software, then the
  * filter; three -- the noise walk in a kernel of its own, feeding the dynamics through a device buffer of 120 B per env-tick,
  * allocated at the first step -- when the environment variable BSKENV_OPNAV_NOISE_SPLIT=1 is set at that time and the buffer
