@@ -4,6 +4,7 @@ There is deliberately no fallback: if the library is missing or no CUDA device i
 product path raises."""
 import ctypes as C
 import os
+import types
 
 from . import build as _build
 
@@ -38,6 +39,9 @@ class OpNavConfig(C.Structure):
                 ("noise_seed", C.c_uint64), ("reserved", C.c_int32 * 8)]
 
 
+# C ABI prefix of each batch -> its configuration struct
+BATCHES = {"bskenv_": Config, "bskenv_opnav_": OpNavConfig}
+
 OPNAV_EXPORTS = ["bskenv_opnav_default_config", "bskenv_opnav_create", "bskenv_opnav_destroy", "bskenv_opnav_last_error",
                  "bskenv_opnav_num_envs", "bskenv_opnav_reset_seeded", "bskenv_opnav_reset_ics", "bskenv_opnav_reset_init",
                  "bskenv_opnav_get_ics", "bskenv_opnav_step", "bskenv_opnav_step_host", "bskenv_opnav_state_dims",
@@ -55,6 +59,24 @@ EXPORTS = ["bskenv_abi_version", "bskenv_default_config", "bskenv_create", "bske
            "bskenv_get_ic_rows"]
 
 
+def _shared_signatures(cfg):
+    """(restype, argtypes) of the entry points both batches export under their prefix; cfg = the batch's config struct."""
+    vp, i64, u64, i32, ci = C.c_void_p, C.c_int64, C.c_uint64, C.c_int32, C.c_int
+    return {"default_config": (None, [C.POINTER(cfg)]), "create": (ci, [C.POINTER(cfg), ci, i64, i64, C.POINTER(vp)]),
+            "destroy": (ci, [vp]), "last_error": (C.c_char_p, [vp]), "num_envs": (i64, [vp]),
+            "reset_seeded": (ci, [vp, u64, vp, vp, vp]), "reset_ics": (ci, [vp] * 5), "reset_init": (ci, [vp] * 4),
+            "get_ics": (ci, [vp] * 3), "state_dims": (ci, [vp, C.POINTER(i32), C.POINTER(i32)]),
+            "get_state": (ci, [vp] * 4), "set_state": (ci, [vp] * 4), "state_field": (ci, [C.c_char_p, C.POINTER(i32)]),
+            "episode_stats": (ci, [vp, vp]), "launch_count": (i64, [vp]), "flops_per_step": (C.c_double, [vp]),
+            "set_ic_pool": (ci, [vp, ci, vp, ci]), "get_ic_rows": (ci, [vp] * 3)}
+
+
+def batch_abi(prefix):
+    """The shared entry points of one batch ("bskenv_" or "bskenv_opnav_"), by their names without the prefix."""
+    L = lib()
+    return types.SimpleNamespace(**{name: getattr(L, prefix + name) for name in _shared_signatures(Config)})
+
+
 def lib_path():
     return _build.LIB
 
@@ -68,110 +90,68 @@ def lib():
         raise RuntimeError(f"{path} is missing: run `python -c 'import __graft_entry__ as g; g.build()'` "
                            "(there is no CPU fallback for the environment step)")
     L = C.CDLL(path)
-    vp, i64, u64, i32 = C.c_void_p, C.c_int64, C.c_uint64, C.c_int32
-    L.bskenv_abi_version.restype = C.c_int
-    L.bskenv_default_config.argtypes = [C.POINTER(Config)]
-    L.bskenv_create.argtypes = [C.POINTER(Config), C.c_int, i64, i64, C.POINTER(vp)]
-    L.bskenv_destroy.argtypes = [vp]
-    L.bskenv_last_error.restype = C.c_char_p
-    L.bskenv_last_error.argtypes = [vp]
-    L.bskenv_num_envs.restype = i64
-    L.bskenv_num_envs.argtypes = [vp]
-    L.bskenv_reset_seeded.argtypes = [vp, u64, vp, vp, vp]
-    L.bskenv_reset_ics.argtypes = [vp, vp, vp, vp, vp]
-    L.bskenv_reset_init.argtypes = [vp, vp, vp, vp]
-    L.bskenv_get_ics.argtypes = [vp, vp, vp]
-    L.bskenv_step.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp]
-    L.bskenv_step_host.argtypes = [vp, vp, vp, vp, vp, vp]
+    vp, ci = C.c_void_p, C.c_int
+    for prefix, cfg in BATCHES.items():
+        for name, (res, args) in _shared_signatures(cfg).items():
+            f = getattr(L, prefix + name)
+            f.restype, f.argtypes = res, args
+    L.bskenv_abi_version.restype = ci
+    L.bskenv_step.argtypes = [vp] * 8
+    L.bskenv_step_host.argtypes = [vp] * 6
     L.bskenv_step_info.argtypes = [vp] * 10
     L.bskenv_step_host_async.argtypes = [vp] * 9
     L.bskenv_step_host_wait.argtypes = [vp]
     L.bskenv_alloc_host.argtypes = [C.c_size_t, C.POINTER(vp)]
     L.bskenv_free_host.argtypes = [vp]
-    L.bskenv_state_dims.argtypes = [vp, C.POINTER(i32), C.POINTER(i32)]
-    L.bskenv_get_state.argtypes = [vp, vp, vp, vp]
-    L.bskenv_set_state.argtypes = [vp, vp, vp, vp]
-    L.bskenv_state_field.argtypes = [C.c_char_p, C.POINTER(i32)]
-    L.bskenv_episode_stats.argtypes = [vp, vp]
-    L.bskenv_launch_count.restype = i64
-    L.bskenv_launch_count.argtypes = [vp]
     L.bskenv_kernel_name.restype = C.c_char_p
     L.bskenv_kernel_name.argtypes = [vp]
-    L.bskenv_set_organisation.argtypes = [vp, C.c_int]
-    L.bskenv_set_param_pool.argtypes = [vp, C.c_int, vp, C.c_int]
+    L.bskenv_set_organisation.argtypes = [vp, ci]
+    L.bskenv_set_param_pool.argtypes = [vp, ci, vp, ci]
     L.bskenv_get_env_params.argtypes = [vp, vp, vp, vp]
-    L.bskenv_set_ic_pool.argtypes = [vp, C.c_int, vp, C.c_int]
-    L.bskenv_get_ic_rows.argtypes = [vp, vp, vp]
-    L.bskenv_fp64_peak.argtypes = [C.c_int, C.c_double, C.POINTER(C.c_double)]
-    L.bskenv_flops_per_step.restype = C.c_double
-    L.bskenv_flops_per_step.argtypes = [vp]
-    L.bskenv_set_ephemeris.argtypes = [vp, C.c_int, C.c_double, C.c_double, C.c_int, C.c_int, vp]
-    L.bskenv_set_gravity_degree2.argtypes = [vp, C.c_int, vp]
-    L.bskenv_opnav_default_config.argtypes = [C.POINTER(OpNavConfig)]
-    L.bskenv_opnav_create.argtypes = [C.POINTER(OpNavConfig), C.c_int, i64, i64, C.POINTER(vp)]
-    L.bskenv_opnav_destroy.argtypes = [vp]
-    L.bskenv_opnav_last_error.restype = C.c_char_p
-    L.bskenv_opnav_last_error.argtypes = [vp]
-    L.bskenv_opnav_num_envs.restype = i64
-    L.bskenv_opnav_num_envs.argtypes = [vp]
-    L.bskenv_opnav_reset_seeded.argtypes = [vp, u64, vp, vp, vp]
-    L.bskenv_opnav_reset_ics.argtypes = [vp, vp, vp, vp, vp]
-    L.bskenv_opnav_reset_init.argtypes = [vp, vp, vp, vp]
-    L.bskenv_opnav_get_ics.argtypes = [vp, vp, vp]
+    L.bskenv_fp64_peak.argtypes = [ci, C.c_double, C.POINTER(C.c_double)]
+    L.bskenv_set_ephemeris.argtypes = [vp, ci, C.c_double, C.c_double, ci, ci, vp]
+    L.bskenv_set_gravity_degree2.argtypes = [vp, ci, vp]
     L.bskenv_opnav_step.argtypes = [vp] * 9
     L.bskenv_opnav_step_host.argtypes = [vp] * 7
     L.bskenv_opnav_step_info.argtypes = [vp] * 11
-    L.bskenv_opnav_state_dims.argtypes = [vp, C.POINTER(i32), C.POINTER(i32)]
-    L.bskenv_opnav_get_state.argtypes = [vp, vp, vp, vp]
-    L.bskenv_opnav_set_state.argtypes = [vp, vp, vp, vp]
-    L.bskenv_opnav_state_field.argtypes = [C.c_char_p, C.POINTER(i32)]
-    L.bskenv_opnav_episode_stats.argtypes = [vp, vp]
-    L.bskenv_opnav_launch_count.restype = i64
-    L.bskenv_opnav_launch_count.argtypes = [vp]
-    L.bskenv_opnav_flops_per_step.restype = C.c_double
-    L.bskenv_opnav_flops_per_step.argtypes = [vp]
-    L.bskenv_opnav_set_ephemeris.argtypes = [vp, C.c_double, C.c_double, C.c_int, C.c_int, vp]
-    L.bskenv_opnav_set_ic_pool.argtypes = [vp, C.c_int, vp, C.c_int]
-    L.bskenv_opnav_get_ic_rows.argtypes = [vp, vp, vp]
+    L.bskenv_opnav_set_ephemeris.argtypes = [vp, C.c_double, C.c_double, ci, ci, vp]
     if L.bskenv_abi_version() != 1:
         raise RuntimeError("libbskenv.so ABI version mismatch")
     _LIB = L
     return L
 
 
-def default_config(**overrides):
-    cfg = Config()
-    lib().bskenv_default_config(C.byref(cfg))
+def batch_config(prefix, **overrides):
+    cfg = BATCHES[prefix]()
+    getattr(lib(), prefix + "default_config")(C.byref(cfg))
     for k, v in overrides.items():
         if not hasattr(cfg, k):
-            raise AttributeError(f"bskenv_config has no field {k!r}")
+            raise AttributeError(f"{prefix}config has no field {k!r}")
         if isinstance(v, (list, tuple)):
             v = (C.c_double * len(v))(*v)
         setattr(cfg, k, v)
     return cfg
 
 
-def state_field(name):
+def batch_state_field(prefix, name):
     is_int = C.c_int32(0)
-    idx = lib().bskenv_state_field(name.encode(), C.byref(is_int))
+    idx = getattr(lib(), prefix + "state_field")(name.encode(), C.byref(is_int))
     if idx < 0:
         raise KeyError(name)
     return idx, bool(is_int.value)
+
+
+def default_config(**overrides):
+    return batch_config("bskenv_", **overrides)
+
+
+def state_field(name):
+    return batch_state_field("bskenv_", name)
 
 
 def opnav_default_config(**overrides):
-    cfg = OpNavConfig()
-    lib().bskenv_opnav_default_config(C.byref(cfg))
-    for k, v in overrides.items():
-        if not hasattr(cfg, k):
-            raise AttributeError(f"bskenv_opnav_config has no field {k!r}")
-        setattr(cfg, k, v)
-    return cfg
+    return batch_config("bskenv_opnav_", **overrides)
 
 
 def opnav_state_field(name):
-    is_int = C.c_int32(0)
-    idx = lib().bskenv_opnav_state_field(name.encode(), C.byref(is_int))
-    if idx < 0:
-        raise KeyError(name)
-    return idx, bool(is_int.value)
+    return batch_state_field("bskenv_opnav_", name)

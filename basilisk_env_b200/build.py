@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.environ.get("BSKENV_LIB") or os.path.join(HERE, "libbskenv.so")   # BSKENV_LIB: load a tuning variant instead
 SOURCES = ["bskenv.cu", "opnav.cu"]
-DEPS = ["bskenv.cu", "leo_core.cuh", "leo_split.cuh", "leo_f32.cuh", "leo_params.h", "leo_host.h", "opnav.cu",
+DEPS = ["bskenv.cu", "batch_common.cuh", "leo_core.cuh", "leo_split.cuh", "leo_f32.cuh", "leo_params.h", "leo_host.h", "opnav.cu",
         "opnav_core.cuh", "opnav_params.h", "opnav_host.h", os.path.join("..", "..", "include", "bskenv.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC"]
 

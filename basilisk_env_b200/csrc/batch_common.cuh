@@ -1,0 +1,286 @@
+// batch_common.cuh -- the handle layer the LEO batch (bskenv.cu) and the opNav batch (opnav.cu) share: the handle core,
+// the IC choice of a reset, and the entry points around the step kernels that differ only in dimensions (create / destroy,
+// ephemeris tables, IC pools, stored ICs, state blocks, statistics, host-buffer mapping, launch ordering).
+#pragma once
+#include <cuda_runtime.h>
+#include <string.h>
+#include <string>
+
+#include "../../include/bskenv.h"
+#include "leo_core.cuh"
+#include "leo_host.h"
+
+#define CU_TRY(h, call)                                                                              \
+    do {                                                                                             \
+        cudaError_t _e = (call);                                                                     \
+        if (_e != cudaSuccess) {                                                                     \
+            (h)->err = std::string(#call) + ": " + cudaGetErrorString(_e);                            \
+            return BSKENV_ECUDA;                                                                     \
+        }                                                                                            \
+    } while (0)
+
+// What every batch handle holds; bskenv_handle and bskenv_opnav_handle derive from it.
+struct BatchCore {
+    int device = 0;
+    int64_t n = 0, stride = 0;  // envs, and the column pitch of the state blocks (n rounded up to whole warps)
+    double *S = nullptr, *ics = nullptr, *stats = nullptr;
+    int64_t *I = nullptr;
+    int sm_count = 0;
+    void *h_stage[8] = {};      // page-locked staging of the host-buffer entry points, one per buffer slot (pageable caller buffers)
+    int host_pending = 0;       // a host-buffer step was queued and not waited for (LEO's bskenv_step_host_async; 0 for opNav)
+    cudaStream_t own_stream = nullptr;  // the stream of the host-buffer entry points
+    cudaEvent_t ev_last = nullptr;      // recorded after every launch queued through the device-buffer entry points
+    int ev_valid = 0;
+    int64_t launches = 0;
+    IcPool icp{};               // loaded initial-condition pool (n_rows = 0: none); rows and per-env record in device memory
+    std::string err;
+};
+
+namespace {
+
+__device__ __forceinline__ double warp_sum(double v)
+{
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+    return v;
+}
+
+// The initial conditions of a reset, stored into `ics`.  mode 0: explicit ICs (row-major [n][DIM]); 1: the stored ones
+// (reset_init); 2: a row of the IC pool when one is loaded (row picked with the parameter row `prow` of this reset, -1 without
+// one), else sample(ic).  The IC-pool record of the env becomes the drawn row, or -1 after explicit or sampled ICs; mode 1
+// keeps it.  ep = the env's episode after the reset.
+template <int DIM, class Sample>
+__device__ __forceinline__ void reset_ics(int mode, const double *__restrict__ ics_in, double *__restrict__ ics, int64_t stride,
+                                          int64_t e, int64_t global_env, uint64_t seed, int64_t ep, int64_t prow, const IcPool &icp,
+                                          Sample sample, double (&ic)[DIM])
+{
+    if (mode == 0) {
+        for (int k = 0; k < DIM; k++) ic[k] = ics_in[e * DIM + k];
+    } else if (mode == 1) {
+        for (int k = 0; k < DIM; k++) ic[k] = ics[(int64_t)k * stride + e];
+    } else if (icp.n_rows > 0) {
+        const int64_t r = leo::ic_pool_row(icp, seed, global_env, ep, prow);
+        for (int k = 0; k < DIM; k++) ic[k] = icp.rows[r * DIM + k];
+        icp.row_of[e] = (int32_t)r; icp.row_ep[e] = ep;
+    } else {
+        sample(ic);
+    }
+    if (icp.row_of && mode != 1 && !(mode == 2 && icp.n_rows > 0)) { icp.row_of[e] = -1; icp.row_ep[e] = ep; }
+    for (int k = 0; k < DIM; k++) ics[(int64_t)k * stride + e] = ic[k];
+}
+
+template <int DIM>
+__global__ void gather_ics_kernel(const double *__restrict__ ics, int64_t stride, int64_t n, double *__restrict__ out)
+{
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    for (int k = 0; k < DIM; k++) out[e * DIM + k] = ics[(int64_t)k * stride + e];
+}
+// get_ic_rows: the recorded row where it belongs to the env's current episode (an in-kernel reset after an unload advances
+// the episode counter without touching the record)
+__global__ void gather_ic_rows_kernel(const int32_t *__restrict__ row_of, const int64_t *__restrict__ row_ep, const int64_t *__restrict__ ep,
+                                      int64_t n, int32_t *__restrict__ out)
+{
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    out[e] = row_ep[e] == ep[e] ? row_of[e] : -1;
+}
+// dense [fields][n] <-> padded [fields][stride]
+template <typename T>
+__global__ void copy_fields_kernel(const T *__restrict__ src, int64_t src_stride, T *__restrict__ dst, int64_t dst_stride,
+                                   int64_t n, int fields)
+{
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n) return;
+    for (int f = 0; f < fields; f++) dst[(int64_t)f * dst_stride + e] = src[(int64_t)f * src_stride + e];
+}
+
+inline int env_grid(const BatchCore *h) { return (int)((h->n + 255) / 256); }
+
+// Launches queued on the caller's streams are ordered before a later host-buffer step (which runs on the handle's own
+// stream) through this event.
+inline cudaError_t note_launch(BatchCore *h, cudaStream_t st)
+{
+    h->ev_valid = 1;
+    return cudaEventRecord(h->ev_last, st);
+}
+
+// The checks of a create call before the handle exists; the message goes to `err`, the calling thread's create error.
+inline int check_create(const char *what, bool args_ok, int device, std::string &err)
+{
+    if (!args_ok) { err = std::string(what) + ": bad arguments"; return BSKENV_EINVAL; }
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
+        cudaGetLastError();
+        err = std::string(what) + ": no CUDA device (this library has no CPU path)";
+        return BSKENV_ENODEV;
+    }
+    if (device < 0 || device >= ndev) { err = std::string(what) + ": device index out of range"; return BSKENV_EINVAL; }
+    return BSKENV_OK;
+}
+
+// The allocations every handle makes: the ordering event, the zeroed state blocks S [nd][stride] and I [ni][stride], the
+// stored ICs [ic_dim][stride] and the n_stats episode statistics.
+inline cudaError_t core_alloc(BatchCore *h, int device, int64_t n_envs, int nd, int ni, int ic_dim, int n_stats)
+{
+    h->device = device; h->n = n_envs; h->stride = (n_envs + 31) / 32 * 32;
+    cudaError_t e = cudaSetDevice(device);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->ev_last, cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&h->sm_count, cudaDevAttrMultiProcessorCount, device);
+    if (e == cudaSuccess) e = cudaMalloc(&h->S, sizeof(double) * nd * h->stride);
+    if (e == cudaSuccess) e = cudaMalloc(&h->I, sizeof(int64_t) * ni * h->stride);
+    if (e == cudaSuccess) e = cudaMalloc(&h->ics, sizeof(double) * ic_dim * h->stride);
+    if (e == cudaSuccess) e = cudaMalloc(&h->stats, sizeof(double) * n_stats);
+    if (e == cudaSuccess) e = cudaMemset(h->S, 0, sizeof(double) * nd * h->stride);
+    if (e == cudaSuccess) e = cudaMemset(h->I, 0, sizeof(int64_t) * ni * h->stride);
+    if (e == cudaSuccess) e = cudaMemset(h->ics, 0, sizeof(double) * ic_dim * h->stride);
+    if (e == cudaSuccess) e = cudaMemset(h->stats, 0, sizeof(double) * n_stats);
+    return e;
+}
+
+// Frees what core_alloc and the shared entry points allocated (the current device is the handle's)
+inline void core_free(BatchCore *h)
+{
+    cudaFree(h->S); cudaFree(h->I); cudaFree(h->ics); cudaFree(h->stats);
+    cudaFree((void *)h->icp.rows); cudaFree(h->icp.row_of); cudaFree(h->icp.row_ep);
+    if (h->own_stream) { cudaStreamSynchronize(h->own_stream); cudaStreamDestroy(h->own_stream); }
+    for (void *p : h->h_stage) cudaFreeHost(p);
+    if (h->ev_last) cudaEventDestroy(h->ev_last);
+}
+
+// Loads a Chebyshev ephemeris table into E (n_seg <= 0: none, back to the analytic model).  The table has to cover one
+// episode, sim time 0 to t_end.  E.coef is the device copy.
+inline int set_ephemeris(BatchCore *h, const char *what, LeoEph &E, double t_end, double t0, double seg_len, int n_seg, int n_coef,
+                         const double *coef)
+{
+    CU_TRY(h, cudaSetDevice(h->device));
+    CU_TRY(h, cudaDeviceSynchronize());                         // a launch in flight may still read the old table
+    cudaFree((void *)E.coef);
+    E.coef = nullptr; E.nseg = 0; E.ncoef = 0; E.t0 = 0.; E.seg_len = 0.;
+    if (n_seg <= 0) return BSKENV_OK;
+    if (!coef || n_coef < 1 || n_coef > 64 || !(seg_len > 0.)) { h->err = std::string(what) + ": bad table shape"; return BSKENV_EINVAL; }
+    if (t0 > 0. || t0 + seg_len * n_seg < t_end) {
+        h->err = std::string(what) + ": the table does not cover one episode [0, (max_length + 1) * step_duration]";
+        return BSKENV_EINVAL;
+    }
+    const size_t bytes = sizeof(double) * (size_t)n_seg * 3 * (size_t)n_coef;
+    double *d = nullptr;
+    CU_TRY(h, cudaMalloc(&d, bytes));
+    E.coef = d;
+    CU_TRY(h, cudaMemcpy(d, coef, bytes, cudaMemcpyHostToDevice));
+    E.nseg = n_seg; E.ncoef = n_coef; E.t0 = t0; E.seg_len = seg_len;
+    return BSKENV_OK;
+}
+
+// Loads n_rows IC rows of dim numbers each (n_rows = 0 unloads the pool: resets sample again, the in-kernel auto-reset).
+// mode_error(): the batch's refusal of `assign` ("" = accepted), checked after the arguments and before the rows.
+template <class ModeError>
+int set_ic_pool(BatchCore *h, const char *what, int n_rows, const double *rows_host, int dim, int assign, ModeError mode_error)
+{
+    if (n_rows < 0 || (n_rows > 0 && !rows_host)) { h->err = std::string(what) + ": bad row count or null rows"; return BSKENV_EINVAL; }
+    if (n_rows > 0) {
+        const std::string merr = mode_error();
+        if (!merr.empty()) { h->err = merr; return BSKENV_EINVAL; }
+        for (int r = 0; r < n_rows; r++) {
+            const std::string err = leo_host::ic_row_check(rows_host + (size_t)r * dim, dim);
+            if (!err.empty()) { h->err = std::string(what) + ": row " + std::to_string(r) + ": " + err; return BSKENV_EINVAL; }
+        }
+    }
+    CU_TRY(h, cudaSetDevice(h->device));
+    CU_TRY(h, cudaDeviceSynchronize());                         // a launch in flight may still read the old pool
+    cudaFree((void *)h->icp.rows);
+    h->icp.rows = nullptr; h->icp.n_rows = 0;
+    if (n_rows == 0) return BSKENV_OK;
+    if (!h->icp.row_of) {                                       // first pool of this handle: the per-env record, all -1
+        CU_TRY(h, cudaMalloc(&h->icp.row_of, sizeof(int32_t) * h->stride));
+        CU_TRY(h, cudaMalloc(&h->icp.row_ep, sizeof(int64_t) * h->stride));
+        CU_TRY(h, cudaMemset(h->icp.row_of, 0xFF, sizeof(int32_t) * h->stride));
+        CU_TRY(h, cudaMemset(h->icp.row_ep, 0, sizeof(int64_t) * h->stride));
+    }
+    double *d_rows = nullptr;
+    const size_t bytes = sizeof(double) * (size_t)n_rows * dim;
+    CU_TRY(h, cudaMalloc(&d_rows, bytes));
+    CU_TRY(h, cudaMemcpy(d_rows, rows_host, bytes, cudaMemcpyHostToDevice));
+    h->icp.rows = d_rows; h->icp.n_rows = n_rows; h->icp.assign = assign;
+    return BSKENV_OK;
+}
+
+// ep_field: the episode counter's field in I
+inline int get_ic_rows(BatchCore *h, const char *what, int ep_field, int32_t *rows_dev, void *stream)
+{
+    if (!rows_dev) { h->err = std::string(what) + ": null rows"; return BSKENV_EINVAL; }
+    CU_TRY(h, cudaSetDevice(h->device));
+    if (!h->icp.row_of) CU_TRY(h, cudaMemsetAsync(rows_dev, 0xFF, sizeof(int32_t) * h->n, (cudaStream_t)stream));
+    else gather_ic_rows_kernel<<<env_grid(h), 256, 0, (cudaStream_t)stream>>>(h->icp.row_of, h->icp.row_ep,
+                                                                              h->I + (size_t)ep_field * h->stride, h->n, rows_dev);
+    CU_TRY(h, cudaGetLastError());
+    return BSKENV_OK;
+}
+
+template <int DIM>
+int get_ics(BatchCore *h, double *ics_dev, void *stream)
+{
+    if (!ics_dev) return BSKENV_EINVAL;
+    CU_TRY(h, cudaSetDevice(h->device));
+    gather_ics_kernel<DIM><<<env_grid(h), 256, 0, (cudaStream_t)stream>>>(h->ics, h->stride, h->n, ics_dev);
+    CU_TRY(h, cudaGetLastError());
+    return BSKENV_OK;
+}
+
+// The persistent state as dense [nd][n] doubles and [ni][n] integers (either may be null)
+inline int get_state(BatchCore *h, int nd, int ni, double *dstate_dev, int64_t *istate_dev, void *stream)
+{
+    CU_TRY(h, cudaSetDevice(h->device));
+    if (dstate_dev) copy_fields_kernel<double><<<env_grid(h), 256, 0, (cudaStream_t)stream>>>(h->S, h->stride, dstate_dev, h->n, h->n, nd);
+    if (istate_dev) copy_fields_kernel<int64_t><<<env_grid(h), 256, 0, (cudaStream_t)stream>>>(h->I, h->stride, istate_dev, h->n, h->n, ni);
+    CU_TRY(h, cudaGetLastError());
+    return BSKENV_OK;
+}
+inline int set_state(BatchCore *h, int nd, int ni, const double *dstate_dev, const int64_t *istate_dev, void *stream)
+{
+    CU_TRY(h, cudaSetDevice(h->device));
+    if (dstate_dev) copy_fields_kernel<double><<<env_grid(h), 256, 0, (cudaStream_t)stream>>>(dstate_dev, h->n, h->S, h->stride, h->n, nd);
+    if (istate_dev) copy_fields_kernel<int64_t><<<env_grid(h), 256, 0, (cudaStream_t)stream>>>(istate_dev, h->n, h->I, h->stride, h->n, ni);
+    CU_TRY(h, cudaGetLastError());
+    CU_TRY(h, note_launch(h, (cudaStream_t)stream));
+    return BSKENV_OK;
+}
+
+// Copies the n_stats episode statistics to the host and zeroes them (after everything queued on the device)
+inline int episode_stats(BatchCore *h, int n_stats, double *stats_host)
+{
+    CU_TRY(h, cudaSetDevice(h->device));
+    CU_TRY(h, cudaDeviceSynchronize());
+    CU_TRY(h, cudaMemcpy(stats_host, h->stats, sizeof(double) * n_stats, cudaMemcpyDeviceToHost));
+    CU_TRY(h, cudaMemset(h->stats, 0, sizeof(double) * n_stats));
+    return BSKENV_OK;
+}
+
+// Host-buffer entry points: the step kernels read the actions from and write their results to PINNED HOST memory directly
+// (zero-copy over PCIe).  Caller buffers that are already page-locked (bskenv_alloc_host, cudaHostRegister, torch pin_memory)
+// are used in place: *dev is their device-visible address, *stage null.  Pageable ones go through the handle's page-locked
+// staging block of `slot` (*stage), and the caller copies in or out with one memcpy.
+inline int host_map(BatchCore *h, const void *user, size_t bytes, int slot, void **dev, void **stage)
+{
+    *stage = nullptr;
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, user) == cudaSuccess && a.type == cudaMemoryTypeHost && a.devicePointer) { *dev = a.devicePointer; return BSKENV_OK; }
+    cudaGetLastError();
+    if (!h->h_stage[slot]) CU_TRY(h, cudaHostAlloc(&h->h_stage[slot], bytes, cudaHostAllocMapped));
+    *stage = h->h_stage[slot];
+    CU_TRY(h, cudaHostGetDevicePointer(dev, *stage, 0));
+    return BSKENV_OK;
+}
+
+// bskenv_state_field / bskenv_opnav_state_field: the index of a named field in the batch's table (-1: none), is_int = which block
+struct FieldEnt { const char *n; int idx; int is_int; };
+template <size_t N>
+int state_field(const FieldEnt (&tab)[N], const char *name, int32_t *is_int)
+{
+    if (!name) return -1;
+    for (const FieldEnt &t : tab)
+        if (!strcmp(t.n, name)) { if (is_int) *is_int = t.is_int; return t.idx; }
+    return -1;
+}
+
+}  // namespace

@@ -22,6 +22,7 @@
 #include "leo_core.cuh"
 #include "leo_split.cuh"
 #include "leo_host.h"
+#include "batch_common.cuh"
 
 #ifndef LEO_LANES
 #define LEO_LANES 32            // envs per warp (tuning builds: 16 / 8 leave the upper lanes idle)
@@ -47,13 +48,6 @@
 namespace {
 
 enum { ST_RET = 0, ST_LEN, ST_COUNT, ST_WHEEL, ST_POWER, ST_DECAY, ST_MAXLEN, ST_STEPS, ST_N };
-
-__device__ __forceinline__ double warp_sum(double v)
-{
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
-    return v;
-}
 
 #ifdef LEO_MAXNREG
 #define LEO_STEP_BOUNDS(MINB) __maxnreg__(LEO_MAXNREG)       // tuning builds: explicit register cap instead of an occupancy target
@@ -381,19 +375,7 @@ leo_reset_kernel(const __grid_constant__ LeoParams P, double *__restrict__ S, in
     if (mode == 2) I[(int64_t)I_EPISODE * stride + e] = ++ep;
     const int64_t prow = (pool.n_rows > 0 && mode != 1) ? leo::pool_row(pool, P.seed, ge, ep) : -1;
     double ic[19];
-    if (mode == 0) {
-        for (int k = 0; k < 19; k++) ic[k] = ics_in[e * 19 + k];
-    } else if (mode == 1) {
-        for (int k = 0; k < 19; k++) ic[k] = ics[(int64_t)k * stride + e];
-    } else if (icp.n_rows > 0) {
-        const int64_t r = leo::ic_pool_row(icp, P.seed, ge, ep, prow);
-        for (int k = 0; k < 19; k++) ic[k] = icp.rows[r * 19 + k];
-        icp.row_of[e] = (int32_t)r; icp.row_ep[e] = ep;
-    } else {
-        leo::sample_ic(P, ge, ep, ic);
-    }
-    if (icp.row_of && mode != 1 && !(mode == 2 && icp.n_rows > 0)) { icp.row_of[e] = -1; icp.row_ep[e] = ep; }
-    for (int k = 0; k < 19; k++) ics[(int64_t)k * stride + e] = ic[k];
+    reset_ics(mode, ics_in, ics, stride, e, ge, P.seed, ep, prow, icp, [&](double (&x)[19]) { leo::sample_ic(P, ge, ep, x); }, ic);
     double ob[5];
     if (pool.n_rows > 0) {
         if (mode != 1) leo::pool_assign(pool, S, stride, e, prow);
@@ -417,31 +399,6 @@ __global__ void gather_params_kernel(const double *__restrict__ S, int64_t strid
     if (row) row[e] = live ? (int32_t)S[(int64_t)(LEO_ND + PE_ROW) * stride + e] : -1;
 }
 
-__global__ void gather_ics_kernel(const double *__restrict__ ics, int64_t stride, int64_t n, double *__restrict__ out)
-{
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= n) return;
-    for (int k = 0; k < 19; k++) out[e * 19 + k] = ics[(int64_t)k * stride + e];
-}
-// bskenv_get_ic_rows: the recorded row where it belongs to the env's current episode (an in-kernel reset after an unload
-// advances the episode counter without touching the record)
-__global__ void gather_ic_rows_kernel(const int32_t *__restrict__ row_of, const int64_t *__restrict__ row_ep, const int64_t *__restrict__ ep,
-                                      int64_t n, int32_t *__restrict__ out)
-{
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= n) return;
-    out[e] = row_ep[e] == ep[e] ? row_of[e] : -1;
-}
-// dense [fields][n] <-> padded [fields][stride]
-template <typename T>
-__global__ void copy_fields_kernel(const T *__restrict__ src, int64_t src_stride, T *__restrict__ dst, int64_t dst_stride,
-                                   int64_t n, int fields)
-{
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= n) return;
-    for (int f = 0; f < fields; f++) dst[(int64_t)f * dst_stride + e] = src[(int64_t)f * src_stride + e];
-}
-
 // 8 independent DFMA chains per thread, everything in registers
 __global__ void __launch_bounds__(256) fp64_peak_kernel(double *out, int iters, double a, double b)
 {
@@ -460,49 +417,20 @@ thread_local std::string g_create_error;
 
 }  // namespace
 
-struct bskenv_handle {
+// The shared core (batch_common.cuh: BatchCore) and what only the LEO batch has.  The host-buffer step is complete when
+// bskenv_step_host[_wait] returns; its staging slots are actions, obs, reward, done, reason, ep_return, ep_length, term_obs.
+struct bskenv_handle : BatchCore {
     bskenv_config cfg;
     LeoParams P;
     LeoParamsF PF;
-    int device;
-    int64_t n, stride;
-    double *S, *ics, *stats;
-    int64_t *I;
     int *sched;                 // work queue head of the step kernel
     int32_t *perm; int *bucket; // lane assignment of the throughput organisation (envs bucketed by action), bucket sizes / cursors
-    double *d_eph[2];           // device copies of the ephemeris tables (Sun position, Earth orientation angles)
-    int sm_count;
-    // host-buffer entry points: page-locked staging (only for pageable caller buffers), own stream, ordering events
-    void *h_stage[8];           // actions, obs, reward, done, reason, ep_return, ep_length, term_obs
-    void *pend_user[8]; size_t pend_bytes[8]; int host_pending;
-    cudaStream_t own_stream;
-    cudaEvent_t ev_last;        // recorded after every launch queued through the device-buffer entry points
-    int ev_valid;
-    int64_t launches;
+    void *pend_user[8]; size_t pend_bytes[8];   // the staged results of the host-buffer step in flight
     const char *kernel_name;    // the step-kernel instantiation of the last launch
     int organisation;           // BSKENV_ORG_*: 0 auto, 1 one thread per env, 2 two warps per env group (small batches)
     LeoPool pool;               // loaded parameter pool (n_rows = 0: none); rows in device memory
     int s_fields;               // double fields allocated per env in S: LEO_ND, or LEO_ND + LEO_NPD once a pool was loaded
-    IcPool icp;                 // loaded initial-condition pool (n_rows = 0: none); rows and per-env record in device memory
-    std::string err;
 };
-
-#define CU_TRY(h, call)                                                                              \
-    do {                                                                                             \
-        cudaError_t _e = (call);                                                                     \
-        if (_e != cudaSuccess) {                                                                     \
-            (h)->err = std::string(#call) + ": " + cudaGetErrorString(_e);                            \
-            return BSKENV_ECUDA;                                                                     \
-        }                                                                                            \
-    } while (0)
-
-// Launches queued on the caller's streams are ordered before a later host-buffer step (which runs on the handle's own
-// stream) through this event; the host-buffer step itself is complete when bskenv_step_host[_wait] returns.
-static cudaError_t note_launch(bskenv_handle *h, cudaStream_t st)
-{
-    h->ev_valid = 1;
-    return cudaEventRecord(h->ev_last, st);
-}
 #define NO_HOST_PENDING(h, what)                                                                                        \
     do {                                                                                                                \
         if ((h)->host_pending) { (h)->err = what ": a host-buffer step is in flight (call bskenv_step_host_wait first)"; return BSKENV_EINVAL; } \
@@ -515,8 +443,7 @@ static cudaError_t note_launch(bskenv_handle *h, cudaStream_t st)
 // the step kernel wrote: mapped caller memory or the staging blocks, which are copied back after this launch.
 static int launch_follow_reset(bskenv_handle *h, const uint8_t *done, double *obs, cudaStream_t st)
 {
-    leo_reset_kernel<<<(int)((h->n + 255) / 256), 256, 0, st>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, 2, nullptr, done, obs,
-                                                                h->pool, h->icp);
+    leo_reset_kernel<<<env_grid(h), 256, 0, st>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, 2, nullptr, done, obs, h->pool, h->icp);
     CU_TRY(h, cudaGetLastError());
     h->launches++;
     return BSKENV_OK;
@@ -665,14 +592,8 @@ int bskenv_set_organisation(bskenv_handle *h, int organisation)
 
 int bskenv_create(const bskenv_config *cfg, int device, int64_t n_envs, int64_t first_env_index, bskenv_handle **out)
 {
-    if (!cfg || !out || n_envs <= 0) { g_create_error = "bskenv_create: bad arguments"; return BSKENV_EINVAL; }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        g_create_error = "bskenv_create: no CUDA device (this library has no CPU path)";
-        return BSKENV_ENODEV;
-    }
-    if (device < 0 || device >= ndev) { g_create_error = "bskenv_create: device index out of range"; return BSKENV_EINVAL; }
+    const int rc = check_create("bskenv_create", cfg && out && n_envs > 0, device, g_create_error);
+    if (rc) return rc;
     bskenv_handle *h = new bskenv_handle();
     h->cfg = *cfg;
     std::string perr = leo_host::build_params(*cfg, h->P);
@@ -683,27 +604,11 @@ int bskenv_create(const bskenv_config *cfg, int device, int64_t n_envs, int64_t 
     }
     leo_host::build_params_f(h->P, h->PF);
     h->P.first_env_index = first_env_index;
-    h->device = device; h->n = n_envs; h->stride = (n_envs + 31) / 32 * 32; h->launches = 0; h->kernel_name = nullptr; h->organisation = BSKENV_ORG_AUTO;
-    h->S = h->ics = h->stats = nullptr; h->I = nullptr; h->sched = nullptr; h->perm = nullptr; h->bucket = nullptr;
-    h->d_eph[0] = h->d_eph[1] = nullptr;
-    h->pool.rows = nullptr; h->pool.n_rows = 0; h->pool.assign = 0; h->s_fields = LEO_ND;
-    h->icp.rows = nullptr; h->icp.row_of = nullptr; h->icp.row_ep = nullptr; h->icp.n_rows = 0; h->icp.assign = 0;
-    for (int k = 0; k < 8; k++) { h->h_stage[k] = nullptr; h->pend_user[k] = nullptr; h->pend_bytes[k] = 0; }
-    h->host_pending = 0; h->own_stream = nullptr; h->ev_last = nullptr; h->ev_valid = 0;
-    cudaError_t e = cudaSetDevice(device);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->ev_last, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&h->sm_count, cudaDevAttrMultiProcessorCount, device);
+    h->s_fields = LEO_ND;       // (the handle is zero-initialised: no pools, BSKENV_ORG_AUTO)
+    cudaError_t e = core_alloc(h, device, n_envs, LEO_ND, LEO_NI, 19, ST_N);
     if (e == cudaSuccess) e = cudaMalloc(&h->sched, sizeof(int) * (size_t)(4 + (n_envs + LEO_LANES - 1) / LEO_LANES));
     if (e == cudaSuccess) e = cudaMalloc(&h->perm, sizeof(int32_t) * h->stride);
     if (e == cudaSuccess) e = cudaMalloc(&h->bucket, sizeof(int) * 8);
-    if (e == cudaSuccess) e = cudaMalloc(&h->S, sizeof(double) * LEO_ND * h->stride);
-    if (e == cudaSuccess) e = cudaMalloc(&h->I, sizeof(int64_t) * LEO_NI * h->stride);
-    if (e == cudaSuccess) e = cudaMalloc(&h->ics, sizeof(double) * 19 * h->stride);
-    if (e == cudaSuccess) e = cudaMalloc(&h->stats, sizeof(double) * ST_N);
-    if (e == cudaSuccess) e = cudaMemset(h->S, 0, sizeof(double) * LEO_ND * h->stride);
-    if (e == cudaSuccess) e = cudaMemset(h->I, 0, sizeof(int64_t) * LEO_NI * h->stride);
-    if (e == cudaSuccess) e = cudaMemset(h->ics, 0, sizeof(double) * 19 * h->stride);
-    if (e == cudaSuccess) e = cudaMemset(h->stats, 0, sizeof(double) * ST_N);
     if (e != cudaSuccess) {
         g_create_error = std::string("bskenv_create: ") + cudaGetErrorString(e);
         bskenv_destroy(h);
@@ -717,12 +622,9 @@ int bskenv_destroy(bskenv_handle *h)
 {
     if (!h) return BSKENV_OK;
     cudaSetDevice(h->device);
-    cudaFree(h->S); cudaFree(h->I); cudaFree(h->ics); cudaFree(h->stats); cudaFree(h->sched); cudaFree(h->perm); cudaFree(h->bucket);
-    cudaFree(h->d_eph[0]); cudaFree(h->d_eph[1]); cudaFree((void *)h->pool.rows);
-    cudaFree((void *)h->icp.rows); cudaFree(h->icp.row_of); cudaFree(h->icp.row_ep);
-    if (h->own_stream) { cudaStreamSynchronize(h->own_stream); cudaStreamDestroy(h->own_stream); }
-    for (int k = 0; k < 8; k++) cudaFreeHost(h->h_stage[k]);
-    if (h->ev_last) cudaEventDestroy(h->ev_last);
+    cudaFree(h->sched); cudaFree(h->perm); cudaFree(h->bucket);
+    cudaFree((void *)h->P.eph_sun.coef); cudaFree((void *)h->P.eph_orient.coef); cudaFree((void *)h->pool.rows);
+    core_free(h);
     delete h;
     return BSKENV_OK;
 }
@@ -740,24 +642,9 @@ int bskenv_set_gravity_degree2(bskenv_handle *h, int enable, const double *cbar)
 int bskenv_set_ephemeris(bskenv_handle *h, int kind, double t0, double seg_len, int n_seg, int n_coef, const double *coef)
 {
     if (!h || kind < 0 || kind > 1) return BSKENV_EINVAL;
-    CU_TRY(h, cudaSetDevice(h->device));
-    CU_TRY(h, cudaDeviceSynchronize());                         // a launch in flight may still read the old table
-    LeoEph &E = kind == 0 ? h->P.eph_sun : h->P.eph_orient;
-    cudaFree(h->d_eph[kind]); h->d_eph[kind] = nullptr;
-    E.coef = nullptr; E.nseg = 0; E.ncoef = 0; E.t0 = 0.; E.seg_len = 0.;
-    if (n_seg <= 0) return BSKENV_OK;                           // back to the analytic model
-    if (!coef || n_coef < 1 || n_coef > 64 || !(seg_len > 0.)) { h->err = "bskenv_set_ephemeris: bad table shape"; return BSKENV_EINVAL; }
     // an episode runs from sim time 0 to (max_length + 1) decision intervals: the table has to cover it
     const double t_end = ((double)h->P.max_length + 1.0) * (double)h->P.step_ns * 1e-9;   // max_length may be INT_MAX
-    if (t0 > 0. || t0 + seg_len * n_seg < t_end) {
-        h->err = "bskenv_set_ephemeris: the table does not cover one episode [0, (max_length + 1) * step_duration]";
-        return BSKENV_EINVAL;
-    }
-    const size_t bytes = sizeof(double) * (size_t)n_seg * 3 * (size_t)n_coef;
-    CU_TRY(h, cudaMalloc(&h->d_eph[kind], bytes));
-    CU_TRY(h, cudaMemcpy(h->d_eph[kind], coef, bytes, cudaMemcpyHostToDevice));
-    E.coef = h->d_eph[kind]; E.nseg = n_seg; E.ncoef = n_coef; E.t0 = t0; E.seg_len = seg_len;
-    return BSKENV_OK;
+    return set_ephemeris(h, "bskenv_set_ephemeris", kind == 0 ? h->P.eph_sun : h->P.eph_orient, t_end, t0, seg_len, n_seg, n_coef, coef);
 }
 
 int bskenv_set_param_pool(bskenv_handle *h, int n_rows, const double *rows_host, int assign)
@@ -829,49 +716,19 @@ int bskenv_set_ic_pool(bskenv_handle *h, int n_rows, const double *ics_host, int
 {
     if (!h) return BSKENV_EINVAL;
     NO_HOST_PENDING(h, "bskenv_set_ic_pool");
-    if (n_rows < 0 || (n_rows > 0 && !ics_host)) { h->err = "bskenv_set_ic_pool: bad row count or null rows"; return BSKENV_EINVAL; }
-    if (n_rows > 0) {
-        if (assign != BSKENV_ICS_BY_INDEX && assign != BSKENV_ICS_PER_EPISODE && assign != BSKENV_ICS_PARAM_ROW) {
-            h->err = "bskenv_set_ic_pool: unknown assignment mode"; return BSKENV_EINVAL;
-        }
-        if (assign == BSKENV_ICS_PARAM_ROW && h->pool.n_rows != n_rows) {
-            h->err = "bskenv_set_ic_pool: BSKENV_ICS_PARAM_ROW needs a loaded parameter pool of the same row count (" +
-                     std::to_string(n_rows) + " IC rows, " + std::to_string(h->pool.n_rows) + " parameter rows)";
-            return BSKENV_EINVAL;
-        }
-        for (int r = 0; r < n_rows; r++) {
-            const std::string err = leo_host::ic_row_check(ics_host + (size_t)r * BSKENV_IC_DIM, BSKENV_IC_DIM);
-            if (!err.empty()) { h->err = "bskenv_set_ic_pool: row " + std::to_string(r) + ": " + err; return BSKENV_EINVAL; }
-        }
-    }
-    CU_TRY(h, cudaSetDevice(h->device));
-    CU_TRY(h, cudaDeviceSynchronize());                         // a launch in flight may still read the old pool
-    cudaFree((void *)h->icp.rows);
-    h->icp.rows = nullptr; h->icp.n_rows = 0;
-    if (n_rows == 0) return BSKENV_OK;                          // unloaded: resets sample again, the in-kernel auto-reset
-    if (!h->icp.row_of) {                                       // first pool of this handle: the per-env record, all -1
-        CU_TRY(h, cudaMalloc(&h->icp.row_of, sizeof(int32_t) * h->stride));
-        CU_TRY(h, cudaMalloc(&h->icp.row_ep, sizeof(int64_t) * h->stride));
-        CU_TRY(h, cudaMemset(h->icp.row_of, 0xFF, sizeof(int32_t) * h->stride));
-        CU_TRY(h, cudaMemset(h->icp.row_ep, 0, sizeof(int64_t) * h->stride));
-    }
-    double *d_rows = nullptr;
-    const size_t bytes = sizeof(double) * (size_t)n_rows * BSKENV_IC_DIM;
-    CU_TRY(h, cudaMalloc(&d_rows, bytes));
-    CU_TRY(h, cudaMemcpy(d_rows, ics_host, bytes, cudaMemcpyHostToDevice));
-    h->icp.rows = d_rows; h->icp.n_rows = n_rows; h->icp.assign = assign;
-    return BSKENV_OK;
+    return set_ic_pool(h, "bskenv_set_ic_pool", n_rows, ics_host, BSKENV_IC_DIM, assign, [&]() -> std::string {
+        if (assign != BSKENV_ICS_BY_INDEX && assign != BSKENV_ICS_PER_EPISODE && assign != BSKENV_ICS_PARAM_ROW)
+            return "bskenv_set_ic_pool: unknown assignment mode";
+        if (assign == BSKENV_ICS_PARAM_ROW && h->pool.n_rows != n_rows)
+            return "bskenv_set_ic_pool: BSKENV_ICS_PARAM_ROW needs a loaded parameter pool of the same row count (" +
+                   std::to_string(n_rows) + " IC rows, " + std::to_string(h->pool.n_rows) + " parameter rows)";
+        return "";
+    });
 }
 
 int bskenv_get_ic_rows(bskenv_handle *h, int32_t *rows_dev, void *stream)
 {
-    if (!h || !rows_dev) { if (h) h->err = "bskenv_get_ic_rows: null rows"; return BSKENV_EINVAL; }
-    CU_TRY(h, cudaSetDevice(h->device));
-    if (!h->icp.row_of) CU_TRY(h, cudaMemsetAsync(rows_dev, 0xFF, sizeof(int32_t) * h->n, (cudaStream_t)stream));
-    else gather_ic_rows_kernel<<<(int)((h->n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->icp.row_of, h->icp.row_ep,
-                                                                                             h->I + (size_t)I_EPISODE * h->stride, h->n, rows_dev);
-    CU_TRY(h, cudaGetLastError());
-    return BSKENV_OK;
+    return h ? get_ic_rows(h, "bskenv_get_ic_rows", I_EPISODE, rows_dev, stream) : BSKENV_EINVAL;
 }
 
 static int do_reset(bskenv_handle *h, int mode, const double *ics_in, const uint8_t *mask, double *obs, void *stream)
@@ -879,8 +736,7 @@ static int do_reset(bskenv_handle *h, int mode, const double *ics_in, const uint
     if (!h) return BSKENV_EINVAL;
     NO_HOST_PENDING(h, "bskenv_reset");
     CU_TRY(h, cudaSetDevice(h->device));
-    const int grid = (int)((h->n + 255) / 256);
-    leo_reset_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, mode, ics_in, mask, obs, h->pool, h->icp);
+    leo_reset_kernel<<<env_grid(h), 256, 0, (cudaStream_t)stream>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, mode, ics_in, mask, obs, h->pool, h->icp);
     CU_TRY(h, cudaGetLastError());
     CU_TRY(h, note_launch(h, (cudaStream_t)stream));
     return BSKENV_OK;
@@ -902,11 +758,7 @@ int bskenv_reset_init(bskenv_handle *h, const uint8_t *mask_dev, double *obs_dev
 }
 int bskenv_get_ics(bskenv_handle *h, double *ics_dev, void *stream)
 {
-    if (!h || !ics_dev) return BSKENV_EINVAL;
-    CU_TRY(h, cudaSetDevice(h->device));
-    gather_ics_kernel<<<(int)((h->n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->ics, h->stride, h->n, ics_dev);
-    CU_TRY(h, cudaGetLastError());
-    return BSKENV_OK;
+    return h ? get_ics<19>(h, ics_dev, stream) : BSKENV_EINVAL;
 }
 
 int bskenv_step(bskenv_handle *h, const int32_t *actions_dev, double *obs_dev, double *reward_dev, uint8_t *done_dev,
@@ -932,31 +784,8 @@ int bskenv_step_info(bskenv_handle *h, const int32_t *actions_dev, double *obs_d
 }
 
 // ---- host-buffer entry points (the reference-facing plugin path) ----------------------------------------------------
-// The step kernel reads the actions from and writes its results to PINNED HOST memory directly (zero-copy over PCIe:
-// 4 B in and 50 B out per env, spread over the whole launch, so no transfer is exposed after the kernel).  Caller buffers
-// that are already page-locked (bskenv_alloc_host, cudaHostRegister, torch pin_memory) are used in place; pageable ones go
-// through page-locked staging owned by the handle plus one memcpy each.
-namespace {
-struct HostMap { void *dev; void *stage; };          // device-visible address, and the staging block behind it (or null)
-bool host_pinned(const void *p, void **dev)
-{
-    cudaPointerAttributes a;
-    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
-    if (a.type != cudaMemoryTypeHost || !a.devicePointer) return false;
-    *dev = a.devicePointer;
-    return true;
-}
-}  // namespace
-
-static int host_map(bskenv_handle *h, const void *user, size_t bytes, int slot, HostMap *m)
-{
-    m->stage = nullptr;
-    if (host_pinned(user, &m->dev)) return BSKENV_OK;
-    if (!h->h_stage[slot]) CU_TRY(h, cudaHostAlloc(&h->h_stage[slot], bytes, cudaHostAllocMapped));
-    m->stage = h->h_stage[slot];
-    CU_TRY(h, cudaHostGetDevicePointer(&m->dev, m->stage, 0));
-    return BSKENV_OK;
-}
+// Zero-copy (batch_common.cuh: host_map): 4 B in and 50 B out per env, spread over the whole launch, so no transfer is
+// exposed after the kernel.
 
 int bskenv_step_host_async(bskenv_handle *h, const int32_t *actions, double *obs, double *reward, uint8_t *done,
                            uint8_t *done_reason, double *term_obs, double *ep_return, int64_t *ep_length)
@@ -969,28 +798,21 @@ int bskenv_step_host_async(bskenv_handle *h, const int32_t *actions, double *obs
     const size_t n = (size_t)h->n;
     if (!h->own_stream) CU_TRY(h, cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
     cudaStream_t st = h->own_stream;
-    HostMap m[8];
-    int rc;
-    if ((rc = host_map(h, actions, n * sizeof(int32_t), 0, &m[0]))) return rc;
-    if ((rc = host_map(h, obs, n * 5 * sizeof(double), 1, &m[1]))) return rc;
-    if ((rc = host_map(h, reward, n * sizeof(double), 2, &m[2]))) return rc;
-    if ((rc = host_map(h, done, n, 3, &m[3]))) return rc;
-    if ((rc = host_map(h, done_reason, n, 4, &m[4]))) return rc;
-    m[5].dev = m[6].dev = m[7].dev = nullptr; m[5].stage = m[6].stage = m[7].stage = nullptr;
-    if (term_obs && (rc = host_map(h, term_obs, n * 5 * sizeof(double), 7, &m[7]))) return rc;
-    if (ep_return) {
-        if ((rc = host_map(h, ep_return, n * sizeof(double), 5, &m[5]))) return rc;
-        if ((rc = host_map(h, ep_length, n * sizeof(int64_t), 6, &m[6]))) return rc;
+    void *user[8] = {(void *)actions, obs, reward, done, done_reason, ep_return, ep_length, term_obs};
+    const size_t bytes[8] = {n * sizeof(int32_t), n * 5 * sizeof(double), n * sizeof(double), n, n, n * sizeof(double), n * sizeof(int64_t), n * 5 * sizeof(double)};
+    void *dev[8] = {}, *stage[8] = {};
+    for (int k = 0; k < 8; k++) {
+        if (!user[k]) continue;
+        const int rc = host_map(h, user[k], bytes[k], k, &dev[k], &stage[k]);
+        if (rc) return rc;
     }
-    if (m[0].stage) memcpy(m[0].stage, actions, n * sizeof(int32_t));
+    if (stage[0]) memcpy(stage[0], actions, bytes[0]);
     // order after whatever the caller queued through bskenv_step / reset / set_state on its own streams
     if (h->ev_valid) CU_TRY(h, cudaStreamWaitEvent(st, h->ev_last, 0));
-    rc = launch_step(h, (const int32_t *)m[0].dev, (double *)m[1].dev, (double *)m[2].dev, (uint8_t *)m[3].dev, (uint8_t *)m[4].dev,
-                     (double *)m[7].dev, st, (double *)m[5].dev, (int64_t *)m[6].dev);
+    const int rc = launch_step(h, (const int32_t *)dev[0], (double *)dev[1], (double *)dev[2], (uint8_t *)dev[3], (uint8_t *)dev[4],
+                               (double *)dev[7], st, (double *)dev[5], (int64_t *)dev[6]);
     if (rc) return rc;
-    void *user[8] = {nullptr, obs, reward, done, done_reason, ep_return, ep_length, term_obs};
-    const size_t bytes[8] = {0, n * 5 * sizeof(double), n * sizeof(double), n, n, n * sizeof(double), n * sizeof(int64_t), n * 5 * sizeof(double)};
-    for (int k = 0; k < 8; k++) { h->pend_user[k] = m[k].stage ? user[k] : nullptr; h->pend_bytes[k] = bytes[k]; }
+    for (int k = 0; k < 8; k++) { h->pend_user[k] = stage[k] ? user[k] : nullptr; h->pend_bytes[k] = bytes[k]; }
     h->host_pending = 1;
     return BSKENV_OK;
 }
@@ -1033,29 +855,15 @@ int bskenv_state_dims(const bskenv_handle *h, int32_t *nd, int32_t *ni)
 }
 int bskenv_get_state(bskenv_handle *h, double *dstate_dev, int64_t *istate_dev, void *stream)
 {
-    if (!h) return BSKENV_EINVAL;
-    CU_TRY(h, cudaSetDevice(h->device));
-    const int grid = (int)((h->n + 255) / 256);
-    if (dstate_dev) copy_fields_kernel<double><<<grid, 256, 0, (cudaStream_t)stream>>>(h->S, h->stride, dstate_dev, h->n, h->n, LEO_ND);
-    if (istate_dev) copy_fields_kernel<int64_t><<<grid, 256, 0, (cudaStream_t)stream>>>(h->I, h->stride, istate_dev, h->n, h->n, LEO_NI);
-    CU_TRY(h, cudaGetLastError());
-    return BSKENV_OK;
+    return h ? get_state(h, LEO_ND, LEO_NI, dstate_dev, istate_dev, stream) : BSKENV_EINVAL;
 }
 int bskenv_set_state(bskenv_handle *h, const double *dstate_dev, const int64_t *istate_dev, void *stream)
 {
-    if (!h) return BSKENV_EINVAL;
-    CU_TRY(h, cudaSetDevice(h->device));
-    const int grid = (int)((h->n + 255) / 256);
-    if (dstate_dev) copy_fields_kernel<double><<<grid, 256, 0, (cudaStream_t)stream>>>(dstate_dev, h->n, h->S, h->stride, h->n, LEO_ND);
-    if (istate_dev) copy_fields_kernel<int64_t><<<grid, 256, 0, (cudaStream_t)stream>>>(istate_dev, h->n, h->I, h->stride, h->n, LEO_NI);
-    CU_TRY(h, cudaGetLastError());
-    CU_TRY(h, note_launch(h, (cudaStream_t)stream));
-    return BSKENV_OK;
+    return h ? set_state(h, LEO_ND, LEO_NI, dstate_dev, istate_dev, stream) : BSKENV_EINVAL;
 }
 int bskenv_state_field(const char *name, int32_t *is_int)
 {
-    struct Ent { const char *n; int idx; int is_int; };
-    static const Ent tab[] = {
+    static const FieldEnt tab[] = {
         {"r_BN_N", F_R, 0}, {"v_BN_N", F_V, 0}, {"sigma_BN", F_SIG, 0}, {"omega_BN_B", F_OMG, 0}, {"Omega", F_WHL, 0},
         {"u_current", F_UCUR, 0}, {"density", F_RHO, 0}, {"storedCharge", F_E, 0}, {"shadowFactor", F_SHADOW, 0},
         {"extTorquePntB_B", F_LDIST, 0}, {"att_guidance", F_GUID, 0}, {"att_reference", F_REF, 0},
@@ -1067,20 +875,12 @@ int bskenv_state_field(const char *name, int32_t *is_int)
         {"dumpPriorTime", I_DUMPPRIOR, 1}, {"lastDeltaHInMsgTime", I_LASTDH, 1}, {"deltaHWriteTime", I_DHTIME, 1},
         {"episode", I_EPISODE, 1}, {"fireCounter", I_FIRE, 1}, {"thrActive", I_THRACTIVE, 1}, {"episode_over", I_OVER, 1},
         {"rwSat", I_RWSAT, 1}};
-    if (!name) return -1;
-    for (const Ent &t : tab)
-        if (!strcmp(t.n, name)) { if (is_int) *is_int = t.is_int; return t.idx; }
-    return -1;
+    return state_field(tab, name, is_int);
 }
 
 int bskenv_episode_stats(bskenv_handle *h, double *stats_host)
 {
-    if (!h || !stats_host) return BSKENV_EINVAL;
-    CU_TRY(h, cudaSetDevice(h->device));
-    CU_TRY(h, cudaDeviceSynchronize());
-    CU_TRY(h, cudaMemcpy(stats_host, h->stats, sizeof(double) * ST_N, cudaMemcpyDeviceToHost));
-    CU_TRY(h, cudaMemset(h->stats, 0, sizeof(double) * ST_N));
-    return BSKENV_OK;
+    return (h && stats_host) ? episode_stats(h, ST_N, stats_host) : BSKENV_EINVAL;
 }
 
 int bskenv_fp64_peak(int device, double seconds, double *tflops)

@@ -18,6 +18,7 @@
 #include "../../include/bskenv.h"
 #include "opnav_core.cuh"
 #include "opnav_host.h"
+#include "batch_common.cuh"
 
 #ifndef ON_NZBUF_MAX_FRAC
 #define ON_NZBUF_MAX_FRAC 0.45   // of the free device memory, for the noise buffer of the three-kernel interval
@@ -29,13 +30,6 @@
 namespace {
 
 enum { OST_RET = 0, OST_LEN, OST_COUNT, OST_MAXLEN, OST_MODES, OST_STEPS, OST_MEAS, OST_BAD, OST_N };
-
-__device__ __forceinline__ double warp_sum_d(double v)
-{
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
-    return v;
-}
 
 // One warp steps a group of 32 consecutive envs; when there are more groups than resident warps the grid is one
 // resident set and the warps pull groups from an atomic queue (same scheme as the LEO step kernel).
@@ -243,7 +237,7 @@ opnav_pass2_kernel(const __grid_constant__ OpNavParams P, double *__restrict__ S
         if (stats) {
             const unsigned any_done = __ballot_sync(0xffffffffu, valid && o.done);
             if (any_done) {
-                double v_ret = warp_sum_d(o.done ? ep_ret : 0.), v_len = warp_sum_d(o.done ? ep_len : 0.);
+                double v_ret = warp_sum(o.done ? ep_ret : 0.), v_len = warp_sum(o.done ? ep_len : 0.);
                 int c_all = __popc(any_done);
                 int c_m = __popc(__ballot_sync(0xffffffffu, valid && o.done && (o.reason & 1)));
                 int c_s = __popc(__ballot_sync(0xffffffffu, valid && o.done && (o.reason & 2)));
@@ -254,7 +248,7 @@ opnav_pass2_kernel(const __grid_constant__ OpNavParams P, double *__restrict__ S
                 }
             }
             const int c_valid = __popc(__ballot_sync(0xffffffffu, valid));
-            double v_meas = warp_sum_d(d_meas), v_bad = warp_sum_d(d_bad);
+            double v_meas = warp_sum(d_meas), v_bad = warp_sum(d_bad);
             if (lane == 0 && c_valid) {
                 atomicAdd(&stats[OST_STEPS], (double)c_valid);
                 atomicAdd(&stats[OST_MEAS], v_meas);
@@ -276,93 +270,39 @@ opnav_reset_kernel(const __grid_constant__ OpNavParams P, double *__restrict__ S
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n) return;
     if (mask && !mask[e]) return;
+    const int64_t ge = P.first_env_index + e;
     int64_t ep = I[(int64_t)OI_EPISODE * stride + e];
+    if (mode == 2) I[(int64_t)OI_EPISODE * stride + e] = ++ep;
     double ic[OPNAV_IC_DIM];
-    if (mode == 0) {
-        for (int k = 0; k < OPNAV_IC_DIM; k++) ic[k] = ics_in[e * OPNAV_IC_DIM + k];
-    } else if (mode == 1) {
-        for (int k = 0; k < OPNAV_IC_DIM; k++) ic[k] = ics[(int64_t)k * stride + e];
-    } else {
-        I[(int64_t)OI_EPISODE * stride + e] = ++ep;
-        if (icp.n_rows > 0) {
-            const int64_t r = leo::ic_pool_row(icp, P.seed, P.first_env_index + e, ep, -1);
-            for (int k = 0; k < OPNAV_IC_DIM; k++) ic[k] = icp.rows[r * OPNAV_IC_DIM + k];
-            icp.row_of[e] = (int32_t)r; icp.row_ep[e] = ep;
-        } else {
-            opnav::sample_ic(P, P.first_env_index + e, ep, ic);
-        }
-    }
-    if (icp.row_of && mode != 1 && !(mode == 2 && icp.n_rows > 0)) { icp.row_of[e] = -1; icp.row_ep[e] = ep; }
-    for (int k = 0; k < OPNAV_IC_DIM; k++) ics[(int64_t)k * stride + e] = ic[k];
+    reset_ics(mode, ics_in, ics, stride, e, ge, P.seed, ep, -1, icp, [&](double (&x)[OPNAV_IC_DIM]) { opnav::sample_ic(P, ge, ep, x); }, ic);
     double ob[4];
     opnav::opnav_reset_env(P, S, I, stride, e, ic, ob);
     if (obs)
         for (int k = 0; k < 4; k++) obs[e * 4 + k] = ob[k];
-}
-__global__ void opnav_gather_ic_rows_kernel(const int32_t *__restrict__ row_of, const int64_t *__restrict__ row_ep,
-                                            const int64_t *__restrict__ ep, int64_t n, int32_t *__restrict__ out)
-{
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= n) return;
-    out[e] = row_ep[e] == ep[e] ? row_of[e] : -1;      // as bskenv.cu: gather_ic_rows_kernel
-}
-__global__ void opnav_gather_ics_kernel(const double *__restrict__ ics, int64_t stride, int64_t n, double *__restrict__ out)
-{
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= n) return;
-    for (int k = 0; k < OPNAV_IC_DIM; k++) out[e * OPNAV_IC_DIM + k] = ics[(int64_t)k * stride + e];
-}
-template <typename T>
-__global__ void opnav_copy_fields_kernel(const T *__restrict__ src, int64_t src_stride, T *__restrict__ dst, int64_t dst_stride,
-                                         int64_t n, int fields)
-{
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= n) return;
-    for (int f = 0; f < fields; f++) dst[(int64_t)f * dst_stride + e] = src[(int64_t)f * src_stride + e];
 }
 
 thread_local std::string g_opnav_create_error;
 
 }  // namespace
 
-struct bskenv_opnav_handle {
+// The shared core (batch_common.cuh: BatchCore) and what only the opNav batch has.  Staging slots of the host-buffer step:
+// actions, obs, reward, done, reason, debug.
+struct bskenv_opnav_handle : BatchCore {
     bskenv_opnav_config cfg;
     OpNavParams P;
-    int device;
-    int64_t n, stride;
-    double *S, *ics, *stats;
-    int64_t *I;
     int *sched;
     int32_t *perm;              // lane assignment of the step kernel (envs bucketed by task set)
     double *mbuf;               // measurements of the interval, first pass -> second pass: [slot][ON_MEAS_W][stride]
     double *nzbuf;              // noise walk of the interval, noise kernel -> dynamics kernel: [ticks_per_step + 1][15][stride]
     int noise_split;            // -1 undecided, 0 fused first pass, 1 three-kernel form (nzbuf allocated)
-    double *d_eph;              // device copy of the Sun ephemeris table
-    int sm_count;
-    void *h_stage[6];           // page-locked staging for pageable caller buffers: actions, obs, reward, done, reason, debug
-    cudaStream_t own_stream;
-    cudaEvent_t ev_last;        // recorded after every launch queued through the device-buffer entry points
-    int ev_valid;
-    int64_t launches;
-    IcPool icp;                 // loaded initial-condition pool (n_rows = 0: none), as in the LEO handle
-    std::string err;
 };
-
-#define ON_TRY(h, call)                                                                              \
-    do {                                                                                             \
-        cudaError_t _e = (call);                                                                     \
-        if (_e != cudaSuccess) {                                                                     \
-            (h)->err = std::string(#call) + ": " + cudaGetErrorString(_e);                            \
-            return BSKENV_ECUDA;                                                                     \
-        }                                                                                            \
-    } while (0)
 
 static int opnav_launch_step(bskenv_opnav_handle *h, const int32_t *act, double *obs, double *rew, uint8_t *done,
                              uint8_t *reason, double *debug, double *term_obs, cudaStream_t st, double *ep_return = nullptr,
                              int64_t *ep_length = nullptr)
 {
     // With an IC pool the second pass runs without its in-kernel reset (auto_reset is read nowhere else) and the reset kernel
-    // follows the interval, as in bskenv.cu: launch_follow_reset.
+    // follows the interval.
     const bool follow = h->icp.n_rows > 0 && h->P.auto_reset;
     OpNavParams P_nr;
     if (follow) { P_nr = h->P; P_nr.auto_reset = 0; }
@@ -383,7 +323,7 @@ static int opnav_launch_step(bskenv_opnav_handle *h, const int32_t *act, double 
     const int full = (int)((groups + wpb - 1) / wpb);
     OnSched sc;
     sc.sched = h->sched; sc.n_groups = (int)groups; sc.dynamic = 0;
-    ON_TRY(h, cudaMemsetAsync(h->sched, 0, sizeof(int) * 8, st));
+    CU_TRY(h, cudaMemsetAsync(h->sched, 0, sizeof(int) * 8, st));
     {   // bucket the envs by flight-software task set (two small launches; see opnav_bucket_*_kernel)
         const int bgrid = (int)((h->n + 255) / 256);
         opnav_bucket_count_kernel<<<bgrid, 256, 0, st>>>(h->I, h->stride, h->n, act, h->sched);
@@ -396,10 +336,10 @@ static int opnav_launch_step(bskenv_opnav_handle *h, const int32_t *act, double 
     const size_t smem_a = sizeof(OnScratchA) * ON_BLOCK, smem_b = sizeof(OnScratchB) * ON_BLOCK;
     static bool attr_set[64] = {false};             // opt in to the dynamic shared memory once per device
     if (!attr_set[h->device & 63]) {
-        ON_TRY(h, cudaFuncSetAttribute(opnav_pass1_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_a));
-        ON_TRY(h, cudaFuncSetAttribute(opnav_pass1_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_a));
-        ON_TRY(h, cudaFuncSetAttribute(opnav_pass2_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
-        ON_TRY(h, cudaFuncSetAttribute(opnav_pass2_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
+        CU_TRY(h, cudaFuncSetAttribute(opnav_pass1_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_a));
+        CU_TRY(h, cudaFuncSetAttribute(opnav_pass1_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_a));
+        CU_TRY(h, cudaFuncSetAttribute(opnav_pass2_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
+        CU_TRY(h, cudaFuncSetAttribute(opnav_pass2_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
         attr_set[h->device & 63] = true;
     }
     if (h->noise_split < 0) {
@@ -421,8 +361,8 @@ static int opnav_launch_step(bskenv_opnav_handle *h, const int32_t *act, double 
         const size_t smem_n = sizeof(OnScratchN) * ON_BLOCK, smem_d = sizeof(OnScratchD) * ON_BLOCK;
         static bool attr_d[64] = {false};
         if (!attr_d[h->device & 63]) {
-            ON_TRY(h, cudaFuncSetAttribute(opnav_dyn_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_d));
-            ON_TRY(h, cudaFuncSetAttribute(opnav_dyn_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_d));
+            CU_TRY(h, cudaFuncSetAttribute(opnav_dyn_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_d));
+            CU_TRY(h, cudaFuncSetAttribute(opnav_dyn_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_d));
             attr_d[h->device & 63] = true;
         }
         opnav_noise_kernel<<<(int)((h->n + ON_BLOCK - 1) / ON_BLOCK), ON_BLOCK, smem_n, st>>>(h->P, h->S, h->I, h->stride, h->n, h->perm, h->nzbuf);
@@ -441,14 +381,14 @@ static int opnav_launch_step(bskenv_opnav_handle *h, const int32_t *act, double 
     else
         opnav_pass2_kernel<2><<<grid2, ON_BLOCK, smem_b, st>>>(PK, h->S, h->I, h->ics, h->stride, h->n, act, obs, rew, done, reason, debug,
                                                           term_obs, h->stats, s2, h->perm, ep_return, ep_length, h->mbuf);
-    ON_TRY(h, cudaGetLastError());
+    CU_TRY(h, cudaGetLastError());
     h->launches += 2;
     if (follow) {           // obs / done: the buffers the second pass wrote (device, mapped host or staging memory)
-        opnav_reset_kernel<<<(int)((h->n + 255) / 256), 256, 0, st>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, 2, nullptr, done, obs, h->icp);
-        ON_TRY(h, cudaGetLastError());
+        opnav_reset_kernel<<<env_grid(h), 256, 0, st>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, 2, nullptr, done, obs, h->icp);
+        CU_TRY(h, cudaGetLastError());
         h->launches++;
     }
-    if (st != h->own_stream || !st) { h->ev_valid = 1; ON_TRY(h, cudaEventRecord(h->ev_last, st)); }
+    if (st != h->own_stream || !st) CU_TRY(h, note_launch(h, st));
     return BSKENV_OK;
 }
 
@@ -463,38 +403,18 @@ double bskenv_opnav_flops_per_step(const bskenv_opnav_handle *h) { return h ? op
 int bskenv_opnav_create(const bskenv_opnav_config *cfg, int device, int64_t n_envs, int64_t first_env_index,
                         bskenv_opnav_handle **out)
 {
-    if (!cfg || !out || n_envs <= 0) { g_opnav_create_error = "bskenv_opnav_create: bad arguments"; return BSKENV_EINVAL; }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
-        cudaGetLastError();
-        g_opnav_create_error = "bskenv_opnav_create: no CUDA device (this library has no CPU path)";
-        return BSKENV_ENODEV;
-    }
-    if (device < 0 || device >= ndev) { g_opnav_create_error = "bskenv_opnav_create: device index out of range"; return BSKENV_EINVAL; }
+    const int rc = check_create("bskenv_opnav_create", cfg && out && n_envs > 0, device, g_opnav_create_error);
+    if (rc) return rc;
     bskenv_opnav_handle *h = new bskenv_opnav_handle();
     h->cfg = *cfg;
     std::string perr = opnav_host::build_params(*cfg, h->P);
     if (!perr.empty()) { g_opnav_create_error = "bskenv_opnav_create: " + perr; delete h; return BSKENV_EINVAL; }
     h->P.first_env_index = first_env_index;
-    h->device = device; h->n = n_envs; h->stride = (n_envs + 31) / 32 * 32; h->launches = 0;
-    h->S = h->ics = h->stats = nullptr; h->I = nullptr; h->sched = nullptr; h->perm = nullptr; h->d_eph = nullptr; h->mbuf = nullptr; h->nzbuf = nullptr; h->noise_split = -1;
-    for (int k = 0; k < 6; k++) h->h_stage[k] = nullptr;
-    h->icp.rows = nullptr; h->icp.row_of = nullptr; h->icp.row_ep = nullptr; h->icp.n_rows = 0; h->icp.assign = 0;
-    h->own_stream = nullptr; h->ev_last = nullptr; h->ev_valid = 0;
-    cudaError_t e = cudaSetDevice(device);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->ev_last, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&h->sm_count, cudaDevAttrMultiProcessorCount, device);
+    h->noise_split = -1;        // (the handle is zero-initialised)
+    cudaError_t e = core_alloc(h, device, n_envs, OPNAV_ND, OPNAV_NI, OPNAV_IC_DIM, OST_N);
     if (e == cudaSuccess) e = cudaMalloc(&h->sched, sizeof(int) * 8);
     if (e == cudaSuccess) e = cudaMalloc(&h->perm, sizeof(int32_t) * h->stride);
     if (e == cudaSuccess) e = cudaMalloc(&h->mbuf, sizeof(double) * (size_t)opnav::opnav_meas_slots(h->P) * ON_MEAS_W * h->stride);
-    if (e == cudaSuccess) e = cudaMalloc(&h->S, sizeof(double) * OPNAV_ND * h->stride);
-    if (e == cudaSuccess) e = cudaMalloc(&h->I, sizeof(int64_t) * OPNAV_NI * h->stride);
-    if (e == cudaSuccess) e = cudaMalloc(&h->ics, sizeof(double) * OPNAV_IC_DIM * h->stride);
-    if (e == cudaSuccess) e = cudaMalloc(&h->stats, sizeof(double) * OST_N);
-    if (e == cudaSuccess) e = cudaMemset(h->S, 0, sizeof(double) * OPNAV_ND * h->stride);
-    if (e == cudaSuccess) e = cudaMemset(h->I, 0, sizeof(int64_t) * OPNAV_NI * h->stride);
-    if (e == cudaSuccess) e = cudaMemset(h->ics, 0, sizeof(double) * OPNAV_IC_DIM * h->stride);
-    if (e == cudaSuccess) e = cudaMemset(h->stats, 0, sizeof(double) * OST_N);
     if (e == cudaSuccess) {              // lane assignment starts as the identity (every slot names a valid env)
         opnav_perm_identity_kernel<<<(int)((h->stride + 255) / 256), 256>>>(h->perm, h->stride, h->n);
         e = cudaGetLastError();
@@ -512,11 +432,8 @@ int bskenv_opnav_destroy(bskenv_opnav_handle *h)
 {
     if (!h) return BSKENV_OK;
     cudaSetDevice(h->device);
-    cudaFree(h->S); cudaFree(h->I); cudaFree(h->ics); cudaFree(h->stats); cudaFree(h->sched); cudaFree(h->perm); cudaFree(h->d_eph); cudaFree(h->mbuf); cudaFree(h->nzbuf);
-    cudaFree((void *)h->icp.rows); cudaFree(h->icp.row_of); cudaFree(h->icp.row_ep);
-    if (h->own_stream) { cudaStreamSynchronize(h->own_stream); cudaStreamDestroy(h->own_stream); }
-    for (int k = 0; k < 6; k++) cudaFreeHost(h->h_stage[k]);
-    if (h->ev_last) cudaEventDestroy(h->ev_last);
+    cudaFree(h->sched); cudaFree(h->perm); cudaFree((void *)h->P.eph_sun.coef); cudaFree(h->mbuf); cudaFree(h->nzbuf);
+    core_free(h);
     delete h;
     return BSKENV_OK;
 }
@@ -524,33 +441,17 @@ int bskenv_opnav_destroy(bskenv_opnav_handle *h)
 int bskenv_opnav_set_ephemeris(bskenv_opnav_handle *h, double t0, double seg_len, int n_seg, int n_coef, const double *coef)
 {
     if (!h) return BSKENV_EINVAL;
-    ON_TRY(h, cudaSetDevice(h->device));
-    ON_TRY(h, cudaDeviceSynchronize());
-    LeoEph &E = h->P.eph_sun;
-    cudaFree(h->d_eph); h->d_eph = nullptr;
-    E.coef = nullptr; E.nseg = 0; E.ncoef = 0; E.t0 = 0.; E.seg_len = 0.;
-    if (n_seg <= 0) return BSKENV_OK;
-    if (!coef || n_coef < 1 || n_coef > 64 || !(seg_len > 0.)) { h->err = "bskenv_opnav_set_ephemeris: bad table shape"; return BSKENV_EINVAL; }
     const double t_end = ((double)h->P.max_length + 1.0) * (double)h->P.ticks_per_step * h->P.dt;   // max_length may be INT_MAX
-    if (t0 > 0. || t0 + seg_len * n_seg < t_end) {
-        h->err = "bskenv_opnav_set_ephemeris: the table does not cover one episode [0, (max_length + 1) * step_duration]";
-        return BSKENV_EINVAL;
-    }
-    const size_t bytes = sizeof(double) * (size_t)n_seg * 3 * (size_t)n_coef;
-    ON_TRY(h, cudaMalloc(&h->d_eph, bytes));
-    ON_TRY(h, cudaMemcpy(h->d_eph, coef, bytes, cudaMemcpyHostToDevice));
-    E.coef = h->d_eph; E.nseg = n_seg; E.ncoef = n_coef; E.t0 = t0; E.seg_len = seg_len;
-    return BSKENV_OK;
+    return set_ephemeris(h, "bskenv_opnav_set_ephemeris", h->P.eph_sun, t_end, t0, seg_len, n_seg, n_coef, coef);
 }
 
 static int opnav_do_reset(bskenv_opnav_handle *h, int mode, const double *ics_in, const uint8_t *mask, double *obs, void *stream)
 {
     if (!h) return BSKENV_EINVAL;
-    ON_TRY(h, cudaSetDevice(h->device));
-    const int grid = (int)((h->n + 255) / 256);
-    opnav_reset_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, mode, ics_in, mask, obs, h->icp);
-    ON_TRY(h, cudaGetLastError());
-    h->ev_valid = 1; ON_TRY(h, cudaEventRecord(h->ev_last, (cudaStream_t)stream));
+    CU_TRY(h, cudaSetDevice(h->device));
+    opnav_reset_kernel<<<env_grid(h), 256, 0, (cudaStream_t)stream>>>(h->P, h->S, h->I, h->ics, h->stride, h->n, mode, ics_in, mask, obs, h->icp);
+    CU_TRY(h, cudaGetLastError());
+    CU_TRY(h, note_launch(h, (cudaStream_t)stream));
     return BSKENV_OK;
 }
 int bskenv_opnav_reset_seeded(bskenv_opnav_handle *h, uint64_t seed, const uint8_t *mask_dev, double *obs_dev, void *stream)
@@ -570,55 +471,22 @@ int bskenv_opnav_reset_init(bskenv_opnav_handle *h, const uint8_t *mask_dev, dou
 }
 int bskenv_opnav_get_ics(bskenv_opnav_handle *h, double *ics_dev, void *stream)
 {
-    if (!h || !ics_dev) return BSKENV_EINVAL;
-    ON_TRY(h, cudaSetDevice(h->device));
-    opnav_gather_ics_kernel<<<(int)((h->n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->ics, h->stride, h->n, ics_dev);
-    ON_TRY(h, cudaGetLastError());
-    return BSKENV_OK;
+    return h ? get_ics<OPNAV_IC_DIM>(h, ics_dev, stream) : BSKENV_EINVAL;
 }
 
 int bskenv_opnav_set_ic_pool(bskenv_opnav_handle *h, int n_rows, const double *ics_host, int assign)
 {
     if (!h) return BSKENV_EINVAL;
-    if (n_rows < 0 || (n_rows > 0 && !ics_host)) { h->err = "bskenv_opnav_set_ic_pool: bad row count or null rows"; return BSKENV_EINVAL; }
-    if (n_rows > 0) {
-        if (assign != BSKENV_ICS_BY_INDEX && assign != BSKENV_ICS_PER_EPISODE) {
-            h->err = "bskenv_opnav_set_ic_pool: unknown assignment mode (the opNav batch has no parameter pool to pair with)";
-            return BSKENV_EINVAL;
-        }
-        for (int r = 0; r < n_rows; r++) {
-            const std::string err = leo_host::ic_row_check(ics_host + (size_t)r * BSKENV_OPNAV_IC_DIM, BSKENV_OPNAV_IC_DIM);
-            if (!err.empty()) { h->err = "bskenv_opnav_set_ic_pool: row " + std::to_string(r) + ": " + err; return BSKENV_EINVAL; }
-        }
-    }
-    ON_TRY(h, cudaSetDevice(h->device));
-    ON_TRY(h, cudaDeviceSynchronize());                         // a launch in flight may still read the old pool
-    cudaFree((void *)h->icp.rows);
-    h->icp.rows = nullptr; h->icp.n_rows = 0;
-    if (n_rows == 0) return BSKENV_OK;
-    if (!h->icp.row_of) {
-        ON_TRY(h, cudaMalloc(&h->icp.row_of, sizeof(int32_t) * h->stride));
-        ON_TRY(h, cudaMalloc(&h->icp.row_ep, sizeof(int64_t) * h->stride));
-        ON_TRY(h, cudaMemset(h->icp.row_of, 0xFF, sizeof(int32_t) * h->stride));
-        ON_TRY(h, cudaMemset(h->icp.row_ep, 0, sizeof(int64_t) * h->stride));
-    }
-    double *d_rows = nullptr;
-    const size_t bytes = sizeof(double) * (size_t)n_rows * BSKENV_OPNAV_IC_DIM;
-    ON_TRY(h, cudaMalloc(&d_rows, bytes));
-    ON_TRY(h, cudaMemcpy(d_rows, ics_host, bytes, cudaMemcpyHostToDevice));
-    h->icp.rows = d_rows; h->icp.n_rows = n_rows; h->icp.assign = assign;
-    return BSKENV_OK;
+    return set_ic_pool(h, "bskenv_opnav_set_ic_pool", n_rows, ics_host, BSKENV_OPNAV_IC_DIM, assign, [&]() -> std::string {
+        if (assign != BSKENV_ICS_BY_INDEX && assign != BSKENV_ICS_PER_EPISODE)
+            return "bskenv_opnav_set_ic_pool: unknown assignment mode (the opNav batch has no parameter pool to pair with)";
+        return "";
+    });
 }
 
 int bskenv_opnav_get_ic_rows(bskenv_opnav_handle *h, int32_t *rows_dev, void *stream)
 {
-    if (!h || !rows_dev) { if (h) h->err = "bskenv_opnav_get_ic_rows: null rows"; return BSKENV_EINVAL; }
-    ON_TRY(h, cudaSetDevice(h->device));
-    if (!h->icp.row_of) ON_TRY(h, cudaMemsetAsync(rows_dev, 0xFF, sizeof(int32_t) * h->n, (cudaStream_t)stream));
-    else opnav_gather_ic_rows_kernel<<<(int)((h->n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->icp.row_of, h->icp.row_ep,
-                                                                                                  h->I + (size_t)OI_EPISODE * h->stride, h->n, rows_dev);
-    ON_TRY(h, cudaGetLastError());
-    return BSKENV_OK;
+    return h ? get_ic_rows(h, "bskenv_opnav_get_ic_rows", OI_EPISODE, rows_dev, stream) : BSKENV_EINVAL;
 }
 
 int bskenv_opnav_step(bskenv_opnav_handle *h, const int32_t *actions_dev, double *obs_dev, double *reward_dev, uint8_t *done_dev,
@@ -626,7 +494,7 @@ int bskenv_opnav_step(bskenv_opnav_handle *h, const int32_t *actions_dev, double
 {
     if (!h) return BSKENV_EINVAL;
     if (!actions_dev || !obs_dev || !reward_dev || !done_dev || !done_reason_dev) { h->err = "bskenv_opnav_step: null buffer"; return BSKENV_EINVAL; }
-    ON_TRY(h, cudaSetDevice(h->device));
+    CU_TRY(h, cudaSetDevice(h->device));
     return opnav_launch_step(h, actions_dev, obs_dev, reward_dev, done_dev, done_reason_dev, debug_dev, term_obs_dev, (cudaStream_t)stream);
 }
 
@@ -637,48 +505,36 @@ int bskenv_opnav_step_info(bskenv_opnav_handle *h, const int32_t *actions_dev, d
     if (!h) return BSKENV_EINVAL;
     if (!actions_dev || !obs_dev || !reward_dev || !done_dev || !done_reason_dev) { h->err = "bskenv_opnav_step_info: null buffer"; return BSKENV_EINVAL; }
     if ((ep_return_dev == nullptr) != (ep_length_dev == nullptr)) { h->err = "bskenv_opnav_step_info: ep_return and ep_length go together"; return BSKENV_EINVAL; }
-    ON_TRY(h, cudaSetDevice(h->device));
+    CU_TRY(h, cudaSetDevice(h->device));
     return opnav_launch_step(h, actions_dev, obs_dev, reward_dev, done_dev, done_reason_dev, debug_dev, term_obs_dev, (cudaStream_t)stream,
                              ep_return_dev, ep_length_dev);
 }
 
-// Host-buffer entry point: zero-copy, as bskenv_step_host (bskenv.cu) -- the kernel reads the actions from and writes its
-// results to page-locked host memory directly; pageable caller buffers go through staging owned by the handle.
-static int opnav_host_map(bskenv_opnav_handle *h, const void *user, size_t bytes, int slot, void **dev, void **stage)
-{
-    *stage = nullptr;
-    cudaPointerAttributes a;
-    if (cudaPointerGetAttributes(&a, user) == cudaSuccess && a.type == cudaMemoryTypeHost && a.devicePointer) { *dev = a.devicePointer; return BSKENV_OK; }
-    cudaGetLastError();
-    if (!h->h_stage[slot]) ON_TRY(h, cudaHostAlloc(&h->h_stage[slot], bytes, cudaHostAllocMapped));
-    *stage = h->h_stage[slot];
-    ON_TRY(h, cudaHostGetDevicePointer(dev, *stage, 0));
-    return BSKENV_OK;
-}
+// Host-buffer entry point: zero-copy (batch_common.cuh: host_map), complete when it returns.
 
 int bskenv_opnav_step_host(bskenv_opnav_handle *h, const int32_t *actions, double *obs, double *reward, uint8_t *done,
                            uint8_t *done_reason, double *debug)
 {
     if (!h) return BSKENV_EINVAL;
     if (!actions || !obs || !reward || !done || !done_reason) { h->err = "bskenv_opnav_step_host: null buffer"; return BSKENV_EINVAL; }
-    ON_TRY(h, cudaSetDevice(h->device));
+    CU_TRY(h, cudaSetDevice(h->device));
     const size_t n = (size_t)h->n;
-    if (!h->own_stream) ON_TRY(h, cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
+    if (!h->own_stream) CU_TRY(h, cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
     cudaStream_t st = h->own_stream;
     void *user[6] = {(void *)actions, obs, reward, done, done_reason, debug};
     const size_t bytes[6] = {n * sizeof(int32_t), n * 4 * sizeof(double), n * sizeof(double), n, n, n * 12 * sizeof(double)};
     void *dev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr}, *stage[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     for (int k = 0; k < 6; k++) {
         if (!user[k]) continue;
-        int rc = opnav_host_map(h, user[k], bytes[k], k, &dev[k], &stage[k]);
+        int rc = host_map(h, user[k], bytes[k], k, &dev[k], &stage[k]);
         if (rc) return rc;
     }
     if (stage[0]) memcpy(stage[0], actions, bytes[0]);
-    if (h->ev_valid) ON_TRY(h, cudaStreamWaitEvent(st, h->ev_last, 0));     // after the caller's device-buffer steps / resets
+    if (h->ev_valid) CU_TRY(h, cudaStreamWaitEvent(st, h->ev_last, 0));     // after the caller's device-buffer steps / resets
     int rc = opnav_launch_step(h, (const int32_t *)dev[0], (double *)dev[1], (double *)dev[2], (uint8_t *)dev[3], (uint8_t *)dev[4],
                                (double *)dev[5], nullptr, st);
     if (rc) return rc;
-    ON_TRY(h, cudaStreamSynchronize(st));
+    CU_TRY(h, cudaStreamSynchronize(st));
     for (int k = 1; k < 6; k++)
         if (stage[k]) memcpy(user[k], stage[k], bytes[k]);
     return BSKENV_OK;
@@ -693,29 +549,15 @@ int bskenv_opnav_state_dims(const bskenv_opnav_handle *h, int32_t *nd, int32_t *
 }
 int bskenv_opnav_get_state(bskenv_opnav_handle *h, double *dstate_dev, int64_t *istate_dev, void *stream)
 {
-    if (!h) return BSKENV_EINVAL;
-    ON_TRY(h, cudaSetDevice(h->device));
-    const int grid = (int)((h->n + 255) / 256);
-    if (dstate_dev) opnav_copy_fields_kernel<double><<<grid, 256, 0, (cudaStream_t)stream>>>(h->S, h->stride, dstate_dev, h->n, h->n, OPNAV_ND);
-    if (istate_dev) opnav_copy_fields_kernel<int64_t><<<grid, 256, 0, (cudaStream_t)stream>>>(h->I, h->stride, istate_dev, h->n, h->n, OPNAV_NI);
-    ON_TRY(h, cudaGetLastError());
-    return BSKENV_OK;
+    return h ? get_state(h, OPNAV_ND, OPNAV_NI, dstate_dev, istate_dev, stream) : BSKENV_EINVAL;
 }
 int bskenv_opnav_set_state(bskenv_opnav_handle *h, const double *dstate_dev, const int64_t *istate_dev, void *stream)
 {
-    if (!h) return BSKENV_EINVAL;
-    ON_TRY(h, cudaSetDevice(h->device));
-    const int grid = (int)((h->n + 255) / 256);
-    if (dstate_dev) opnav_copy_fields_kernel<double><<<grid, 256, 0, (cudaStream_t)stream>>>(dstate_dev, h->n, h->S, h->stride, h->n, OPNAV_ND);
-    if (istate_dev) opnav_copy_fields_kernel<int64_t><<<grid, 256, 0, (cudaStream_t)stream>>>(istate_dev, h->n, h->I, h->stride, h->n, OPNAV_NI);
-    ON_TRY(h, cudaGetLastError());
-    h->ev_valid = 1; ON_TRY(h, cudaEventRecord(h->ev_last, (cudaStream_t)stream));
-    return BSKENV_OK;
+    return h ? set_state(h, OPNAV_ND, OPNAV_NI, dstate_dev, istate_dev, stream) : BSKENV_EINVAL;
 }
 int bskenv_opnav_state_field(const char *name, int32_t *is_int)
 {
-    struct Ent { const char *n; int idx; int is_int; };
-    static const Ent tab[] = {
+    static const FieldEnt tab[] = {
         {"r_BN_N", OF_R, 0}, {"v_BN_N", OF_V, 0}, {"sigma_BN", OF_SIG, 0}, {"omega_BN_B", OF_OMG, 0}, {"Omega", OF_WHL, 0},
         {"reactionwheel_cmds", OF_RWCMD, 0}, {"navErrors", OF_NAVERR, 0}, {"sun_point_data", OF_SUNPT, 0},
         {"shadowFactor", OF_SHADOW, 0}, {"filter_state", OF_FSTATE, 0}, {"filter_sBar", OF_FS, 0},
@@ -724,20 +566,12 @@ int bskenv_opnav_state_field(const char *name, int32_t *is_int)
         {"modeCounter", OI_MODECNT, 1}, {"first_run", OI_FIRST, 1}, {"MRPSwitchCount", OI_SWITCH, 1}, {"episode", OI_EPISODE, 1},
         {"episode_over", OI_OVER, 1}, {"n_meas", OI_NMEAS, 1}, {"n_bad", OI_NBAD, 1}, {"filter_tick", OI_FTICK, 1},
         {"sun_point_written", OI_SUNPT_W, 1}, {"n_images", OI_NIMG, 1}};
-    if (!name) return -1;
-    for (const Ent &t : tab)
-        if (!strcmp(t.n, name)) { if (is_int) *is_int = t.is_int; return t.idx; }
-    return -1;
+    return state_field(tab, name, is_int);
 }
 
 int bskenv_opnav_episode_stats(bskenv_opnav_handle *h, double *stats_host)
 {
-    if (!h || !stats_host) return BSKENV_EINVAL;
-    ON_TRY(h, cudaSetDevice(h->device));
-    ON_TRY(h, cudaDeviceSynchronize());
-    ON_TRY(h, cudaMemcpy(stats_host, h->stats, sizeof(double) * OST_N, cudaMemcpyDeviceToHost));
-    ON_TRY(h, cudaMemset(h->stats, 0, sizeof(double) * OST_N));
-    return BSKENV_OK;
+    return (h && stats_host) ? episode_stats(h, OST_N, stats_host) : BSKENV_EINVAL;
 }
 
 }  // extern "C"

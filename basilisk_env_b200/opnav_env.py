@@ -15,9 +15,8 @@ import ctypes as C
 import numpy as np
 import torch
 
-from . import _native
 from . import spaces
-from .vec_env import BskEnvError, all_reduce_stats
+from .vec_env import BatchVecEnv, BskEnvError
 
 OBS_DIM, DEBUG_DIM, IC_DIM = 4, 12, 12
 DONE_MAXLEN, DONE_MODES = 1, 2
@@ -53,73 +52,23 @@ def configure_initial_conditions(rng=None):
     return np.concatenate([rN, vN, rError, vError])
 
 
-class OpNavVecEnv:
+class OpNavVecEnv(BatchVecEnv):
     """N opNav environments on one GPU (see LeoPowerAttVecEnv for the conventions).
 
     **config : overrides of `bskenv_opnav_config` fields (include/bskenv.h), e.g. camera_reenable=1."""
+    _abi = "bskenv_opnav_"
+    OBS_DIM, IC_DIM, STAT_NAMES = OBS_DIM, IC_DIM, STAT_NAMES
+    IC_ASSIGN = {"by_index": 0, "per_episode": 1}
+    FIELD_WIDTH = {"r_BN_N": 3, "v_BN_N": 3, "sigma_BN": 3, "omega_BN_B": 3, "Omega": 4, "reactionwheel_cmds": 4,
+                   "navErrors": 15, "sun_point_data": 3, "filter_state": 6, "filter_sBar": 21, "sim_obs": 4, "sim_states": 12}
 
     def __init__(self, num_envs, device=0, first_env_index=0, seed=0, auto_reset=False, **config):
-        if not torch.cuda.is_available():
-            raise BskEnvError("OpNavVecEnv needs a CUDA device: the environment step has no CPU path")
-        self.device = torch.device("cuda", device) if isinstance(device, int) else torch.device(device)
-        if self.device.type != "cuda":
-            raise BskEnvError("OpNavVecEnv needs a CUDA device: the environment step has no CPU path")
-        self.num_envs = int(num_envs)
-        self.first_env_index = int(first_env_index)
-        self.seed_value = int(seed)
-        self._L = _native.lib()
-        config.setdefault("noise_seed", self.seed_value & (2**64 - 1))
-        self.cfg = _native.opnav_default_config(auto_reset=int(bool(auto_reset)), **config)
-        self.auto_reset = bool(auto_reset)
-        h = C.c_void_p()
-        dev_index = self.device.index if self.device.index is not None else torch.cuda.current_device()
-        rc = self._L.bskenv_opnav_create(C.byref(self.cfg), dev_index, self.num_envs, self.first_env_index, C.byref(h))
-        if rc != 0:
-            raise BskEnvError(f"bskenv_opnav_create failed ({rc}): {self._L.bskenv_opnav_last_error(None).decode()}")
-        self._h = h
-        n = self.num_envs
+        config.setdefault("noise_seed", int(seed) & (2**64 - 1))
+        super().__init__(num_envs, device, first_env_index, seed, auto_reset, config)
         with torch.cuda.device(self.device):
-            self.obs = torch.zeros((n, OBS_DIM), dtype=torch.float64, device=self.device)
-            self.term_obs = torch.zeros((n, OBS_DIM), dtype=torch.float64, device=self.device)
-            self.debug = torch.zeros((n, DEBUG_DIM), dtype=torch.float64, device=self.device)
-            self.reward = torch.zeros(n, dtype=torch.float64, device=self.device)
-            self.done = torch.zeros(n, dtype=torch.uint8, device=self.device)
-            self.done_reason = torch.zeros(n, dtype=torch.uint8, device=self.device)
-            self.episode_r = torch.zeros(n, dtype=torch.float64, device=self.device)
-            self.episode_l = torch.zeros(n, dtype=torch.int64, device=self.device)
-        self.observation_space = spaces.Box(-1e16, 1e16, shape=(OBS_DIM, 1))
+            self.debug = torch.zeros((self.num_envs, DEBUG_DIM), dtype=torch.float64, device=self.device)
         self.action_space = spaces.Discrete(2)
-        self.max_length = int(self.cfg.max_length)
         self.step_duration = float(self.cfg.step_duration_min)
-        nd, ni = C.c_int32(), C.c_int32()
-        self._L.bskenv_opnav_state_dims(self._h, C.byref(nd), C.byref(ni))
-        self.n_double_fields, self.n_int_fields = nd.value, ni.value
-
-    def close(self):
-        if getattr(self, "_h", None) is not None and self._h.value:
-            self._L.bskenv_opnav_destroy(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def _check(self, rc, what):
-        if rc != 0:
-            raise BskEnvError(f"{what} failed ({rc}): {self._L.bskenv_opnav_last_error(self._h).decode()}")
-
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-
-    def _mask_ptr(self, mask):
-        if mask is None:
-            return None, None
-        m = torch.as_tensor(mask).to(device=self.device, dtype=torch.uint8).contiguous()
-        if m.numel() != self.num_envs:
-            raise ValueError("mask must have one entry per env")
-        return m, C.c_void_p(m.data_ptr())
 
     def set_ephemeris(self, table):
         """SURVEY 8(f)-4: Sun position relative to the Mars barycentre [m] from a Chebyshev table
@@ -130,63 +79,6 @@ class OpNavVecEnv:
         coef = np.ascontiguousarray(table.coef, dtype=np.float64)
         self._check(self._L.bskenv_opnav_set_ephemeris(self._h, float(table.t0), float(table.seg_len), coef.shape[0],
                                                        coef.shape[2], coef.ctypes.data), "set_ephemeris")
-
-    def set_ic_pool(self, ics, assign="per_episode"):
-        """Load a pool of initial conditions [K, 12] (rN vN rError vError) that `reset()` and the auto-reset of `step` draw
-        from instead of the built-in sampler (include/bskenv.h: bskenv_opnav_set_ic_pool); None unloads it.
-        assign : "per_episode" (row drawn per (seed, global env index, episode)) or "by_index" (global env index mod K)."""
-        if ics is None:
-            self._check(self._L.bskenv_opnav_set_ic_pool(self._h, 0, None, 0), "bskenv_opnav_set_ic_pool")
-            return
-        rows = ics.detach().cpu().numpy() if torch.is_tensor(ics) else ics
-        rows = np.ascontiguousarray(rows, dtype=np.float64)
-        if rows.ndim != 2 or rows.shape[1] != IC_DIM or rows.shape[0] == 0:
-            raise ValueError(f"ics must have shape (K, {IC_DIM}) with K > 0")
-        self._check(self._L.bskenv_opnav_set_ic_pool(self._h, rows.shape[0], rows.ctypes.data, IC_ASSIGN[assign]),
-                    "bskenv_opnav_set_ic_pool")
-
-    def ic_rows(self):
-        """The IC-pool row each env's current episode started from (int32 [N]; -1 = sampled or explicit ICs)."""
-        row = torch.empty(self.num_envs, dtype=torch.int32, device=self.device)
-        self._check(self._L.bskenv_opnav_get_ic_rows(self._h, C.c_void_p(row.data_ptr()), self._stream()),
-                    "bskenv_opnav_get_ic_rows")
-        return row
-
-    def reset(self, seed=None, mask=None):
-        """Sample fresh initial conditions on the device; returns the initial observation [N,4] (zeros)."""
-        if seed is not None:
-            self.seed_value = int(seed)
-        keep, mp = self._mask_ptr(mask)
-        self._check(self._L.bskenv_opnav_reset_seeded(self._h, C.c_uint64(self.seed_value & (2**64 - 1)), mp,
-                                                      C.c_void_p(self.obs.data_ptr()), self._stream()),
-                    "bskenv_opnav_reset_seeded")
-        del keep
-        return self.obs
-
-    def reset_ics(self, ics, mask=None):
-        """Reset from explicit initial conditions: [N,12] rows [rN vN rError vError]."""
-        t = torch.as_tensor(np.asarray(ics, dtype=np.float64) if not torch.is_tensor(ics) else ics)
-        t = t.to(device=self.device, dtype=torch.float64).contiguous()
-        if tuple(t.shape) != (self.num_envs, IC_DIM):
-            raise ValueError(f"ics must have shape ({self.num_envs}, {IC_DIM})")
-        keep, mp = self._mask_ptr(mask)
-        self._check(self._L.bskenv_opnav_reset_ics(self._h, C.c_void_p(t.data_ptr()), mp, C.c_void_p(self.obs.data_ptr()),
-                                                   self._stream()), "bskenv_opnav_reset_ics")
-        torch.cuda.current_stream(self.device).synchronize()
-        del keep
-        return self.obs
-
-    def reset_init(self, mask=None):
-        keep, mp = self._mask_ptr(mask)
-        self._check(self._L.bskenv_opnav_reset_init(self._h, mp, C.c_void_p(self.obs.data_ptr()), self._stream()),
-                    "bskenv_opnav_reset_init")
-        del keep
-        return self.obs
-
-    def initial_conditions(self):
-        out = torch.empty((self.num_envs, IC_DIM), dtype=torch.float64, device=self.device)
-        self._check(self._L.bskenv_opnav_get_ics(self._h, C.c_void_p(out.data_ptr()), self._stream()), "bskenv_opnav_get_ics")
-        return out
 
     def step(self, actions):
         """actions: int32 CUDA tensor [N] (0 OpNav pointing + imaging / 1 sun-safe pointing).  Returns device tensors
@@ -230,45 +122,6 @@ class OpNavVecEnv:
                                                    reason.ctypes.data, dbg.ctypes.data if dbg is not None else None),
                     "bskenv_opnav_step_host")
         return obs, rew, done, reason, dbg
-
-    def get_state(self):
-        d = torch.empty((self.n_double_fields, self.num_envs), dtype=torch.float64, device=self.device)
-        i = torch.empty((self.n_int_fields, self.num_envs), dtype=torch.int64, device=self.device)
-        self._check(self._L.bskenv_opnav_get_state(self._h, C.c_void_p(d.data_ptr()), C.c_void_p(i.data_ptr()),
-                                                   self._stream()), "bskenv_opnav_get_state")
-        return d, i
-
-    def set_state(self, dstate, istate):
-        d = dstate.to(device=self.device, dtype=torch.float64).contiguous()
-        i = istate.to(device=self.device, dtype=torch.int64).contiguous()
-        if tuple(d.shape) != (self.n_double_fields, self.num_envs) or tuple(i.shape) != (self.n_int_fields, self.num_envs):
-            raise ValueError("state blocks have the wrong shape")
-        self._check(self._L.bskenv_opnav_set_state(self._h, C.c_void_p(d.data_ptr()), C.c_void_p(i.data_ptr()),
-                                                   self._stream()), "bskenv_opnav_set_state")
-        torch.cuda.current_stream(self.device).synchronize()
-
-    def field(self, name, state=None):
-        idx, is_int = _native.opnav_state_field(name)
-        d, i = state if state is not None else self.get_state()
-        return (i if is_int else d)[idx:idx + _FIELD_WIDTH.get(name, 1)]
-
-    def episode_stats(self, all_reduce=False):
-        buf = np.zeros(8)
-        self._check(self._L.bskenv_opnav_episode_stats(self._h, buf.ctypes.data), "bskenv_opnav_episode_stats")
-        if all_reduce:
-            buf = all_reduce_stats(buf, self.device)
-        return dict(zip(STAT_NAMES, (float(x) for x in buf)))
-
-    def launch_count(self):
-        return int(self._L.bskenv_opnav_launch_count(self._h))
-
-    def flops_per_step(self):
-        return float(self._L.bskenv_opnav_flops_per_step(self._h))
-
-
-IC_ASSIGN = {"by_index": 0, "per_episode": 1}
-_FIELD_WIDTH = {"r_BN_N": 3, "v_BN_N": 3, "sigma_BN": 3, "omega_BN_B": 3, "Omega": 4, "reactionwheel_cmds": 4,
-                "navErrors": 15, "sun_point_data": 3, "filter_state": 6, "filter_sBar": 21, "sim_obs": 4, "sim_states": 12}
 
 
 class scenario_OpNav:

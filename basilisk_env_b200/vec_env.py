@@ -17,6 +17,13 @@ DONE_MAXLEN, DONE_WHEEL, DONE_POWER, DONE_DECAY = 1, 2, 4, 8
 OBS_DIM, IC_DIM = 5, 19
 STAT_NAMES = ("return_sum", "length_sum", "episodes", "wheel_failures", "power_failures", "orbit_decays",
               "max_length_ends", "env_steps")
+ORGANISATIONS = {"auto": 0, "thread": 1, "split": 2, "thread_index": 3}
+PARAM_ASSIGN = {"by_index": 0, "per_episode": 1}
+IC_ASSIGN = {"by_index": 0, "per_episode": 1, "param_row": 2}
+_FIELD_WIDTH = {"r_BN_N": 3, "v_BN_N": 3, "sigma_BN": 3, "omega_BN_B": 3, "Omega": 4, "u_current": 4,
+                "extTorquePntB_B": 3, "att_guidance": 12, "att_reference": 9, "commandedControlTorque": 3,
+                "rwTorqueCommand": 4, "wheelDeltaH": 3, "ThrustOnCmd": 8, "thrOnTimeRemaining": 8, "OnTimeRequest": 8,
+                "sim_obs": 5, "fireCounter": 8}
 
 
 class BskEnvError(RuntimeError):
@@ -32,7 +39,175 @@ def shard_range(num_envs_total, rank, world_size):
     return lo, lo + base + (1 if rank < rem else 0)
 
 
-class LeoPowerAttVecEnv:
+class BatchVecEnv:
+    """What the LEO and the opNav batch share: one handle of the batch's C ABI (`_abi`: the prefix of its entry points), the
+    device output buffers, resets, the IC pool, the persistent state and the episode statistics.  A subclass sets the class
+    attributes below, `action_space` and `step_duration`, and adds its step."""
+    _abi = ""                   # "bskenv_" or "bskenv_opnav_"
+    OBS_DIM = IC_DIM = 0
+    IC_ASSIGN = {}
+    STAT_NAMES = ()
+    FIELD_WIDTH = {}
+
+    def __init__(self, num_envs, device, first_env_index, seed, auto_reset, config):
+        if not torch.cuda.is_available():
+            raise BskEnvError(f"{type(self).__name__} needs a CUDA device: the environment step has no CPU path")
+        self.device = torch.device("cuda", device) if isinstance(device, int) else torch.device(device)
+        if self.device.type != "cuda":
+            raise BskEnvError(f"{type(self).__name__} needs a CUDA device: the environment step has no CPU path")
+        self.num_envs = int(num_envs)
+        self.first_env_index = int(first_env_index)
+        self.seed_value = int(seed)
+        self._L = _native.lib()
+        self._f = _native.batch_abi(self._abi)
+        self.cfg = _native.batch_config(self._abi, auto_reset=int(bool(auto_reset)), **config)
+        self.auto_reset = bool(auto_reset)
+        h = C.c_void_p()
+        dev_index = self.device.index if self.device.index is not None else torch.cuda.current_device()
+        rc = self._f.create(C.byref(self.cfg), dev_index, self.num_envs, self.first_env_index, C.byref(h))
+        if rc != 0:
+            raise BskEnvError(f"{self._f.create.__name__} failed ({rc}): {self._f.last_error(None).decode()}")
+        self._h = h
+        n = self.num_envs
+        with torch.cuda.device(self.device):
+            self.obs = torch.zeros((n, self.OBS_DIM), dtype=torch.float64, device=self.device)
+            self.term_obs = torch.zeros((n, self.OBS_DIM), dtype=torch.float64, device=self.device)
+            self.reward = torch.zeros(n, dtype=torch.float64, device=self.device)
+            self.done = torch.zeros(n, dtype=torch.uint8, device=self.device)
+            self.done_reason = torch.zeros(n, dtype=torch.uint8, device=self.device)
+            # per env: the reference's reward_total and curr_step, the `info['episode']` record where done
+            self.episode_r = torch.zeros(n, dtype=torch.float64, device=self.device)
+            self.episode_l = torch.zeros(n, dtype=torch.int64, device=self.device)
+        self.observation_space = spaces.Box(-1e16, 1e16, shape=(self.OBS_DIM, 1))
+        self.max_length = int(self.cfg.max_length)
+        nd, ni = C.c_int32(), C.c_int32()
+        self._f.state_dims(self._h, C.byref(nd), C.byref(ni))
+        self.n_double_fields, self.n_int_fields = nd.value, ni.value
+
+    # ------------------------------------------------------------------------------------------
+    def close(self):
+        if getattr(self, "_h", None) is not None and self._h.value:
+            self._f.destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _check(self, rc, what):
+        if rc != 0:
+            raise BskEnvError(f"{what} failed ({rc}): {self._f.last_error(self._h).decode()}")
+
+    def _call(self, fn, *args):
+        self._check(fn(*args), fn.__name__)
+
+    def _stream(self):
+        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    def _mask_ptr(self, mask):
+        if mask is None:
+            return None, None
+        m = torch.as_tensor(mask).to(device=self.device, dtype=torch.uint8).contiguous()
+        if m.numel() != self.num_envs:
+            raise ValueError("mask must have one entry per env")
+        return m, C.c_void_p(m.data_ptr())
+
+    # ------------------------------------------------------------------------------------------
+    def set_ic_pool(self, ics, assign="per_episode"):
+        """Load a pool of initial conditions [K, IC_DIM] that `reset()` and the auto-reset of `step` draw from instead of the
+        built-in sampler (include/bskenv.h: bskenv_set_ic_pool); None unloads it.
+        assign : "per_episode" (row drawn per (seed, global env index, episode)) or "by_index" (global env index mod K)."""
+        if ics is None:
+            self._call(self._f.set_ic_pool, self._h, 0, None, 0)
+            return
+        rows = ics.detach().cpu().numpy() if torch.is_tensor(ics) else ics
+        rows = np.ascontiguousarray(rows, dtype=np.float64)
+        if rows.ndim != 2 or rows.shape[1] != self.IC_DIM or rows.shape[0] == 0:
+            raise ValueError(f"ics must have shape (K, {self.IC_DIM}) with K > 0")
+        self._call(self._f.set_ic_pool, self._h, rows.shape[0], rows.ctypes.data, self.IC_ASSIGN[assign])
+
+    def ic_rows(self):
+        """The IC-pool row each env's current episode started from (int32 [N]; -1 = sampled or explicit ICs)."""
+        row = torch.empty(self.num_envs, dtype=torch.int32, device=self.device)
+        self._call(self._f.get_ic_rows, self._h, C.c_void_p(row.data_ptr()), self._stream())
+        return row
+
+    def reset(self, seed=None, mask=None):
+        """Sample fresh initial conditions on the device (or draw them from the IC pool) and return the initial
+        observation [N, OBS_DIM]."""
+        if seed is not None:
+            self.seed_value = int(seed)
+        keep, mp = self._mask_ptr(mask)
+        self._call(self._f.reset_seeded, self._h, C.c_uint64(self.seed_value & (2**64 - 1)), mp, C.c_void_p(self.obs.data_ptr()),
+                   self._stream())
+        del keep
+        return self.obs
+
+    def reset_ics(self, ics, mask=None):
+        """Reset from explicit initial conditions: [N, IC_DIM] rows."""
+        t = torch.as_tensor(np.asarray(ics, dtype=np.float64) if not torch.is_tensor(ics) else ics)
+        t = t.to(device=self.device, dtype=torch.float64).contiguous()
+        if tuple(t.shape) != (self.num_envs, self.IC_DIM):
+            raise ValueError(f"ics must have shape ({self.num_envs}, {self.IC_DIM})")
+        keep, mp = self._mask_ptr(mask)
+        self._call(self._f.reset_ics, self._h, C.c_void_p(t.data_ptr()), mp, C.c_void_p(self.obs.data_ptr()), self._stream())
+        torch.cuda.current_stream(self.device).synchronize()   # `t` may be a temporary
+        del keep
+        return self.obs
+
+    def reset_init(self, mask=None):
+        """Rebuild every (masked) env from its stored initial conditions."""
+        keep, mp = self._mask_ptr(mask)
+        self._call(self._f.reset_init, self._h, mp, C.c_void_p(self.obs.data_ptr()), self._stream())
+        del keep
+        return self.obs
+
+    def initial_conditions(self):
+        out = torch.empty((self.num_envs, self.IC_DIM), dtype=torch.float64, device=self.device)
+        self._call(self._f.get_ics, self._h, C.c_void_p(out.data_ptr()), self._stream())
+        return out
+
+    # ------------------------------------------------------------------------------------------
+    def get_state(self):
+        """Whole persistent state (a checkpoint): (double [n_double_fields, N], int64 [n_int_fields, N])."""
+        d = torch.empty((self.n_double_fields, self.num_envs), dtype=torch.float64, device=self.device)
+        i = torch.empty((self.n_int_fields, self.num_envs), dtype=torch.int64, device=self.device)
+        self._call(self._f.get_state, self._h, C.c_void_p(d.data_ptr()), C.c_void_p(i.data_ptr()), self._stream())
+        return d, i
+
+    def set_state(self, dstate, istate):
+        d = dstate.to(device=self.device, dtype=torch.float64).contiguous()
+        i = istate.to(device=self.device, dtype=torch.int64).contiguous()
+        if tuple(d.shape) != (self.n_double_fields, self.num_envs) or tuple(i.shape) != (self.n_int_fields, self.num_envs):
+            raise ValueError("state blocks have the wrong shape")
+        self._call(self._f.set_state, self._h, C.c_void_p(d.data_ptr()), C.c_void_p(i.data_ptr()), self._stream())
+        torch.cuda.current_stream(self.device).synchronize()
+
+    def field(self, name, state=None):
+        """Named slice of the state, e.g. field("r_BN_N") -> [3, N]."""
+        idx, is_int = _native.batch_state_field(self._abi, name)
+        d, i = state if state is not None else self.get_state()
+        return (i if is_int else d)[idx:idx + self.FIELD_WIDTH.get(name, 1)]
+
+    def episode_stats(self, all_reduce=False):
+        """Episode statistics of this shard since the last call (dict of floats).  With `all_reduce`
+        the eight numbers are summed over the process group -- the only collective of the design."""
+        buf = np.zeros(8)
+        self._call(self._f.episode_stats, self._h, buf.ctypes.data)
+        if all_reduce:
+            buf = all_reduce_stats(buf, self.device)
+        return dict(zip(self.STAT_NAMES, (float(x) for x in buf)))
+
+    def launch_count(self):
+        return int(self._f.launch_count(self._h))
+
+    def flops_per_step(self):
+        return float(self._f.flops_per_step(self._h))
+
+
+class LeoPowerAttVecEnv(BatchVecEnv):
     """N environments on one GPU.
 
     Parameters
@@ -47,71 +222,15 @@ class LeoPowerAttVecEnv:
     organisation : "auto" | "thread" | "split": work organisation of the step kernel (see `set_organisation`).
     **config : overrides of `bskenv_config` fields (include/bskenv.h), e.g. step_duration=60.
     """
+    _abi = "bskenv_"
+    OBS_DIM, IC_DIM, IC_ASSIGN, STAT_NAMES, FIELD_WIDTH = OBS_DIM, IC_DIM, IC_ASSIGN, STAT_NAMES, _FIELD_WIDTH
 
     def __init__(self, num_envs, device=0, first_env_index=0, seed=0, auto_reset=False, organisation="auto", **config):
-        if not torch.cuda.is_available():
-            raise BskEnvError("LeoPowerAttVecEnv needs a CUDA device: the environment step has no CPU path")
-        self.device = torch.device("cuda", device) if isinstance(device, int) else torch.device(device)
-        if self.device.type != "cuda":
-            raise BskEnvError("LeoPowerAttVecEnv needs a CUDA device: the environment step has no CPU path")
-        self.num_envs = int(num_envs)
-        self.first_env_index = int(first_env_index)
-        self.seed_value = int(seed)
-        self._L = _native.lib()
-        self.cfg = _native.default_config(auto_reset=int(bool(auto_reset)), **config)
-        self.auto_reset = bool(auto_reset)
-        h = C.c_void_p()
-        dev_index = self.device.index if self.device.index is not None else torch.cuda.current_device()
-        rc = self._L.bskenv_create(C.byref(self.cfg), dev_index, self.num_envs, self.first_env_index, C.byref(h))
-        if rc != 0:
-            raise BskEnvError(f"bskenv_create failed ({rc}): {self._L.bskenv_last_error(None).decode()}")
-        self._h = h
-        n = self.num_envs
-        with torch.cuda.device(self.device):
-            self.obs = torch.zeros((n, OBS_DIM), dtype=torch.float64, device=self.device)
-            self.term_obs = torch.zeros((n, OBS_DIM), dtype=torch.float64, device=self.device)
-            self.reward = torch.zeros(n, dtype=torch.float64, device=self.device)
-            self.done = torch.zeros(n, dtype=torch.uint8, device=self.device)
-            self.done_reason = torch.zeros(n, dtype=torch.uint8, device=self.device)
-            # ENV:130-136 per env: reward_total and curr_step, the `info['episode']` record where done
-            self.episode_r = torch.zeros(n, dtype=torch.float64, device=self.device)
-            self.episode_l = torch.zeros(n, dtype=torch.int64, device=self.device)
-        self.observation_space = spaces.Box(-1e16, 1e16, shape=(OBS_DIM, 1))
+        super().__init__(num_envs, device, first_env_index, seed, auto_reset, config)
         self.action_space = spaces.Discrete(3)
-        self.max_length = int(self.cfg.max_length)
         self.step_duration = float(self.cfg.step_duration)
-        nd, ni = C.c_int32(), C.c_int32()
-        self._L.bskenv_state_dims(self._h, C.byref(nd), C.byref(ni))
-        self.n_double_fields, self.n_int_fields = nd.value, ni.value
         if organisation != "auto":
             self.set_organisation(organisation)
-
-    # ------------------------------------------------------------------------------------------
-    def close(self):
-        if getattr(self, "_h", None) is not None and self._h.value:
-            self._L.bskenv_destroy(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def _check(self, rc, what):
-        if rc != 0:
-            raise BskEnvError(f"{what} failed ({rc}): {self._L.bskenv_last_error(self._h).decode()}")
-
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-
-    def _mask_ptr(self, mask):
-        if mask is None:
-            return None, None
-        m = torch.as_tensor(mask).to(device=self.device, dtype=torch.uint8).contiguous()
-        if m.numel() != self.num_envs:
-            raise ValueError("mask must have one entry per env")
-        return m, C.c_void_p(m.data_ptr())
 
     # ------------------------------------------------------------------------------------------
     # ---- SURVEY 8(f)-4: ephemeris tables and the planet-fixed degree-2 field (set before reset) ----
@@ -182,25 +301,9 @@ class LeoPowerAttVecEnv:
             None to unload the pool.
         assign : "per_episode" (row drawn per (seed, global env index, episode)), "by_index" (row = global env index mod K)
             or "param_row" (row = the env's parameter-pool row: a scenario table, see `set_scenario_pool`)."""
-        if ics is None:
-            self._check(self._L.bskenv_set_ic_pool(self._h, 0, None, 0), "bskenv_set_ic_pool")
-            return
-        if torch.is_tensor(ics):
-            rows = ics.detach().cpu().numpy()
-        elif len(ics) and isinstance(ics[0], dict):
-            rows = np.stack([ic_row(ic) for ic in ics])
-        else:
-            rows = ics
-        rows = np.ascontiguousarray(rows, dtype=np.float64)
-        if rows.ndim != 2 or rows.shape[1] != IC_DIM or rows.shape[0] == 0:
-            raise ValueError(f"ics must have shape (K, {IC_DIM}) with K > 0")
-        self._check(self._L.bskenv_set_ic_pool(self._h, rows.shape[0], rows.ctypes.data, IC_ASSIGN[assign]), "bskenv_set_ic_pool")
-
-    def ic_rows(self):
-        """The IC-pool row each env's current episode started from (int32 [N]; -1 = sampled or explicit ICs)."""
-        row = torch.empty(self.num_envs, dtype=torch.int32, device=self.device)
-        self._check(self._L.bskenv_get_ic_rows(self._h, C.c_void_p(row.data_ptr()), self._stream()), "bskenv_get_ic_rows")
-        return row
+        if ics is not None and not torch.is_tensor(ics) and len(ics) and isinstance(ics[0], dict):
+            ics = np.stack([ic_row(ic) for ic in ics])
+        super().set_ic_pool(ics, assign)
 
     def set_scenario_pool(self, scenarios, assign="per_episode"):
         """Load K full reference `initial_conditions` dicts (the shape `initial_conditions.set_ICs()` returns) as a scenario
@@ -217,43 +320,6 @@ class LeoPowerAttVecEnv:
         self.set_param_pool(params, assign=assign)
         self.set_ic_pool(ics, assign="param_row")
 
-    def reset(self, seed=None, mask=None):
-        """Sample fresh initial conditions on the device and return the initial observation [N,5]."""
-        if seed is not None:
-            self.seed_value = int(seed)
-        keep, mp = self._mask_ptr(mask)
-        self._check(self._L.bskenv_reset_seeded(self._h, C.c_uint64(self.seed_value & (2**64 - 1)), mp,
-                                                C.c_void_p(self.obs.data_ptr()), self._stream()), "bskenv_reset_seeded")
-        del keep
-        return self.obs
-
-    def reset_ics(self, ics, mask=None):
-        """Reset from explicit initial conditions: [N,19] rows (see initial_conditions.ic_row)."""
-        t = torch.as_tensor(np.asarray(ics, dtype=np.float64) if not torch.is_tensor(ics) else ics)
-        t = t.to(device=self.device, dtype=torch.float64).contiguous()
-        if tuple(t.shape) != (self.num_envs, IC_DIM):
-            raise ValueError(f"ics must have shape ({self.num_envs}, {IC_DIM})")
-        keep, mp = self._mask_ptr(mask)
-        self._check(self._L.bskenv_reset_ics(self._h, C.c_void_p(t.data_ptr()), mp, C.c_void_p(self.obs.data_ptr()),
-                                             self._stream()), "bskenv_reset_ics")
-        torch.cuda.current_stream(self.device).synchronize()   # `t` may be a temporary
-        del keep
-        return self.obs
-
-    def reset_init(self, mask=None):
-        """Rebuild every (masked) env from its stored initial conditions (ENV:202-216)."""
-        keep, mp = self._mask_ptr(mask)
-        self._check(self._L.bskenv_reset_init(self._h, mp, C.c_void_p(self.obs.data_ptr()), self._stream()),
-                    "bskenv_reset_init")
-        del keep
-        return self.obs
-
-    def initial_conditions(self):
-        out = torch.empty((self.num_envs, IC_DIM), dtype=torch.float64, device=self.device)
-        self._check(self._L.bskenv_get_ics(self._h, C.c_void_p(out.data_ptr()), self._stream()), "bskenv_get_ics")
-        return out
-
-    # ------------------------------------------------------------------------------------------
     def step(self, actions):
         """actions: int32 CUDA tensor [N] (0 nadir / 1 sun / 2 desat).  Returns device tensors
         (obs [N,5] f64, reward [N] f64, done [N] u8, info) without synchronising."""
@@ -316,43 +382,6 @@ class LeoPowerAttVecEnv:
         self.step_host_async(actions, out)
         return self.step_host_wait()
 
-    # ------------------------------------------------------------------------------------------
-    def get_state(self):
-        """Whole persistent state (a checkpoint): (double [n_double_fields, N], int64 [n_int_fields, N])."""
-        d = torch.empty((self.n_double_fields, self.num_envs), dtype=torch.float64, device=self.device)
-        i = torch.empty((self.n_int_fields, self.num_envs), dtype=torch.int64, device=self.device)
-        self._check(self._L.bskenv_get_state(self._h, C.c_void_p(d.data_ptr()), C.c_void_p(i.data_ptr()), self._stream()),
-                    "bskenv_get_state")
-        return d, i
-
-    def set_state(self, dstate, istate):
-        d = dstate.to(device=self.device, dtype=torch.float64).contiguous()
-        i = istate.to(device=self.device, dtype=torch.int64).contiguous()
-        if tuple(d.shape) != (self.n_double_fields, self.num_envs) or tuple(i.shape) != (self.n_int_fields, self.num_envs):
-            raise ValueError("state blocks have the wrong shape")
-        self._check(self._L.bskenv_set_state(self._h, C.c_void_p(d.data_ptr()), C.c_void_p(i.data_ptr()), self._stream()),
-                    "bskenv_set_state")
-        torch.cuda.current_stream(self.device).synchronize()
-
-    def field(self, name, state=None):
-        """Named slice of the state, e.g. field("r_BN_N") -> [3, N]."""
-        idx, is_int = _native.state_field(name)
-        d, i = state if state is not None else self.get_state()
-        width = _FIELD_WIDTH.get(name, 1)
-        return (i if is_int else d)[idx:idx + width]
-
-    def episode_stats(self, all_reduce=False):
-        """Episode statistics of this shard since the last call (dict of floats).  With `all_reduce`
-        the eight numbers are summed over the process group -- the only collective of the design."""
-        buf = np.zeros(8)
-        self._check(self._L.bskenv_episode_stats(self._h, buf.ctypes.data), "bskenv_episode_stats")
-        if all_reduce:
-            buf = all_reduce_stats(buf, self.device)
-        return dict(zip(STAT_NAMES, (float(x) for x in buf)))
-
-    def launch_count(self):
-        return int(self._L.bskenv_launch_count(self._h))
-
     def kernel_name(self):
         """The step-kernel instantiation the last step launched (as ncu lists it)."""
         return self._L.bskenv_kernel_name(self._h).decode()
@@ -363,18 +392,6 @@ class LeoPowerAttVecEnv:
         organisation) or "thread_index" (one thread per env, lanes in index order: no bucketing).  Same arithmetic."""
         org = ORGANISATIONS[organisation] if isinstance(organisation, str) else int(organisation)
         self._check(self._L.bskenv_set_organisation(self._h, org), "bskenv_set_organisation")
-
-    def flops_per_step(self):
-        return float(self._L.bskenv_flops_per_step(self._h))
-
-
-ORGANISATIONS = {"auto": 0, "thread": 1, "split": 2, "thread_index": 3}
-PARAM_ASSIGN = {"by_index": 0, "per_episode": 1}
-IC_ASSIGN = {"by_index": 0, "per_episode": 1, "param_row": 2}
-_FIELD_WIDTH = {"r_BN_N": 3, "v_BN_N": 3, "sigma_BN": 3, "omega_BN_B": 3, "Omega": 4, "u_current": 4,
-                "extTorquePntB_B": 3, "att_guidance": 12, "att_reference": 9, "commandedControlTorque": 3,
-                "rwTorqueCommand": 4, "wheelDeltaH": 3, "ThrustOnCmd": 8, "thrOnTimeRemaining": 8, "OnTimeRequest": 8,
-                "sim_obs": 5, "fireCounter": 8}
 
 
 def all_reduce_stats(buf, device=None):
