@@ -1,6 +1,7 @@
 // batch_common.cuh -- the handle layer the LEO batch (bskenv.cu) and the opNav batch (opnav.cu) share: the handle core,
 // the IC choice of a reset, and the entry points around the step kernels that differ only in dimensions (create / destroy,
-// ephemeris tables, IC pools, stored ICs, state blocks, statistics, host-buffer mapping, launch ordering).
+// ephemeris tables, IC pools, stored ICs, state blocks, statistics, host-buffer mapping, launch ordering), the lane
+// bucketing before a step and the dynamic-shared-memory opt-in of the step kernels.
 #pragma once
 #include <cuda_runtime.h>
 #include <string.h>
@@ -10,11 +11,11 @@
 #include "leo_core.cuh"
 #include "leo_host.h"
 
-#define CU_TRY(h, call)                                                                              \
+#define CU_TRY(h, ...)         /* variadic: the call may name a template with several arguments */          \
     do {                                                                                             \
-        cudaError_t _e = (call);                                                                     \
+        cudaError_t _e = (__VA_ARGS__);                                                              \
         if (_e != cudaSuccess) {                                                                     \
-            (h)->err = std::string(#call) + ": " + cudaGetErrorString(_e);                            \
+            (h)->err = std::string(#__VA_ARGS__) + ": " + cudaGetErrorString(_e);                     \
             return BSKENV_ECUDA;                                                                     \
         }                                                                                            \
     } while (0)
@@ -95,7 +96,59 @@ __global__ void copy_fields_kernel(const T *__restrict__ src, int64_t src_stride
     for (int f = 0; f < fields; f++) dst[(int64_t)f * dst_stride + e] = src[(int64_t)f * src_stride + e];
 }
 
+// Lane bucketing before a step: a counting sort of the envs into the lane permutation `perm` of the step kernel, so that a
+// warp takes 32 envs of one bucket (warp-aggregated atomics, one count and one fill launch).  rank(e) = the position of env
+// e's bucket in the permutation, 0 .. NB - 1; bucket rank r starts after the sizes of all lower ranks.  bucket[0 .. NB-1] =
+// sizes, bucket[NB .. 2 NB-1] = cursors, zeroed before the count launch.  Within a bucket the envs of a warp are in index
+// order and the warps in the order they reach the cursor.
+template <int NB, class Rank>
+__global__ void __launch_bounds__(256) bucket_count_kernel(int64_t n, const Rank rank, int *__restrict__ bucket)
+{
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int r = e < n ? rank(e) : -1;
+#pragma unroll
+    for (int c = 0; c < NB; c++) {
+        const unsigned m = __ballot_sync(0xffffffffu, r == c);
+        if ((threadIdx.x & 31) == 0 && m) atomicAdd(&bucket[c], __popc(m));
+    }
+}
+template <int NB, class Rank>
+__global__ void __launch_bounds__(256) bucket_fill_kernel(int64_t n, const Rank rank, int *__restrict__ bucket, int32_t *__restrict__ perm)
+{
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int r = e < n ? rank(e) : -1;
+    const int lane = threadIdx.x & 31;
+    int size[NB];                                               // final since the count launch: loaded before the first atomic
+#pragma unroll
+    for (int c = 0; c < NB; c++) size[c] = bucket[c];
+    int first = 0;                                              // start of bucket c in the permutation
+#pragma unroll
+    for (int c = 0; c < NB; c++) {
+        const unsigned m = __ballot_sync(0xffffffffu, r == c);
+        if (m) {
+            const int leader = __ffs(m) - 1;
+            int base = 0;
+            if (lane == leader) base = atomicAdd(&bucket[NB + c], __popc(m));
+            base = __shfl_sync(0xffffffffu, base, leader);
+            if (r == c) perm[first + base + __popc(m & ((1u << lane) - 1))] = (int32_t)e;
+        }
+        first += size[c];
+    }
+}
+
 inline int env_grid(const BatchCore *h) { return (int)((h->n + 255) / 256); }
+
+// Opts Kernel in to `bytes` of dynamic shared memory (beyond the 48 KB default) once per device; every launch of Kernel asks
+// for the same amount.  One flag array per kernel.
+template <auto Kernel>
+cudaError_t allow_dynamic_smem(int device, size_t bytes)
+{
+    static bool done[64] = {};
+    if (done[device & 63]) return cudaSuccess;
+    const cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    if (e == cudaSuccess) done[device & 63] = true;
+    return e;
+}
 
 // Launches queued on the caller's streams are ordered before a later host-buffer step (which runs on the handle's own
 // stream) through this event.
@@ -270,6 +323,31 @@ inline int host_map(BatchCore *h, const void *user, size_t bytes, int slot, void
     *stage = h->h_stage[slot];
     CU_TRY(h, cudaHostGetDevicePointer(dev, *stage, 0));
     return BSKENV_OK;
+}
+
+// The start of a host-buffer step on the handle's own stream: maps the k caller buffers through host_map (slot s = user[s],
+// null when not passed; dev[s] = the address the kernels use, stage[s] = its staging block or null), copies the actions
+// (slot 0) into their stage, and orders the stream after whatever the caller queued on its own streams through the
+// device-buffer entry points.
+inline int host_step_begin(BatchCore *h, int k, void *const *user, const size_t *bytes, void **dev, void **stage)
+{
+    if (!h->own_stream) CU_TRY(h, cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
+    for (int s = 0; s < k; s++) {
+        dev[s] = stage[s] = nullptr;
+        if (!user[s]) continue;
+        const int rc = host_map(h, user[s], bytes[s], s, &dev[s], &stage[s]);
+        if (rc) return rc;
+    }
+    if (stage[0]) memcpy(stage[0], user[0], bytes[0]);
+    if (h->ev_valid) CU_TRY(h, cudaStreamWaitEvent(h->own_stream, h->ev_last, 0));
+    return BSKENV_OK;
+}
+// ... and its end, once the stream has completed: the staged results (slots 1 .. k-1 with both a caller buffer and a stage)
+// copied to the caller
+inline void host_step_copy_back(int k, void *const *user, void *const *stage, const size_t *bytes)
+{
+    for (int s = 1; s < k; s++)
+        if (user[s] && stage[s]) memcpy(user[s], stage[s], bytes[s]);
 }
 
 // bskenv_state_field / bskenv_opnav_state_field: the index of a named field in the batch's table (-1: none), is_int = which block

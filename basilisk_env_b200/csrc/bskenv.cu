@@ -6,12 +6,14 @@
 //                     basilisk_env/simulators/leoPowerAttitudeSimulator.py:590-595, and the gym
 //                     bookkeeping of basilisk_env/envs/leoPowerAttitudeEnvironment.py:65-145);
 //                     warp-shuffle reduction of the episode statistics; optional in-kernel auto-reset.
+//   leo_step_penv_kernel  the same body (leo_step_body) with per-env spacecraft parameters from a parameter pool.
+//   leo_split_kernel  small batches: the same interval with the work of one env split over two warps (leo_split.cuh).
 //   leo_reset_kernel  simulator construction + initial observation (reference ...Simulator.py:67-117,
 //                     ...Environment.py:172-216) from explicit, stored or device-sampled ICs.
 //   fp64_peak_kernel  DFMA microbenchmark = the roofline denominator.
-// There is no CPU path in this library.
+// The lane bucketing before a step (bucket_count_kernel + bucket_fill_kernel) is shared with the opNav batch
+// (batch_common.cuh).  There is no CPU path in this library.
 #include <cuda_runtime.h>
-#include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
 #include <string>
@@ -24,9 +26,6 @@
 #include "leo_host.h"
 #include "batch_common.cuh"
 
-#ifndef LEO_LANES
-#define LEO_LANES 32            // envs per warp (tuning builds: 16 / 8 leave the upper lanes idle)
-#endif
 #ifndef LEO_MIN_BLOCKS
 #define LEO_MIN_BLOCKS 3        // resident blocks per SM: 3 x 128 threads x 168 registers
 #endif
@@ -72,44 +71,17 @@ struct LeoSched { int *sched; int n_groups; int dynamic; int n_chunks; int *prog
 
 // Lane assignment of the throughput organisation.  The three modes run different flight software (hillPoint vs inertial3D;
 // the desat chain, the thruster latch and the exact thruster steps only after action 2): a warp of mixed actions executes
-// all of it, 180 times per interval.  Before the launch the envs are bucketed by action (counting sort, warp-aggregated
-// atomics: leo_bucket_count_kernel + leo_bucket_fill_kernel) and a warp takes 32 slots of the permutation: the state is
-// gathered / scattered at the chunk boundaries (12 times per 1800 ticks), the tick loop diverges only in the at most three
-// warps that straddle a bucket boundary.  Per-env arithmetic does not depend on the lane an env runs in: results are
-// bit-identical with and without (tests/test_gpu_round2.py).  bucket[0..3] = sizes, bucket[4..7] = cursors.  Order of the
-// buckets in the permutation: action 2 (the desat chain: the slowest warps), 0, 1, unknown -- the work queue hands out the
-// long items first, so that the tail of a launch is made of the short ones.
-__device__ __forceinline__ int leo_action_class(int action) { return (action >= 0 && action <= 2) ? action : 3; }
-__global__ void __launch_bounds__(256)
-leo_bucket_count_kernel(int64_t n, const int32_t *__restrict__ actions, int *__restrict__ bucket)
-{
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int cls = e < n ? leo_action_class(actions[e]) : -1;
-#pragma unroll
-    for (int c = 0; c < 4; c++) {
-        const unsigned m = __ballot_sync(0xffffffffu, cls == c);
-        if ((threadIdx.x & 31) == 0 && m) atomicAdd(&bucket[c], __popc(m));
-    }
-}
-__global__ void __launch_bounds__(256)
-leo_bucket_fill_kernel(int64_t n, const int32_t *__restrict__ actions, int *__restrict__ bucket, int32_t *__restrict__ perm)
-{
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int cls = e < n ? leo_action_class(actions[e]) : -1;
-    const int lane = threadIdx.x & 31;
-    const int n0 = bucket[0], n1 = bucket[1], n2 = bucket[2];
-#pragma unroll
-    for (int c = 0; c < 4; c++) {
-        const unsigned m = __ballot_sync(0xffffffffu, cls == c);
-        if (!m) continue;
-        const int leader = __ffs(m) - 1;
-        int base = 0;
-        if (lane == leader) base = atomicAdd(&bucket[4 + c], __popc(m));
-        base = __shfl_sync(0xffffffffu, base, leader);
-        const int first = c == 2 ? 0 : (c == 0 ? n2 : (c == 1 ? n2 + n0 : n0 + n1 + n2));     // slowest bucket first in the queue
-        if (cls == c) perm[first + base + __popc(m & ((1u << lane) - 1))] = (int32_t)e;
-    }
-}
+// all of it, 180 times per interval.  Before the launch the envs are bucketed by action (batch_common.cuh:
+// bucket_count_kernel + bucket_fill_kernel) and a warp takes 32 slots of the permutation: the state is gathered / scattered
+// at the chunk boundaries (12 times per 1800 ticks), the tick loop diverges only in the at most three warps that straddle a
+// bucket boundary.  Per-env arithmetic does not depend on the lane an env runs in: results are bit-identical with and
+// without (tests/test_gpu_round2.py).  bucket[0..3] = sizes, bucket[4..7] = cursors, in bucket order: action 2 (the desat
+// chain: the slowest warps), 0, 1, unknown -- the work queue hands out the long items first, so that the tail of a launch
+// is made of the short ones.
+struct LeoActionRank {
+    const int32_t *actions;
+    __device__ int operator()(int64_t e) const { const int a = actions[e]; return a == 2 ? 0 : (a == 0 ? 1 : (a == 1 ? 2 : 3)); }
+};
 
 __device__ __forceinline__ void chunk_publish(int *p, int v)
 {
@@ -184,24 +156,24 @@ __device__ __forceinline__ void step_finish(const LeoParams &P, double *__restri
     }
 }
 
-// MINB = resident blocks per SM the register allocation is made for.  LEO_MIN_BLOCKS (3 blocks x 128 threads x 168 registers,
-// a few spilled values) is the throughput organisation.  MINB = 1 is the SMALL-BATCH organisation (BASELINE configs[1], 4096
-// envs): when the whole batch fits one block per SM anyway, every warp runs alone on its SM sub-partition at its dependent-
-// issue latency, occupancy buys nothing and the full register file (255 registers, nothing spilled onto the dependency
-// chain) is worth 20 % (DESIGN.md section 5b).
-template <int NRW, int J2, bool DIAG, bool F32, int MINB>
-__global__ void LEO_STEP_BOUNDS(MINB)
-leo_step_kernel(const __grid_constant__ LeoParams P, const __grid_constant__ LeoParamsF PF, double *__restrict__ S, int64_t *__restrict__ I, double *__restrict__ ics,
-                int64_t stride, int64_t n, const int32_t *__restrict__ actions, double *__restrict__ obs,
-                double *__restrict__ reward, uint8_t *__restrict__ done, uint8_t *__restrict__ reason,
-                double *__restrict__ term_obs, double *__restrict__ stats, const LeoSched sc,
-                double *__restrict__ ep_return, int64_t *__restrict__ ep_length)
+// One decision interval of the one-thread-per-env organisation, the body of both step kernels: work items from the queue
+// or the warp's own group (LeoSched), slot -> env through the lane permutation, leo_step_env chunk by chunk with the
+// chunk hand-over between work items, step_finish after the last chunk.  PA = the parameter accessor of leo_step_env
+// (leo::ParBatch: the batch configuration; leo::ParEnv: per-env parameters, whose auto-reset assigns a row of `pool`).
+// tid = threadIdx.x, read by the kernel: there the compiler knows its range from the launch bounds.
+template <int NRW, int J2, bool DIAG, bool F32, class PA>
+__device__ __forceinline__ void leo_step_body(unsigned tid, const LeoParams &P, const LeoParamsF &PF, const LeoPool &pool, double *__restrict__ S,
+                                              int64_t *__restrict__ I, double *__restrict__ ics, int64_t stride, int64_t n,
+                                              const int32_t *__restrict__ actions, double *__restrict__ obs, double *__restrict__ reward,
+                                              uint8_t *__restrict__ done, uint8_t *__restrict__ reason, double *__restrict__ term_obs,
+                                              double *__restrict__ stats, const LeoSched &sc, double *__restrict__ ep_return,
+                                              int64_t *__restrict__ ep_length)
 {
-    extern __shared__ double bus_smem[];          // [LEO_NM][LEO_BLOCK]: per-thread message bus (leo_core.cuh: MBus)
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    extern __shared__ double bus_smem[];          // [LEO_NM (ParEnv: LEO_NM_PENV)][LEO_BLOCK]: per-thread message bus (leo_core.cuh: MBus)
+    const int lane = tid & 31, warp = tid >> 5;
     leo::MBus bus;
     bus.p = nullptr;
-    bus.a = (uint32_t)__cvta_generic_to_shared(bus_smem) + threadIdx.x * (uint32_t)sizeof(double);
+    bus.a = (uint32_t)__cvta_generic_to_shared(bus_smem) + tid * (uint32_t)sizeof(double);
     for (bool more = true; more; more = sc.dynamic != 0) {
         int g, c_first = 0, c_end = sc.n_chunks;
         if (sc.dynamic) {
@@ -219,25 +191,42 @@ leo_step_kernel(const __grid_constant__ LeoParams P, const __grid_constant__ Leo
         } else {
             g = blockIdx.x * (LEO_BLOCK / 32) + warp;
         }
-        const int64_t slot = (int64_t)g * LEO_LANES + lane;
-        const bool valid = lane < LEO_LANES && slot < n;
+        const int64_t slot = (int64_t)g * 32 + lane;
+        const bool valid = slot < n;
         const int64_t e = (valid && sc.perm) ? (int64_t)sc.perm[slot] : slot;     // envs of one action per warp (see LeoSched)
         leo::StepOut o;
         o.done = 0; o.reason = 0; o.reward = 0.;
         for (int c = c_first; c < c_end; c++) {
-        if (valid) leo::leo_step_env<NRW, J2, DIAG, F32>(P, S, I, stride, e, bus, actions[e], o, PF, c, sc.n_chunks);
-        if (c + 1 < sc.n_chunks) {                              // chunk boundary inside the interval: publish and go on
-            if (sc.dynamic) {
-                __threadfence();
-                __syncwarp();
-                if (lane == 0) chunk_publish(sc.progress + g, c + 1);
+            if (valid) leo::leo_step_env<NRW, J2, DIAG, F32, PA>(P, S, I, stride, e, bus, actions[e], o, PF, c, sc.n_chunks);
+            if (c + 1 < sc.n_chunks) {                          // chunk boundary inside the interval: publish and go on
+                if (sc.dynamic) {
+                    __threadfence();
+                    __syncwarp();
+                    if (lane == 0) chunk_publish(sc.progress + g, c + 1);
+                }
+                continue;
             }
-            continue;
-        }
-        step_finish(P, S, I, ics, stride, e, valid, lane, o, obs, reward, done, reason, term_obs, stats, ep_return, ep_length);
+            step_finish<PA>(P, S, I, ics, stride, e, valid, lane, o, obs, reward, done, reason, term_obs, stats, ep_return, ep_length, pool);
         }   // chunks of this item
         __syncwarp();
     }
+}
+
+// MINB = resident blocks per SM the register allocation is made for.  LEO_MIN_BLOCKS (3 blocks x 128 threads x 168 registers,
+// a few spilled values) is the throughput organisation.  MINB = 1 is the SMALL-BATCH organisation (BASELINE configs[1], 4096
+// envs): when the whole batch fits one block per SM anyway, every warp runs alone on its SM sub-partition at its dependent-
+// issue latency, occupancy buys nothing and the full register file (255 registers, nothing spilled onto the dependency
+// chain) is worth 20 % (DESIGN.md section 5b).
+template <int NRW, int J2, bool DIAG, bool F32, int MINB>
+__global__ void LEO_STEP_BOUNDS(MINB)
+leo_step_kernel(const __grid_constant__ LeoParams P, const __grid_constant__ LeoParamsF PF, double *__restrict__ S, int64_t *__restrict__ I, double *__restrict__ ics,
+                int64_t stride, int64_t n, const int32_t *__restrict__ actions, double *__restrict__ obs,
+                double *__restrict__ reward, uint8_t *__restrict__ done, uint8_t *__restrict__ reason,
+                double *__restrict__ term_obs, double *__restrict__ stats, const LeoSched sc,
+                double *__restrict__ ep_return, int64_t *__restrict__ ep_length)
+{
+    leo_step_body<NRW, J2, DIAG, F32, leo::ParBatch>(threadIdx.x, P, PF, LeoPool{}, S, I, ics, stride, n, actions, obs, reward, done, reason, term_obs,
+                                                     stats, sc, ep_return, ep_length);
 }
 
 // The same organisation with per-env spacecraft parameters (bskenv_set_param_pool): leo_step_env<..., ParEnv> reads each
@@ -254,48 +243,8 @@ leo_step_penv_kernel(const __grid_constant__ LeoParams P, const LeoPool pool, do
                      int64_t *__restrict__ ep_length)
 {
     static_assert(NRW == 3 && DIAG && J2 != 2, "per-env parameters are built for the reference configuration");
-    extern __shared__ double bus_smem[];          // [LEO_NM_PENV][LEO_BLOCK]
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    leo::MBus bus;
-    bus.p = nullptr;
-    bus.a = (uint32_t)__cvta_generic_to_shared(bus_smem) + threadIdx.x * (uint32_t)sizeof(double);
-    for (bool more = true; more; more = sc.dynamic != 0) {
-        int g, c_first = 0, c_end = sc.n_chunks;
-        if (sc.dynamic) {
-            g = 0;
-            if (lane == 0) g = atomicAdd(&sc.sched[0], 1);
-            g = __shfl_sync(0xffffffffu, g, 0);
-            if (g >= sc.n_groups * sc.n_chunks) break;
-            c_first = g / sc.n_groups; c_end = c_first + 1;
-            g -= c_first * sc.n_groups;
-            if (c_first > 0) {
-                if (lane == 0)
-                    while (chunk_peek(sc.progress + g) < c_first) __nanosleep(200);
-                __syncwarp();
-            }
-        } else {
-            g = blockIdx.x * (LEO_BLOCK / 32) + warp;
-        }
-        const int64_t slot = (int64_t)g * LEO_LANES + lane;
-        const bool valid = lane < LEO_LANES && slot < n;
-        const int64_t e = (valid && sc.perm) ? (int64_t)sc.perm[slot] : slot;
-        leo::StepOut o;
-        o.done = 0; o.reason = 0; o.reward = 0.;
-        for (int c = c_first; c < c_end; c++) {
-            if (valid) leo::leo_step_env<NRW, J2, DIAG, false, leo::ParEnv>(P, S, I, stride, e, bus, actions[e], o, LeoParamsF(), c, sc.n_chunks);
-            if (c + 1 < sc.n_chunks) {
-                if (sc.dynamic) {
-                    __threadfence();
-                    __syncwarp();
-                    if (lane == 0) chunk_publish(sc.progress + g, c + 1);
-                }
-                continue;
-            }
-            step_finish<leo::ParEnv>(P, S, I, ics, stride, e, valid, lane, o, obs, reward, done, reason, term_obs, stats, ep_return,
-                                     ep_length, pool);
-        }
-        __syncwarp();
-    }
+    leo_step_body<NRW, J2, DIAG, false, leo::ParEnv>(threadIdx.x, P, LeoParamsF(), pool, S, I, ics, stride, n, actions, obs, reward, done, reason,
+                                                     term_obs, stats, sc, ep_return, ep_length);
 }
 
 // Ragged batches in the split organisation: the lanes of the last group that have no env step a DUPLICATE of the last env
@@ -345,16 +294,8 @@ leo_split_kernel(const __grid_constant__ LeoParams P, double *__restrict__ S, in
     }
     leo::StepOut o;
     o.done = 0; o.reason = 0; o.reward = 0.;
-#ifdef LEO_SPLIT_PROF
-    long long tc[8]; tc[0] = clock64();
-    for (int c = 0; c < n_chunks; c++) { leo::split_dyn<NRW, J2, DIAG>(P, S, I, stride, e, bus, box, bar, action, o, c, n_chunks); tc[c + 1] = clock64(); }
-    step_finish(P, S, I, ics, stride, e, valid, lane, o, obs, reward, done, reason, term_obs, stats, ep_return, ep_length);
-    if (lane == 0) printf("BLK %d total %lld chunks %lld %lld %lld %lld %lld %lld finish %lld\n", blockIdx.x, clock64() - tc[0], tc[1] - tc[0], tc[2] - tc[1], tc[3] - tc[2],
-                          tc[4] - tc[3], tc[5] - tc[4], tc[6] - tc[5], clock64() - tc[6]);
-#else
     for (int c = 0; c < n_chunks; c++) leo::split_dyn<NRW, J2, DIAG>(P, S, I, stride, e, bus, box, bar, action, o, c, n_chunks);
     step_finish(P, S, I, ics, stride, e, valid, lane, o, obs, reward, done, reason, term_obs, stats, ep_return, ep_length);
-#endif
 }
 
 // mode 0: explicit ICs (row-major [n][19]); 1: stored ICs (reset_init); 2: device-sampled ICs, or a row of the IC pool.
@@ -459,7 +400,7 @@ static int launch_step(bskenv_handle *h, const int32_t *act, double *obs, double
     if (follow) { P_nr = h->P; P_nr.auto_reset = 0; }
     const LeoParams &PK = follow ? P_nr : h->P;
     const int wpb = LEO_BLOCK / 32;
-    const int64_t groups = (h->n + LEO_LANES - 1) / LEO_LANES;
+    const int64_t groups = (h->n + 31) / 32;
     const int resident = h->sm_count * LEO_MIN_BLOCKS;          // blocks of one full resident set
     int grid = (int)((groups + wpb - 1) / wpb);
 #ifndef LEO_SMALL_BLOCKS
@@ -488,18 +429,13 @@ static int launch_step(bskenv_handle *h, const int32_t *act, double *obs, double
         const int dgrid = (int)((groups + G - 1) / G);
         if (h->n % 32) leo_pad_kernel<<<1, 256, 0, st>>>(h->S, h->I, h->stride, h->n);
         const size_t smem = LEO_BUS_BYTES + LEO_SPLIT_BOX_BYTES;
-        static bool split_attr[64][2] = {{false}};
-        const int which = h->P.nrw == 3 ? 0 : 1;
-        if (!split_attr[h->device & 63][which]) {
-            if (which == 0) CU_TRY(h, cudaFuncSetAttribute(leo_split_kernel<3, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            else CU_TRY(h, cudaFuncSetAttribute(leo_split_kernel<4, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            split_attr[h->device & 63][which] = true;
-        }
-        if (which == 0) {
+        if (h->P.nrw == 3) {
+            CU_TRY(h, allow_dynamic_smem<leo_split_kernel<3, 0, true>>(h->device, smem));
             h->kernel_name = "leo_split_kernel<3,0,true>";
             leo_split_kernel<3, 0, true><<<dgrid, 64 * G, smem, st>>>(PK, h->S, h->I, h->ics, h->stride, h->n, act, obs, rew, done, reason, term_obs,
                                                                  h->stats, (int)groups, sc.n_chunks, ep_return, ep_length);
         } else {
+            CU_TRY(h, allow_dynamic_smem<leo_split_kernel<4, 1, false>>(h->device, smem));
             h->kernel_name = "leo_split_kernel<4,1,false>";
             leo_split_kernel<4, 1, false><<<dgrid, 64 * G, smem, st>>>(PK, h->S, h->I, h->ics, h->stride, h->n, act, obs, rew, done, reason, term_obs,
                                                                   h->stats, (int)groups, sc.n_chunks, ep_return, ep_length);
@@ -512,38 +448,31 @@ static int launch_step(bskenv_handle *h, const int32_t *act, double *obs, double
     }
     if (!small && h->organisation != BSKENV_ORG_THREAD_INDEX) {      // bucket the envs by action (LeoSched)
         const int bgrid = (int)((h->n + 255) / 256);
+        const LeoActionRank rank{act};
         CU_TRY(h, cudaMemsetAsync(h->bucket, 0, sizeof(int) * 8, st));
-        leo_bucket_count_kernel<<<bgrid, 256, 0, st>>>(h->n, act, h->bucket);
-        leo_bucket_fill_kernel<<<bgrid, 256, 0, st>>>(h->n, act, h->bucket, h->perm);
+        bucket_count_kernel<4><<<bgrid, 256, 0, st>>>(h->n, rank, h->bucket);
+        bucket_fill_kernel<4><<<bgrid, 256, 0, st>>>(h->n, rank, h->bucket, h->perm);
         sc.perm = h->perm;
         h->launches += 2;
     }
 #define LEO_STR_(x) #x
 #define LEO_STR(x) LEO_STR_(x)
-#define LEO_LAUNCH_B(NRW, J2, DIAG, F32, MINB)                                                                 \
-    do {                                                                                                       \
-        static bool attr_set[64] = {false};      /* opt in to > 48 KB of dynamic shared memory once per device */  \
-        const size_t bus_bytes = (J2) == 2 ? LEO_BUS_BYTES_PFIX : LEO_BUS_BYTES;                                \
-        if (!attr_set[h->device & 63]) {                                                                       \
-            CU_TRY(h, cudaFuncSetAttribute(leo_step_kernel<NRW, J2, DIAG, F32, MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bus_bytes)); \
-            attr_set[h->device & 63] = true;                                                                   \
-        }                                                                                                      \
-        h->kernel_name = "leo_step_kernel<" #NRW "," #J2 "," #DIAG "," #F32 "," LEO_STR(MINB) ">";              \
-        leo_step_kernel<NRW, J2, DIAG, F32, MINB><<<grid, LEO_BLOCK, bus_bytes, st>>>(PK, h->PF, h->S, h->I, h->ics, h->stride, h->n, act, obs, \
-                                                                                 rew, done, reason, term_obs, h->stats, sc, ep_return, ep_length); \
+    // KERNEL<<<...>>>(PK, ARG2, ...): ARG2 = the reduced-precision parameter block of leo_step_kernel or the parameter pool of
+    // leo_step_penv_kernel
+#define LEO_LAUNCH_K(NAME, SMEM, ARG2, ...)                                                                                 \
+    do {                                                                                                                   \
+        CU_TRY(h, allow_dynamic_smem<__VA_ARGS__>(h->device, SMEM));                                                       \
+        h->kernel_name = NAME;                                                                                             \
+        __VA_ARGS__<<<grid, LEO_BLOCK, SMEM, st>>>(PK, ARG2, h->S, h->I, h->ics, h->stride, h->n, act, obs, rew, done, reason, \
+                                                   term_obs, h->stats, sc, ep_return, ep_length);                         \
     } while (0)
+#define LEO_LAUNCH_B(NRW, J2, DIAG, F32, MINB)                                                                         \
+    LEO_LAUNCH_K("leo_step_kernel<" #NRW "," #J2 "," #DIAG "," #F32 "," LEO_STR(MINB) ">", (J2) == 2 ? LEO_BUS_BYTES_PFIX : LEO_BUS_BYTES, \
+                 h->PF, leo_step_kernel<NRW, J2, DIAG, F32, MINB>)
 #define LEO_LAUNCH(NRW, J2, DIAG, F32) LEO_LAUNCH_B(NRW, J2, DIAG, F32, LEO_MIN_BLOCKS)
-#define LEO_LAUNCH_PENV(J2)                                                                                    \
-    do {                                                                                                       \
-        static bool attr_set[64] = {false};                                                                    \
-        if (!attr_set[h->device & 63]) {                                                                       \
-            CU_TRY(h, cudaFuncSetAttribute(leo_step_penv_kernel<3, J2, true, LEO_MIN_BLOCKS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LEO_BUS_BYTES_PENV)); \
-            attr_set[h->device & 63] = true;                                                                   \
-        }                                                                                                      \
-        h->kernel_name = "leo_step_penv_kernel<3," #J2 ",true," LEO_STR(LEO_MIN_BLOCKS) ">";                    \
-        leo_step_penv_kernel<3, J2, true, LEO_MIN_BLOCKS><<<grid, LEO_BLOCK, LEO_BUS_BYTES_PENV, st>>>(PK, h->pool, h->S, h->I, h->ics, \
-            h->stride, h->n, act, obs, rew, done, reason, term_obs, h->stats, sc, ep_return, ep_length);        \
-    } while (0)
+#define LEO_LAUNCH_PENV(J2)                                                                                            \
+    LEO_LAUNCH_K("leo_step_penv_kernel<3," #J2 ",true," LEO_STR(LEO_MIN_BLOCKS) ">", LEO_BUS_BYTES_PENV, h->pool,          \
+                 leo_step_penv_kernel<3, J2, true, LEO_MIN_BLOCKS>)
     if (penv) { if (h->cfg.use_j2) LEO_LAUNCH_PENV(1); else LEO_LAUNCH_PENV(0); }    // (bskenv_set_param_pool checks the configuration)
     // small-batch organisation: built for the reference configuration and for the stress configuration
     else if (small &&!h->P.grav_pfix && !h->P.mixed && h->P.nrw == 3 && !h->cfg.use_j2 && h->P.diag) LEO_LAUNCH_B(3, 0, true, false, 1);
@@ -564,6 +493,7 @@ static int launch_step(bskenv_handle *h, const int32_t *act, double *obs, double
 #undef LEO_LAUNCH
 #undef LEO_LAUNCH_B
 #undef LEO_LAUNCH_PENV
+#undef LEO_LAUNCH_K
     CU_TRY(h, cudaGetLastError());
     h->launches++;
     if (follow) { const int rc = launch_follow_reset(h, done, obs, st); if (rc) return rc; }
@@ -606,7 +536,7 @@ int bskenv_create(const bskenv_config *cfg, int device, int64_t n_envs, int64_t 
     h->P.first_env_index = first_env_index;
     h->s_fields = LEO_ND;       // (the handle is zero-initialised: no pools, BSKENV_ORG_AUTO)
     cudaError_t e = core_alloc(h, device, n_envs, LEO_ND, LEO_NI, 19, ST_N);
-    if (e == cudaSuccess) e = cudaMalloc(&h->sched, sizeof(int) * (size_t)(4 + (n_envs + LEO_LANES - 1) / LEO_LANES));
+    if (e == cudaSuccess) e = cudaMalloc(&h->sched, sizeof(int) * (size_t)(4 + (n_envs + 31) / 32));
     if (e == cudaSuccess) e = cudaMalloc(&h->perm, sizeof(int32_t) * h->stride);
     if (e == cudaSuccess) e = cudaMalloc(&h->bucket, sizeof(int) * 8);
     if (e != cudaSuccess) {
@@ -796,21 +726,13 @@ int bskenv_step_host_async(bskenv_handle *h, const int32_t *actions, double *obs
     if (h->host_pending) { h->err = "bskenv_step_host_async: the previous host step has not been waited for"; return BSKENV_EINVAL; }
     CU_TRY(h, cudaSetDevice(h->device));
     const size_t n = (size_t)h->n;
-    if (!h->own_stream) CU_TRY(h, cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
-    cudaStream_t st = h->own_stream;
     void *user[8] = {(void *)actions, obs, reward, done, done_reason, ep_return, ep_length, term_obs};
     const size_t bytes[8] = {n * sizeof(int32_t), n * 5 * sizeof(double), n * sizeof(double), n, n, n * sizeof(double), n * sizeof(int64_t), n * 5 * sizeof(double)};
-    void *dev[8] = {}, *stage[8] = {};
-    for (int k = 0; k < 8; k++) {
-        if (!user[k]) continue;
-        const int rc = host_map(h, user[k], bytes[k], k, &dev[k], &stage[k]);
-        if (rc) return rc;
-    }
-    if (stage[0]) memcpy(stage[0], actions, bytes[0]);
-    // order after whatever the caller queued through bskenv_step / reset / set_state on its own streams
-    if (h->ev_valid) CU_TRY(h, cudaStreamWaitEvent(st, h->ev_last, 0));
-    const int rc = launch_step(h, (const int32_t *)dev[0], (double *)dev[1], (double *)dev[2], (uint8_t *)dev[3], (uint8_t *)dev[4],
-                               (double *)dev[7], st, (double *)dev[5], (int64_t *)dev[6]);
+    void *dev[8], *stage[8];
+    int rc = host_step_begin(h, 8, user, bytes, dev, stage);
+    if (rc) return rc;
+    rc = launch_step(h, (const int32_t *)dev[0], (double *)dev[1], (double *)dev[2], (uint8_t *)dev[3], (uint8_t *)dev[4],
+                     (double *)dev[7], h->own_stream, (double *)dev[5], (int64_t *)dev[6]);
     if (rc) return rc;
     for (int k = 0; k < 8; k++) { h->pend_user[k] = stage[k] ? user[k] : nullptr; h->pend_bytes[k] = bytes[k]; }
     h->host_pending = 1;
@@ -823,8 +745,7 @@ int bskenv_step_host_wait(bskenv_handle *h)
     if (!h->host_pending) return BSKENV_OK;
     h->host_pending = 0;
     CU_TRY(h, cudaStreamSynchronize(h->own_stream));
-    for (int k = 1; k < 8; k++)
-        if (h->pend_user[k]) memcpy(h->pend_user[k], h->h_stage[k], h->pend_bytes[k]);
+    host_step_copy_back(8, h->pend_user, h->h_stage, h->pend_bytes);
     return BSKENV_OK;
 }
 

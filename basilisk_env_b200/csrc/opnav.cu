@@ -7,8 +7,11 @@
 //                       and the gym bookkeeping of envs/opNavEnvironment.py:55-125): noise walk + dynamics / flight
 //                       software, then the filter + observation / reward; warp-shuffle reduction of the episode
 //                       statistics; optional in-kernel auto-reset.
+//   opnav_noise_kernel, opnav_dyn_kernel
+//                       the opt-in three-kernel form of the first pass: the noise walk of the interval, then the rest.
 //   opnav_reset_kernel  simulator construction + initial observation from explicit, stored or device-sampled ICs.
-// There is no CPU path in this library.
+// The lane bucketing before a step (bucket_count_kernel + bucket_fill_kernel) is shared with the LEO batch
+// (batch_common.cuh).  There is no CPU path in this library.
 #include <cuda_runtime.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -45,8 +48,8 @@ struct OnSched { int *sched; int n_groups; int dynamic; };
 // eclipse + cssWlsEst + sunSafePoint); with one env per lane in index order a warp of mixed actions runs both, 3000 times.
 // Before the step, envs are therefore bucketed by the task set they WILL run (first-interval event, action, or the mode in
 // force for an unknown action) and the warps of the step kernel take 32 envs of one bucket: the persistent state is read and
-// written once per decision (gathered, 97 fields per env), the tick loop is divergence-free.  sched[1..2] = bucket sizes,
-// sched[3..4] = bucket cursors.
+// written once per decision (gathered, 97 fields per env), the tick loop is divergence-free (batch_common.cuh:
+// bucket_count_kernel + bucket_fill_kernel, task set 0 first).  sched[1..2] = bucket sizes, sched[3..4] = bucket cursors.
 __device__ __forceinline__ int opnav_task_set(const int64_t *__restrict__ I, int64_t stride, int64_t e, int action)
 {
     if (I[(int64_t)OI_FIRST * stride + e]) return 0;
@@ -54,33 +57,10 @@ __device__ __forceinline__ int opnav_task_set(const int64_t *__restrict__ I, int
     // bskenv_opnav_set_state) is the sun-safe set, so that every env lands in exactly one of the two buckets
     return action == 0 ? 0 : (action == 1 ? 1 : (I[(int64_t)OI_MODE * stride + e] != 0 ? 1 : 0));
 }
-__global__ void __launch_bounds__(256)
-opnav_bucket_count_kernel(const int64_t *__restrict__ I, int64_t stride, int64_t n, const int32_t *__restrict__ actions, int *__restrict__ sched)
-{
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const bool valid = e < n;
-    const int cls = valid ? opnav_task_set(I, stride, e, actions[e]) : -1;
-    const unsigned m0 = __ballot_sync(0xffffffffu, cls == 0);
-    if ((threadIdx.x & 31) == 0 && m0) atomicAdd(&sched[1], __popc(m0));
-}
-__global__ void __launch_bounds__(256)
-opnav_bucket_fill_kernel(const int64_t *__restrict__ I, int64_t stride, int64_t n, const int32_t *__restrict__ actions, int *__restrict__ sched,
-                         int32_t *__restrict__ perm)
-{
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const bool valid = e < n;
-    const int cls = valid ? opnav_task_set(I, stride, e, actions[e]) : -1;
-    const int lane = threadIdx.x & 31;
-#pragma unroll
-    for (int c = 0; c < 2; c++) {
-        const unsigned m = __ballot_sync(0xffffffffu, cls == c);
-        if (!m) continue;
-        int base = 0;
-        if (lane == __ffs(m) - 1) base = atomicAdd(&sched[3 + c], __popc(m));
-        base = __shfl_sync(0xffffffffu, base, __ffs(m) - 1);
-        if (cls == c) perm[(c == 0 ? 0 : sched[1]) + base + __popc(m & ((1u << lane) - 1))] = (int32_t)e;
-    }
-}
+struct OnTaskSetRank {
+    const int64_t *I; int64_t stride; const int32_t *actions;
+    __device__ int operator()(int64_t e) const { return opnav_task_set(I, stride, e, actions[e]); }
+};
 
 __global__ void opnav_perm_identity_kernel(int32_t *__restrict__ perm, int64_t stride, int64_t n)
 {
@@ -315,33 +295,25 @@ static int opnav_launch_step(bskenv_opnav_handle *h, const int32_t *act, double 
     const int64_t set2 = (int64_t)h->sm_count * 2 * ON_BLOCK, set3 = (int64_t)h->sm_count * 3 * ON_BLOCK;
     const int64_t n2 = (h->n + set2 - 1) / set2, n3 = (h->n + set3 - 1) / set3;
     const int minb1 = (ON_MIN_BLOCKS == 3 && n3 * 379 < n2 * 302) ? 3 : 2, minb2 = ON_MIN_BLOCKS == 3 ? 3 : 2;
-#ifdef ON_DYN_FORCE_MINB
-    const int minb1_dyn = ON_DYN_FORCE_MINB;
-#else
-    const int minb1_dyn = minb1;
-#endif
     const int full = (int)((groups + wpb - 1) / wpb);
     OnSched sc;
     sc.sched = h->sched; sc.n_groups = (int)groups; sc.dynamic = 0;
     CU_TRY(h, cudaMemsetAsync(h->sched, 0, sizeof(int) * 8, st));
-    {   // bucket the envs by flight-software task set (two small launches; see opnav_bucket_*_kernel)
+    {   // bucket the envs by flight-software task set (two small launches; see opnav_task_set)
         const int bgrid = (int)((h->n + 255) / 256);
-        opnav_bucket_count_kernel<<<bgrid, 256, 0, st>>>(h->I, h->stride, h->n, act, h->sched);
-        opnav_bucket_fill_kernel<<<bgrid, 256, 0, st>>>(h->I, h->stride, h->n, act, h->sched, h->perm);
+        const OnTaskSetRank rank{h->I, h->stride, act};
+        bucket_count_kernel<2><<<bgrid, 256, 0, st>>>(h->n, rank, h->sched + 1);
+        bucket_fill_kernel<2><<<bgrid, 256, 0, st>>>(h->n, rank, h->sched + 1, h->perm);
     }
     OnSched s1 = sc, s2 = sc;
     const int r1 = h->sm_count * minb1, r2 = h->sm_count * minb2;
     s1.dynamic = full > r1; s2.dynamic = full > r2;
     const int grid1 = full > r1 ? r1 : full, grid2 = full > r2 ? r2 : full;
     const size_t smem_a = sizeof(OnScratchA) * ON_BLOCK, smem_b = sizeof(OnScratchB) * ON_BLOCK;
-    static bool attr_set[64] = {false};             // opt in to the dynamic shared memory once per device
-    if (!attr_set[h->device & 63]) {
-        CU_TRY(h, cudaFuncSetAttribute(opnav_pass1_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_a));
-        CU_TRY(h, cudaFuncSetAttribute(opnav_pass1_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_a));
-        CU_TRY(h, cudaFuncSetAttribute(opnav_pass2_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
-        CU_TRY(h, cudaFuncSetAttribute(opnav_pass2_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
-        attr_set[h->device & 63] = true;
-    }
+    CU_TRY(h, allow_dynamic_smem<opnav_pass1_kernel<2>>(h->device, smem_a));
+    CU_TRY(h, allow_dynamic_smem<opnav_pass1_kernel<3>>(h->device, smem_a));
+    CU_TRY(h, allow_dynamic_smem<opnav_pass2_kernel<2>>(h->device, smem_b));
+    CU_TRY(h, allow_dynamic_smem<opnav_pass2_kernel<3>>(h->device, smem_b));
     if (h->noise_split < 0) {
         // Three-kernel form: OPT-IN (BSKENV_OPNAV_NOISE_SPLIT=1), and only when the noise buffer fits -- 120 B per env-tick, at most
         // ON_NZBUF_MAX_FRAC of the free device memory (113664 envs x 3001 ticks = 40.9 GB).  Measured on a B200: 118.6 against
@@ -359,17 +331,13 @@ static int opnav_launch_step(bskenv_opnav_handle *h, const int32_t *act, double 
     }
     if (h->noise_split == 1) {
         const size_t smem_n = sizeof(OnScratchN) * ON_BLOCK, smem_d = sizeof(OnScratchD) * ON_BLOCK;
-        static bool attr_d[64] = {false};
-        if (!attr_d[h->device & 63]) {
-            CU_TRY(h, cudaFuncSetAttribute(opnav_dyn_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_d));
-            CU_TRY(h, cudaFuncSetAttribute(opnav_dyn_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_d));
-            attr_d[h->device & 63] = true;
-        }
+        CU_TRY(h, allow_dynamic_smem<opnav_dyn_kernel<2>>(h->device, smem_d));
+        CU_TRY(h, allow_dynamic_smem<opnav_dyn_kernel<3>>(h->device, smem_d));
         opnav_noise_kernel<<<(int)((h->n + ON_BLOCK - 1) / ON_BLOCK), ON_BLOCK, smem_n, st>>>(h->P, h->S, h->I, h->stride, h->n, h->perm, h->nzbuf);
         OnSched sd = sc;
-        const int rd = h->sm_count * minb1_dyn, gridd = full > rd ? rd : full;
+        const int rd = h->sm_count * minb1, gridd = full > rd ? rd : full;
         sd.dynamic = full > rd;
-        if (minb1_dyn == 3) opnav_dyn_kernel<3><<<gridd, ON_BLOCK, smem_d, st>>>(h->P, h->S, h->I, h->stride, h->n, act, sd, h->perm, h->mbuf, h->nzbuf);
+        if (minb1 == 3) opnav_dyn_kernel<3><<<gridd, ON_BLOCK, smem_d, st>>>(h->P, h->S, h->I, h->stride, h->n, act, sd, h->perm, h->mbuf, h->nzbuf);
         else opnav_dyn_kernel<2><<<gridd, ON_BLOCK, smem_d, st>>>(h->P, h->S, h->I, h->stride, h->n, act, sd, h->perm, h->mbuf, h->nzbuf);
         h->launches += 1;
     }
@@ -519,24 +487,16 @@ int bskenv_opnav_step_host(bskenv_opnav_handle *h, const int32_t *actions, doubl
     if (!actions || !obs || !reward || !done || !done_reason) { h->err = "bskenv_opnav_step_host: null buffer"; return BSKENV_EINVAL; }
     CU_TRY(h, cudaSetDevice(h->device));
     const size_t n = (size_t)h->n;
-    if (!h->own_stream) CU_TRY(h, cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
-    cudaStream_t st = h->own_stream;
     void *user[6] = {(void *)actions, obs, reward, done, done_reason, debug};
     const size_t bytes[6] = {n * sizeof(int32_t), n * 4 * sizeof(double), n * sizeof(double), n, n, n * 12 * sizeof(double)};
-    void *dev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr}, *stage[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    for (int k = 0; k < 6; k++) {
-        if (!user[k]) continue;
-        int rc = host_map(h, user[k], bytes[k], k, &dev[k], &stage[k]);
-        if (rc) return rc;
-    }
-    if (stage[0]) memcpy(stage[0], actions, bytes[0]);
-    if (h->ev_valid) CU_TRY(h, cudaStreamWaitEvent(st, h->ev_last, 0));     // after the caller's device-buffer steps / resets
-    int rc = opnav_launch_step(h, (const int32_t *)dev[0], (double *)dev[1], (double *)dev[2], (uint8_t *)dev[3], (uint8_t *)dev[4],
-                               (double *)dev[5], nullptr, st);
+    void *dev[6], *stage[6];
+    int rc = host_step_begin(h, 6, user, bytes, dev, stage);
     if (rc) return rc;
-    CU_TRY(h, cudaStreamSynchronize(st));
-    for (int k = 1; k < 6; k++)
-        if (stage[k]) memcpy(user[k], stage[k], bytes[k]);
+    rc = opnav_launch_step(h, (const int32_t *)dev[0], (double *)dev[1], (double *)dev[2], (uint8_t *)dev[3], (uint8_t *)dev[4],
+                           (double *)dev[5], nullptr, h->own_stream);
+    if (rc) return rc;
+    CU_TRY(h, cudaStreamSynchronize(h->own_stream));
+    host_step_copy_back(6, user, stage, bytes);
     return BSKENV_OK;
 }
 

@@ -36,7 +36,7 @@ env = LeoPowerAttVecEnv(60000, device=0, auto_reset=True, step_duration=6.0, max
 env.reset()
 for t in range(3):
     env.step(torch.full((60000,), t % 3, dtype=torch.int32, device="cuda"))
-# ... and with mixed actions: the envs are bucketed by action (leo_bucket_*_kernel), the step kernel gathers through the permutation
+# ... and with mixed actions: the envs are bucketed by action (bucket_count_kernel + bucket_fill_kernel), the step kernel gathers through the permutation
 gq = torch.Generator(device="cuda"); gq.manual_seed(1)
 for t in range(2):
     env.step(torch.randint(0, 4, (60000,), dtype=torch.int32, device="cuda", generator=gq))
