@@ -47,7 +47,8 @@ OPNAV_EXPORTS = ["bskenv_opnav_default_config", "bskenv_opnav_create", "bskenv_o
                  "bskenv_opnav_get_ics", "bskenv_opnav_step", "bskenv_opnav_step_host", "bskenv_opnav_state_dims",
                  "bskenv_opnav_get_state", "bskenv_opnav_set_state", "bskenv_opnav_state_field",
                  "bskenv_opnav_episode_stats", "bskenv_opnav_launch_count", "bskenv_opnav_flops_per_step",
-                 "bskenv_opnav_set_ephemeris", "bskenv_opnav_step_info", "bskenv_opnav_set_ic_pool", "bskenv_opnav_get_ic_rows"]
+                 "bskenv_opnav_set_ephemeris", "bskenv_opnav_step_info", "bskenv_opnav_set_ic_pool", "bskenv_opnav_get_ic_rows",
+                 "bskenv_opnav_snapshot_width", "bskenv_opnav_snapshot", "bskenv_opnav_restore"]
 
 EXPORTS = ["bskenv_abi_version", "bskenv_default_config", "bskenv_create", "bskenv_destroy", "bskenv_last_error",
            "bskenv_num_envs", "bskenv_reset_seeded", "bskenv_reset_ics", "bskenv_reset_init", "bskenv_get_ics",
@@ -56,7 +57,7 @@ EXPORTS = ["bskenv_abi_version", "bskenv_default_config", "bskenv_create", "bske
            "bskenv_flops_per_step", "bskenv_set_ephemeris", "bskenv_set_gravity_degree2", "bskenv_step_info",
            "bskenv_step_host_async", "bskenv_step_host_wait", "bskenv_alloc_host", "bskenv_free_host", "bskenv_kernel_name",
            "bskenv_set_organisation", "bskenv_set_param_pool", "bskenv_get_env_params", "bskenv_set_ic_pool",
-           "bskenv_get_ic_rows"]
+           "bskenv_get_ic_rows", "bskenv_snapshot_width", "bskenv_snapshot", "bskenv_restore"]
 
 
 def _shared_signatures(cfg):
@@ -68,7 +69,8 @@ def _shared_signatures(cfg):
             "get_ics": (ci, [vp] * 3), "state_dims": (ci, [vp, C.POINTER(i32), C.POINTER(i32)]),
             "get_state": (ci, [vp] * 4), "set_state": (ci, [vp] * 4), "state_field": (ci, [C.c_char_p, C.POINTER(i32)]),
             "episode_stats": (ci, [vp, vp]), "launch_count": (i64, [vp]), "flops_per_step": (C.c_double, [vp]),
-            "set_ic_pool": (ci, [vp, ci, vp, ci]), "get_ic_rows": (ci, [vp] * 3)}
+            "set_ic_pool": (ci, [vp, ci, vp, ci]), "get_ic_rows": (ci, [vp] * 3),
+            "snapshot_width": (ci, [vp]), "snapshot": (ci, [vp, i64, vp, vp, vp]), "restore": (ci, [vp, i64, vp, vp, vp, vp])}
 
 
 def batch_abi(prefix):

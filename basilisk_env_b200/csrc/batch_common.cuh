@@ -34,7 +34,23 @@ struct BatchCore {
     int ev_valid = 0;
     int64_t launches = 0;
     IcPool icp{};               // loaded initial-condition pool (n_rows = 0: none); rows and per-env record in device memory
+    uint64_t fingerprint = 0;   // of the configuration (snapshot records), set at create
+    unsigned long long *snap_chk = nullptr;     // check words of snapshot / restore (allocated at first use)
+    uint32_t *snap_owner = nullptr;             // [n]: lowest record position naming each env (restore with explicit indices)
     std::string err;
+};
+
+// FNV-1a, 64 bit: the configuration fingerprint of snapshot records, fed field by field (no padding or reserved words)
+struct Fnv64 {
+    uint64_t h = 14695981039346656037ull;
+    template <typename T>
+    void add(const T &v)
+    {
+        const unsigned char *p = reinterpret_cast<const unsigned char *>(&v);
+        for (size_t i = 0; i < sizeof(T); i++) { h ^= p[i]; h *= 1099511628211ull; }
+    }
+    template <typename T, size_t N>
+    void add(const T (&v)[N]) { for (size_t i = 0; i < N; i++) add(v[i]); }
 };
 
 namespace {
@@ -196,6 +212,7 @@ inline void core_free(BatchCore *h)
 {
     cudaFree(h->S); cudaFree(h->I); cudaFree(h->ics); cudaFree(h->stats);
     cudaFree((void *)h->icp.rows); cudaFree(h->icp.row_of); cudaFree(h->icp.row_ep);
+    cudaFree(h->snap_chk); cudaFree(h->snap_owner);
     if (h->own_stream) { cudaStreamSynchronize(h->own_stream); cudaStreamDestroy(h->own_stream); }
     for (void *p : h->h_stage) cudaFreeHost(p);
     if (h->ev_last) cudaEventDestroy(h->ev_last);
@@ -348,6 +365,216 @@ inline void host_step_copy_back(int k, void *const *user, void *const *stage, co
 {
     for (int s = 1; s < k; s++)
         if (user[s] && stage[s]) memcpy(user[s], stage[s], bytes[s]);
+}
+
+// ---- per-env state snapshots (bskenv_snapshot / bskenv_restore and the opNav pair) ----------------------------------------
+// A record is one row of L::W 8-byte words: header (kind << 16 | version, W, fingerprint, source global index), the ND double
+// and NI integer state fields, the DIC stored ICs, the NPD-field parameter block (LEO; PROW = its pool-row field) and the
+// IC-pool row.  EP = the episode counter's field in I.  The kernels move SNAP_ROWS records per block through a shared-memory
+// tile of odd pitch (conflict-free 8-byte accesses both ways): state columns on one side -- one warp reads one field of 32
+// records, coalesced when the envs are consecutive -- and one contiguous run of SNAP_ROWS * W record words on the other.
+template <int KIND_, int ND_, int NI_, int DIC_, int NPD_, int PROW_, int EP_>
+struct SnapLayout {
+    enum : int {
+        KIND = KIND_, ND = ND_, NI = NI_, DIC = DIC_, NPD = NPD_, PROW = PROW_, EP = EP_,
+        OFF_S = 4, OFF_I = OFF_S + ND, OFF_IC = OFF_I + NI, OFF_P = OFF_IC + DIC, OFF_ROW = OFF_P + NPD, W = OFF_ROW + 1,
+        PITCH = W | 1
+    };
+    static constexpr int64_t TAG = (int64_t)KIND << 16 | BSKENV_SNAPSHOT_VERSION;
+};
+#define SNAP_ROWS 32
+#define SNAP_THREADS 256
+
+// What the snapshot kernels address of a handle.  live: the parameter block behind the state fields holds each env's values
+// (a parameter pool is loaded); otherwise a snapshot writes `batch` (SnapBlock) and a restore leaves the block alone.
+struct SnapCols {
+    double *S; int64_t *I; double *ics; int32_t *row_of; int64_t *row_ep;
+    int64_t stride, n, first_env_index; uint64_t fingerprint; int live;
+};
+template <int NPD> struct SnapBlock { double v[NPD > 0 ? NPD : 1]; };
+
+// Word w (>= 0) of env e's record
+template <class L>
+__device__ __forceinline__ double snap_word(const SnapCols &c, const SnapBlock<L::NPD> &batch, int64_t e, int w)
+{
+    const int64_t s = c.stride;
+    if (w < L::OFF_S) {
+        const int64_t v = w == 0 ? L::TAG : (w == 1 ? (int64_t)L::W : (w == 2 ? (int64_t)c.fingerprint : c.first_env_index + e));
+        return __longlong_as_double(v);
+    }
+    if (w < L::OFF_I) return c.S[(int64_t)(w - L::OFF_S) * s + e];
+    if (w < L::OFF_IC) return __longlong_as_double(c.I[(int64_t)(w - L::OFF_I) * s + e]);
+    if (w < L::OFF_P) return c.ics[(int64_t)(w - L::OFF_IC) * s + e];
+    if (w < L::OFF_ROW) return c.live ? c.S[(int64_t)(L::ND + w - L::OFF_P) * s + e] : batch.v[w - L::OFF_P];
+    const int64_t row = (c.row_of && c.row_ep[e] == c.I[(int64_t)L::EP * s + e]) ? (int64_t)c.row_of[e] : -1;
+    return __longlong_as_double(row);
+}
+
+// m records of the envs `envs` (null: envs 0 .. m-1) -> rec [m][W]
+template <class L>
+__global__ void __launch_bounds__(SNAP_THREADS)
+snapshot_gather_kernel(const SnapCols c, const SnapBlock<L::NPD> batch, int64_t m, const int64_t *__restrict__ envs, double *__restrict__ rec)
+{
+    __shared__ double tile[SNAP_ROWS * L::PITCH];
+    const int64_t r0 = (int64_t)blockIdx.x * SNAP_ROWS;
+    const int rows = (int)(m - r0 < SNAP_ROWS ? m - r0 : SNAP_ROWS);
+    for (int t = threadIdx.x; t < SNAP_ROWS * L::W; t += SNAP_THREADS) {     // a warp: one word of 32 records
+        const int r = t % SNAP_ROWS, w = t / SNAP_ROWS;
+        if (r < rows) tile[r * L::PITCH + w] = snap_word<L>(c, batch, envs ? envs[r0 + r] : r0 + r, w);
+    }
+    __syncthreads();
+    double *out = rec + r0 * L::W;
+    for (int t = threadIdx.x; t < rows * L::W; t += SNAP_THREADS) out[t] = tile[(t / L::W) * L::PITCH + t % L::W];
+}
+
+// rec [m][W] -> the envs `envs` (null: 0 .. m-1); obs (may be null) [n][B::OD] = B::obs of each restored env.  B = the batch's
+// snapshot traits: layout L, parameter block type Params, observation dimension OD, obs(P, record row, out).
+template <class B>
+__global__ void __launch_bounds__(SNAP_THREADS)
+restore_scatter_kernel(const __grid_constant__ typename B::Params P, const SnapCols c, int64_t m, const int64_t *__restrict__ envs,
+                       const double *__restrict__ rec, double *__restrict__ obs)
+{
+    using L = typename B::L;
+    __shared__ double tile[SNAP_ROWS * L::PITCH];
+    const int64_t r0 = (int64_t)blockIdx.x * SNAP_ROWS;
+    const int rows = (int)(m - r0 < SNAP_ROWS ? m - r0 : SNAP_ROWS);
+    const double *in = rec + r0 * L::W;
+    for (int t = threadIdx.x; t < rows * L::W; t += SNAP_THREADS) tile[(t / L::W) * L::PITCH + t % L::W] = in[t];
+    __syncthreads();
+    const int64_t s = c.stride;
+    for (int t = threadIdx.x; t < SNAP_ROWS * (L::W - L::OFF_S); t += SNAP_THREADS) {
+        const int r = t % SNAP_ROWS, w = L::OFF_S + t / SNAP_ROWS;
+        if (r >= rows) continue;
+        const int64_t e = envs ? envs[r0 + r] : r0 + r;
+        const double v = tile[r * L::PITCH + w];
+        if (w < L::OFF_I) c.S[(int64_t)(w - L::OFF_S) * s + e] = v;
+        else if (w < L::OFF_IC) c.I[(int64_t)(w - L::OFF_I) * s + e] = __double_as_longlong(v);
+        else if (w < L::OFF_P) c.ics[(int64_t)(w - L::OFF_IC) * s + e] = v;
+        else if (w < L::OFF_ROW) { if (c.live) c.S[(int64_t)(L::ND + w - L::OFF_P) * s + e] = v; }
+        else if (c.row_of) {
+            c.row_of[e] = (int32_t)__double_as_longlong(v);
+            c.row_ep[e] = __double_as_longlong(tile[r * L::PITCH + L::OFF_I + L::EP]);
+        }
+    }
+    if (obs && (int)threadIdx.x < rows) {
+        const int64_t e = envs ? envs[r0 + threadIdx.x] : r0 + threadIdx.x;
+        B::obs(P, tile + threadIdx.x * L::PITCH, obs + e * B::OD);
+    }
+}
+
+// Checks before a restore (rec != null) or a snapshot with explicit indices (rec == null).  chk[0] = the smallest
+// (position << 8 | reason) over offending records, chk[1] = 1 when a record carries an IC-pool row; owner[e] = the lowest
+// position naming env e (snapshot_dup_kernel then flags every later one).
+enum { SNAP_BAD_KIND = 1, SNAP_BAD_WIDTH, SNAP_BAD_FINGERPRINT, SNAP_NO_PARAM_POOL, SNAP_BAD_INDEX, SNAP_DUP_INDEX };
+template <class L>
+__global__ void snapshot_check_kernel(int64_t m, const int64_t *__restrict__ envs, int64_t n, const double *__restrict__ rec,
+                                      uint64_t fingerprint, int live, uint32_t *__restrict__ owner, unsigned long long *__restrict__ chk)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= m) return;
+    int bad = 0;
+    if (rec) {
+        const double *row = rec + i * L::W;
+        if (__double_as_longlong(row[0]) != L::TAG) bad = SNAP_BAD_KIND;
+        else if (__double_as_longlong(row[1]) != (int64_t)L::W) bad = SNAP_BAD_WIDTH;
+        else if ((uint64_t)__double_as_longlong(row[2]) != fingerprint) bad = SNAP_BAD_FINGERPRINT;
+        else if (L::PROW >= 0 && !live && row[L::OFF_P + (L::PROW >= 0 ? L::PROW : 0)] >= 0.0) bad = SNAP_NO_PARAM_POOL;
+        else if (__double_as_longlong(row[L::OFF_ROW]) >= 0) chk[1] = 1ull;
+    }
+    if (!bad && envs) {
+        const int64_t e = envs[i];
+        if (e < 0 || e >= n) bad = SNAP_BAD_INDEX;
+        else if (owner) atomicMin(&owner[e], (uint32_t)i);
+    }
+    if (bad) atomicMin(&chk[0], (unsigned long long)i << 8 | (unsigned long long)bad);
+}
+__global__ void snapshot_dup_kernel(int64_t m, const int64_t *__restrict__ envs, int64_t n, const uint32_t *__restrict__ owner,
+                                    unsigned long long *__restrict__ chk)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= m) return;
+    const int64_t e = envs[i];
+    if (e >= 0 && e < n && owner[e] < (uint32_t)i) atomicMin(&chk[0], (unsigned long long)i << 8 | SNAP_DUP_INDEX);
+}
+
+// Runs the checks on `st`, reads the check words back and waits for the stream.  *rows_needed: a record carries an IC-pool row.
+template <class L>
+int snapshot_checks(BatchCore *h, const char *what, int64_t m, const int64_t *envs, const double *rec, int live, cudaStream_t st,
+                    bool *rows_needed)
+{
+    if (!h->snap_chk) CU_TRY(h, cudaMalloc(&h->snap_chk, 2 * sizeof(unsigned long long)));
+    const bool dup = rec && envs;
+    if (dup && !h->snap_owner) CU_TRY(h, cudaMalloc(&h->snap_owner, sizeof(uint32_t) * h->stride));
+    CU_TRY(h, cudaMemsetAsync(h->snap_chk, 0xFF, sizeof(unsigned long long), st));
+    CU_TRY(h, cudaMemsetAsync(h->snap_chk + 1, 0, sizeof(unsigned long long), st));
+    if (dup) CU_TRY(h, cudaMemsetAsync(h->snap_owner, 0xFF, sizeof(uint32_t) * h->n, st));
+    const int grid = (int)((m + 255) / 256);
+    snapshot_check_kernel<L><<<grid, 256, 0, st>>>(m, envs, h->n, rec, h->fingerprint, live, dup ? h->snap_owner : nullptr, h->snap_chk);
+    if (dup) snapshot_dup_kernel<<<grid, 256, 0, st>>>(m, envs, h->n, h->snap_owner, h->snap_chk);
+    CU_TRY(h, cudaGetLastError());
+    unsigned long long w[2];
+    CU_TRY(h, cudaMemcpyAsync(w, h->snap_chk, sizeof(w), cudaMemcpyDeviceToHost, st));
+    CU_TRY(h, cudaStreamSynchronize(st));
+    if (w[0] != ~0ull) {
+        static const char *why[] = {"", "not a record of this batch kind and format version", "record width differs",
+                                    "configuration fingerprint differs from this handle's", "carries a parameter-pool row and no parameter pool is loaded",
+                                    "env index outside [0, n)", "env index named twice"};
+        h->err = std::string(what) + ": record " + std::to_string(w[0] >> 8) + ": " + why[w[0] & 0xFF];
+        return BSKENV_EINVAL;
+    }
+    *rows_needed = w[1] != 0;
+    return BSKENV_OK;
+}
+
+inline int snapshot_args(BatchCore *h, const char *what, int64_t m, const int64_t *envs, const void *rec)
+{
+    if (!rec || m < 1 || (!envs && m != h->n)) {
+        h->err = std::string(what) + ": null records, m < 1, or no env indices and m != n";
+        return BSKENV_EINVAL;
+    }
+    return BSKENV_OK;
+}
+
+// bskenv_snapshot / bskenv_opnav_snapshot: c = the handle's columns (row_of / row_ep included), batch = the parameter block of
+// the configuration (LEO, written where c.live is 0)
+template <class L>
+int snapshot(BatchCore *h, const char *what, int64_t m, const int64_t *envs, double *rec, const SnapCols &c,
+             const SnapBlock<L::NPD> &batch, void *stream)
+{
+    int rc = snapshot_args(h, what, m, envs, rec);
+    if (rc) return rc;
+    CU_TRY(h, cudaSetDevice(h->device));
+    const cudaStream_t st = (cudaStream_t)stream;
+    bool unused;
+    if (envs && (rc = snapshot_checks<L>(h, what, m, envs, nullptr, c.live, st, &unused))) return rc;
+    snapshot_gather_kernel<L><<<(int)((m + SNAP_ROWS - 1) / SNAP_ROWS), SNAP_THREADS, 0, st>>>(c, batch, m, envs, rec);
+    CU_TRY(h, cudaGetLastError());
+    return BSKENV_OK;
+}
+
+// bskenv_restore / bskenv_opnav_restore: checks, then (the IC-pool record allocated at the first record that carries a row,
+// as set_ic_pool does) the scatter
+template <class B>
+int restore(BatchCore *h, const char *what, int64_t m, const int64_t *envs, const double *rec, double *obs, SnapCols c,
+            const typename B::Params &P, void *stream)
+{
+    int rc = snapshot_args(h, what, m, envs, rec);
+    if (rc) return rc;
+    CU_TRY(h, cudaSetDevice(h->device));
+    const cudaStream_t st = (cudaStream_t)stream;
+    bool rows_needed = false;
+    if ((rc = snapshot_checks<typename B::L>(h, what, m, envs, rec, c.live, st, &rows_needed))) return rc;
+    if (rows_needed && !h->icp.row_of) {
+        CU_TRY(h, cudaMalloc(&h->icp.row_of, sizeof(int32_t) * h->stride));
+        CU_TRY(h, cudaMalloc(&h->icp.row_ep, sizeof(int64_t) * h->stride));
+        CU_TRY(h, cudaMemsetAsync(h->icp.row_of, 0xFF, sizeof(int32_t) * h->stride, st));
+        CU_TRY(h, cudaMemsetAsync(h->icp.row_ep, 0, sizeof(int64_t) * h->stride, st));
+    }
+    c.row_of = h->icp.row_of; c.row_ep = h->icp.row_ep;
+    restore_scatter_kernel<B><<<(int)((m + SNAP_ROWS - 1) / SNAP_ROWS), SNAP_THREADS, 0, st>>>(P, c, m, envs, rec, obs);
+    CU_TRY(h, cudaGetLastError());
+    CU_TRY(h, note_launch(h, st));
+    return BSKENV_OK;
 }
 
 // bskenv_state_field / bskenv_opnav_state_field: the index of a named field in the batch's table (-1: none), is_int = which block

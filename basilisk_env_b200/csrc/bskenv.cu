@@ -11,8 +11,9 @@
 //   leo_reset_kernel  simulator construction + initial observation (reference ...Simulator.py:67-117,
 //                     ...Environment.py:172-216) from explicit, stored or device-sampled ICs.
 //   fp64_peak_kernel  DFMA microbenchmark = the roofline denominator.
-// The lane bucketing before a step (bucket_count_kernel + bucket_fill_kernel) is shared with the opNav batch
-// (batch_common.cuh).  There is no CPU path in this library.
+// The lane bucketing before a step (bucket_count_kernel + bucket_fill_kernel) and the per-env state snapshot kernels
+// (snapshot_gather_kernel, restore_scatter_kernel and their checks) are shared with the opNav batch (batch_common.cuh).
+// There is no CPU path in this library.
 #include <cuda_runtime.h>
 #include <stdlib.h>
 #include <string.h>
@@ -340,6 +341,45 @@ __global__ void gather_params_kernel(const double *__restrict__ S, int64_t strid
     if (row) row[e] = live ? (int32_t)S[(int64_t)(LEO_ND + PE_ROW) * stride + e] : -1;
 }
 
+// Snapshot records of the LEO batch (batch_common.cuh: SnapLayout; include/bskenv.h: BSKENV_SNAP_*).  The observation of a
+// restored env is the one its source returned last: the reset's initial observation of the stored ICs while curr_step is 0
+// (fresh from a reset or an auto-reset), else the last simulator observation F_OBS normalised as at the end of leo_step_env.
+struct LeoSnap {
+    using L = SnapLayout<BSKENV_SNAPSHOT_KIND_LEO, LEO_ND, LEO_NI, BSKENV_IC_DIM, LEO_NPD, PE_ROW, I_EPISODE>;
+    using Params = LeoParams;
+    enum : int { OD = BSKENV_OBS_DIM };
+    __device__ static void obs(const LeoParams &P, const double *row, double *ob)
+    {
+        if (__double_as_longlong(row[L::OFF_I + I_STEP]) == 0) {
+            double ic[19];
+            for (int k = 0; k < 19; k++) ic[k] = row[L::OFF_IC + k];
+            leo::reset_obs(P, ic, leo::ic_w4(ic), ob);
+        } else {
+            const double *f = row + L::OFF_S + F_OBS;
+            ob[0] = f[0]; ob[1] = f[1]; ob[2] = f[2] / P.wheel_limit; ob[3] = f[3] / P.power_max; ob[4] = f[4];
+        }
+    }
+};
+static_assert(LeoSnap::L::OFF_S == BSKENV_SNAP_S && LeoSnap::L::OFF_I == BSKENV_SNAP_I && LeoSnap::L::OFF_IC == BSKENV_SNAP_ICS &&
+              LeoSnap::L::OFF_P == BSKENV_SNAP_PARAMS && LeoSnap::L::OFF_ROW == BSKENV_SNAP_ICROW && LeoSnap::L::W == BSKENV_SNAPSHOT_W,
+              "include/bskenv.h: the LEO record layout");
+
+// The configuration fingerprint of snapshot records: the named fields of bskenv_config except the reserved words and
+// auto_reset (handle policy)
+static uint64_t leo_fingerprint(const bskenv_config &c)
+{
+    Fnv64 f;
+    f.add(c.abi_version); f.add(c.dynRate); f.add(c.fswRate); f.add(c.step_duration);
+    f.add(c.mass); f.add(c.width); f.add(c.depth); f.add(c.height);
+    f.add(c.planetRadius); f.add(c.baseDensity); f.add(c.scaleHeight); f.add(c.disturbance_magnitude);
+    f.add(c.nHat_B); f.add(c.panelArea); f.add(c.panelEfficiency); f.add(c.powerDraw); f.add(c.storageCapacity);
+    f.add(c.sigma_R0N); f.add(c.K); f.add(c.Ki); f.add(c.P); f.add(c.hs_min); f.add(c.thrMinFireTime);
+    f.add(c.thrForceSign); f.add(c.maxCounterValue); f.add(c.max_length);
+    f.add(c.wheel_limit_rpm); f.add(c.power_max); f.add(c.failure_penalty);
+    f.add(c.use_j2); f.add(c.hill_cel_pun); f.add(c.rw_set); f.add(c.precision);
+    return f.h;
+}
+
 // 8 independent DFMA chains per thread, everything in registers
 __global__ void __launch_bounds__(256) fp64_peak_kernel(double *out, int iters, double a, double b)
 {
@@ -534,6 +574,7 @@ int bskenv_create(const bskenv_config *cfg, int device, int64_t n_envs, int64_t 
     }
     leo_host::build_params_f(h->P, h->PF);
     h->P.first_env_index = first_env_index;
+    h->fingerprint = leo_fingerprint(*cfg);
     h->s_fields = LEO_ND;       // (the handle is zero-initialised: no pools, BSKENV_ORG_AUTO)
     cudaError_t e = core_alloc(h, device, n_envs, LEO_ND, LEO_NI, 19, ST_N);
     if (e == cudaSuccess) e = cudaMalloc(&h->sched, sizeof(int) * (size_t)(4 + (n_envs + 31) / 32));
@@ -782,6 +823,35 @@ int bskenv_set_state(bskenv_handle *h, const double *dstate_dev, const int64_t *
 {
     return h ? set_state(h, LEO_ND, LEO_NI, dstate_dev, istate_dev, stream) : BSKENV_EINVAL;
 }
+// ---- per-env state snapshots (batch_common.cuh: snapshot / restore) ----
+static SnapCols leo_snap_cols(bskenv_handle *h)
+{
+    // the parameter block holds the envs' values only while a pool is loaded (as bskenv_get_env_params reads it); a pool
+    // once loaded and unloaded leaves it allocated and stale
+    return SnapCols{h->S, h->I, h->ics, h->icp.row_of, h->icp.row_ep, h->stride, h->n, h->P.first_env_index, h->fingerprint,
+                    h->pool.n_rows > 0 ? 1 : 0};
+}
+int bskenv_snapshot_width(const bskenv_handle *h)
+{
+    (void)h;
+    return BSKENV_SNAPSHOT_W;
+}
+int bskenv_snapshot(bskenv_handle *h, int64_t m, const int64_t *envs_dev, double *rec_dev, void *stream)
+{
+    if (!h) return BSKENV_EINVAL;
+    SnapBlock<LEO_NPD> batch;   // the parameter block of the configuration itself, pool row -1 (as bskenv_set_param_pool derives it)
+    double raw[BSKENV_PARAM_DIM];
+    leo_host::param_row_get(h->cfg, raw);
+    leo_host::param_row_derive(h->P, raw, -1.0, batch.v);
+    return snapshot<LeoSnap::L>(h, "bskenv_snapshot", m, envs_dev, rec_dev, leo_snap_cols(h), batch, stream);
+}
+int bskenv_restore(bskenv_handle *h, int64_t m, const int64_t *envs_dev, const double *rec_dev, double *obs_dev, void *stream)
+{
+    if (!h) return BSKENV_EINVAL;
+    NO_HOST_PENDING(h, "bskenv_restore");
+    return restore<LeoSnap>(h, "bskenv_restore", m, envs_dev, rec_dev, obs_dev, leo_snap_cols(h), h->P, stream);
+}
+
 int bskenv_state_field(const char *name, int32_t *is_int)
 {
     static const FieldEnt tab[] = {

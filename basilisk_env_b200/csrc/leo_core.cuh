@@ -776,6 +776,20 @@ LEO_HD_NOINLINE void sample_ic(const LeoParams &P, int64_t global_env, int64_t e
 // reset: LEOPowerAttitudeSimulator.__init__ (SIM:67-117) + InitializeSimulationAndDiscover, and the
 // initial observation of leoPowerAttEnv.reset (ENV:188-190)
 // ------------------------------------------------------------------------------------------------
+// rw_set 1: the fourth wheel starts at the mean speed of the three sampled ones [RPM]
+LEO_HD double ic_w4(const double (&ic)[19]) { return (ic[15] + ic[16] + ic[17]) / 3.0; }
+// The initial observation of a reset from its ICs (w4 = ic_w4(ic), taken by the caller before it writes the state: the
+// stores may alias `ic` for all the compiler knows): SIM:347-351 (wheel speeds in RPM, un-converted: SIM:306) then
+// ENV:189-190.  Also what bskenv_restore returns for an env fresh from a reset.
+LEO_HD void reset_obs(const LeoParams &P, const double (&ic)[19], double w4, double *obs)
+{
+    obs[0] = sqrt(ic[6] * ic[6] + ic[7] * ic[7] + ic[8] * ic[8]);
+    obs[1] = sqrt(ic[9] * ic[9] + ic[10] * ic[10] + ic[11] * ic[11]);
+    obs[2] = sqrt(ic[15] * ic[15] + ic[16] * ic[16] + ic[17] * ic[17] + (P.nrw == 4 ? w4 * w4 : 0.0)) / P.wheel_limit;
+    obs[3] = ic[18] / 3600.0 / P.power_max;
+    obs[4] = 0.0;
+}
+
 template <class PA = ParBatch>
 LEO_HD void leo_reset_env(const LeoParams &P, double *S, int64_t *I, int64_t stride, int64_t e, const double (&ic)[19],
                           double *obs /* 5, may be null */)
@@ -790,19 +804,13 @@ LEO_HD void leo_reset_env(const LeoParams &P, double *S, int64_t *I, int64_t str
     const double dist_mag = PA::dist_mag(P, S, stride, e);
     for (int k = 0; k < 3; k++) SD(F_LDIST + k) = dist_mag * ic[12 + k];               // SIM:295 (quirk Q4: raw vector)
     for (int k = 0; k < 3; k++) SD(F_WHL + k) = ic[15 + k] * P.wheel_rpm2rad;       // SIM:303-305
-    const double w4 = (ic[15] + ic[16] + ic[17]) / 3.0;                              // rw_set 1: fourth wheel at the mean speed
+    const double w4 = ic_w4(ic);
     if (P.nrw == 4) SD(F_WHL + 3) = w4 * P.wheel_rpm2rad;
     SD(F_E) = ic[18];
     SI(I_TICK) = -1;
     SI(I_MASK) = LEO_TASK_ALL;       // every task starts enabled
     SI(I_INITREQ) = 1;               // Reset_thrMomentumManagement
-    if (obs) { // SIM:347-351 (wheel speeds in RPM, un-converted: SIM:306) then ENV:189-190
-        obs[0] = sqrt(ic[6] * ic[6] + ic[7] * ic[7] + ic[8] * ic[8]);
-        obs[1] = sqrt(ic[9] * ic[9] + ic[10] * ic[10] + ic[11] * ic[11]);
-        obs[2] = sqrt(ic[15] * ic[15] + ic[16] * ic[16] + ic[17] * ic[17] + (P.nrw == 4 ? w4 * w4 : 0.0)) / P.wheel_limit;
-        obs[3] = ic[18] / 3600.0 / P.power_max;
-        obs[4] = 0.0;
-    }
+    if (obs) reset_obs(P, ic, w4, obs);
 #undef SD
 #undef SI
 }

@@ -10,8 +10,9 @@
 //   opnav_noise_kernel, opnav_dyn_kernel
 //                       the opt-in three-kernel form of the first pass: the noise walk of the interval, then the rest.
 //   opnav_reset_kernel  simulator construction + initial observation from explicit, stored or device-sampled ICs.
-// The lane bucketing before a step (bucket_count_kernel + bucket_fill_kernel) is shared with the LEO batch
-// (batch_common.cuh).  There is no CPU path in this library.
+// The lane bucketing before a step (bucket_count_kernel + bucket_fill_kernel) and the per-env state snapshot kernels
+// (snapshot_gather_kernel, restore_scatter_kernel and their checks) are shared with the LEO batch (batch_common.cuh).
+// There is no CPU path in this library.
 #include <cuda_runtime.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -261,6 +262,33 @@ opnav_reset_kernel(const __grid_constant__ OpNavParams P, double *__restrict__ S
         for (int k = 0; k < 4; k++) obs[e * 4 + k] = ob[k];
 }
 
+// Snapshot records of the opNav batch (batch_common.cuh: SnapLayout; include/bskenv.h: BSKENV_OPNAV_SNAP_*): no parameter
+// block.  The observation of a restored env is OF_OBS, where the second pass stores the observation it returns and
+// opnav_reset_env leaves zeros, the initial observation (ONS:152).
+struct OpNavSnap {
+    using L = SnapLayout<BSKENV_SNAPSHOT_KIND_OPNAV, OPNAV_ND, OPNAV_NI, OPNAV_IC_DIM, 0, -1, OI_EPISODE>;
+    using Params = OpNavParams;
+    enum : int { OD = BSKENV_OPNAV_OBS_DIM };
+    __device__ static void obs(const OpNavParams &, const double *row, double *ob)
+    {
+        for (int k = 0; k < OD; k++) ob[k] = row[L::OFF_S + OF_OBS + k];
+    }
+};
+static_assert(OpNavSnap::L::OFF_S == BSKENV_OPNAV_SNAP_S && OpNavSnap::L::OFF_I == BSKENV_OPNAV_SNAP_I &&
+              OpNavSnap::L::OFF_IC == BSKENV_OPNAV_SNAP_ICS && OpNavSnap::L::OFF_ROW == BSKENV_OPNAV_SNAP_ICROW &&
+              OpNavSnap::L::W == BSKENV_OPNAV_SNAPSHOT_W, "include/bskenv.h: the opNav record layout");
+
+// The configuration fingerprint of snapshot records: the named fields of bskenv_opnav_config except the reserved words,
+// auto_reset and noise_seed (handle policy)
+static uint64_t opnav_fingerprint(const bskenv_opnav_config &c)
+{
+    Fnv64 f;
+    f.add(c.abi_version); f.add(c.dynRate); f.add(c.fswRate); f.add(c.step_duration_min);
+    f.add(c.max_length); f.add(c.numModes); f.add(c.nav_noise); f.add(c.camera_reenable); f.add(c.sample_orbit);
+    f.add(c.pixel_noise_std); f.add(c.circle_unc); f.add(c.reward_mult);
+    return f.h;
+}
+
 thread_local std::string g_opnav_create_error;
 
 }  // namespace
@@ -378,6 +406,7 @@ int bskenv_opnav_create(const bskenv_opnav_config *cfg, int device, int64_t n_en
     std::string perr = opnav_host::build_params(*cfg, h->P);
     if (!perr.empty()) { g_opnav_create_error = "bskenv_opnav_create: " + perr; delete h; return BSKENV_EINVAL; }
     h->P.first_env_index = first_env_index;
+    h->fingerprint = opnav_fingerprint(*cfg);
     h->noise_split = -1;        // (the handle is zero-initialised)
     cudaError_t e = core_alloc(h, device, n_envs, OPNAV_ND, OPNAV_NI, OPNAV_IC_DIM, OST_N);
     if (e == cudaSuccess) e = cudaMalloc(&h->sched, sizeof(int) * 8);
@@ -515,6 +544,27 @@ int bskenv_opnav_set_state(bskenv_opnav_handle *h, const double *dstate_dev, con
 {
     return h ? set_state(h, OPNAV_ND, OPNAV_NI, dstate_dev, istate_dev, stream) : BSKENV_EINVAL;
 }
+// ---- per-env state snapshots (batch_common.cuh: snapshot / restore) ----
+static SnapCols opnav_snap_cols(bskenv_opnav_handle *h)
+{
+    return SnapCols{h->S, h->I, h->ics, h->icp.row_of, h->icp.row_ep, h->stride, h->n, h->P.first_env_index, h->fingerprint, 0};
+}
+int bskenv_opnav_snapshot_width(const bskenv_opnav_handle *h)
+{
+    (void)h;
+    return BSKENV_OPNAV_SNAPSHOT_W;
+}
+int bskenv_opnav_snapshot(bskenv_opnav_handle *h, int64_t m, const int64_t *envs_dev, double *rec_dev, void *stream)
+{
+    return h ? snapshot<OpNavSnap::L>(h, "bskenv_opnav_snapshot", m, envs_dev, rec_dev, opnav_snap_cols(h), SnapBlock<0>{}, stream)
+             : BSKENV_EINVAL;
+}
+int bskenv_opnav_restore(bskenv_opnav_handle *h, int64_t m, const int64_t *envs_dev, const double *rec_dev, double *obs_dev, void *stream)
+{
+    return h ? restore<OpNavSnap>(h, "bskenv_opnav_restore", m, envs_dev, rec_dev, obs_dev, opnav_snap_cols(h), h->P, stream)
+             : BSKENV_EINVAL;
+}
+
 int bskenv_opnav_state_field(const char *name, int32_t *is_int)
 {
     static const FieldEnt tab[] = {

@@ -185,6 +185,36 @@ class BatchVecEnv:
         self._call(self._f.set_state, self._h, C.c_void_p(d.data_ptr()), C.c_void_p(i.data_ptr()), self._stream())
         torch.cuda.current_stream(self.device).synchronize()
 
+    def _env_index(self, envs):
+        if envs is None:
+            return None, None
+        idx = torch.as_tensor(envs).to(device=self.device, dtype=torch.int64).reshape(-1).contiguous()
+        return idx, C.c_void_p(idx.data_ptr())
+
+    def snapshot(self, envs=None):
+        """Per-env state records (include/bskenv.h: bskenv_snapshot): float64 [m, W] on this handle's device, one row per env
+        of `envs` (indices, None = every env in index order).  A record holds everything a step or a reset reads of its env and
+        can be restored into any env of any handle with the same configuration (`restore`)."""
+        idx, ip = self._env_index(envs)
+        m = self.num_envs if idx is None else idx.numel()
+        rec = torch.empty((m, int(self._f.snapshot_width(self._h))), dtype=torch.float64, device=self.device)
+        self._call(self._f.snapshot, self._h, m, ip, C.c_void_p(rec.data_ptr()), self._stream())
+        self._snap_keep = idx           # keep alive until the gather has consumed it
+        return rec
+
+    def restore(self, records, envs=None):
+        """Write records [m, W] (from `snapshot` of this or another handle; `.to(self.device)` moves them) into the envs `envs`
+        (indices, None = every env in index order) and return `obs`, in which each restored env's row is the observation its
+        source returned last.  Waits for the current stream (the records are checked on the device first)."""
+        idx, ip = self._env_index(envs)
+        r = records.to(device=self.device, dtype=torch.float64).contiguous()
+        m = self.num_envs if idx is None else idx.numel()
+        if tuple(r.shape) != (m, int(self._f.snapshot_width(self._h))):
+            raise ValueError(f"records must have shape ({m}, {int(self._f.snapshot_width(self._h))})")
+        self._call(self._f.restore, self._h, m, ip, C.c_void_p(r.data_ptr()), C.c_void_p(self.obs.data_ptr()), self._stream())
+        self._snap_keep = (r, idx)      # keep alive until the scatter has consumed them
+        return self.obs
+
     def field(self, name, state=None):
         """Named slice of the state, e.g. field("r_BN_N") -> [3, N]."""
         idx, is_int = _native.batch_state_field(self._abi, name)

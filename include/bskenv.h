@@ -165,7 +165,7 @@ int bskenv_get_env_params(bskenv_handle *h, double *params_dev /* [n][14] */, in
  * bskenv_set_param_pool with another row count or an unload.  Refused while a host-buffer step is in flight.
  * bskenv_get_ic_rows: the pool row each env's current episode started from (int32[n], device memory); -1 = sampled or
  * explicit ICs, or a reset before the pool was loaded.  The row is not part of the state (bskenv_state_dims, get_state /
- * set_state): a checkpoint does not carry it. */
+ * set_state): a checkpoint does not carry it; a snapshot record (bskenv_snapshot) does. */
 #define BSKENV_ICS_BY_INDEX 0
 #define BSKENV_ICS_PER_EPISODE 1
 #define BSKENV_ICS_PARAM_ROW 2
@@ -233,6 +233,67 @@ int bskenv_set_state(bskenv_handle *h, const double *dstate_dev, const int64_t *
 /* index of a named state field (e.g. "r_BN_N", "sigma_BN", "Omega", "storedCharge"); -1 if unknown.
  * `is_int` receives 1 for int64 fields. */
 int bskenv_state_field(const char *name, int32_t *is_int);
+
+/* Per-env state snapshots (branching, restarts from mid-episode states, moving envs between shards or GPUs, checkpoints
+ * that survive parameter and IC pools).  A RECORD is everything a step or a reset reads of one env, as one row of W 8-byte
+ * words; records are row-major [m][W] in device memory.  Integer words are bit-cast into the double words (memcpy).
+ *   words                    content
+ *   0                        (int64) kind << 16 | format version: BSKENV_SNAPSHOT_KIND_LEO / _OPNAV, BSKENV_SNAPSHOT_VERSION
+ *   1                        (int64) W
+ *   2                        (uint64) fingerprint of the handle's configuration: a 64-bit FNV-1a hash of the named fields of
+ *                            bskenv_config (bskenv_opnav_config) in declaration order, without the reserved words, auto_reset
+ *                            and (opNav) noise_seed, which are handle policy rather than the meaning of the state
+ *   3                        (int64) global index of the source env (information only)
+ *   BSKENV_SNAP_S ..         the LEO_ND = 89 double state fields (bskenv_get_state's first block)
+ *   BSKENV_SNAP_I ..         the LEO_NI = 22 int64 state fields (its second block)
+ *   BSKENV_SNAP_ICS ..       the 19 stored initial conditions (bskenv_get_ics; what bskenv_reset_init replays)
+ *   BSKENV_SNAP_PARAMS ..    the 37 derived values of the env's spacecraft parameters (bskenv_set_param_pool), the pool row
+ *                            among them (word BSKENV_SNAP_PARAMS + 22, -1 = the batch configuration).  Without a loaded
+ *                            parameter pool the block this configuration derives for itself, row -1.
+ *   BSKENV_SNAP_ICROW        (int64) the IC-pool row of the current episode, as bskenv_get_ic_rows reports it (-1 = none)
+ * opNav: header, 83 double and 14 int64 state fields, 12 stored ICs, IC-pool row (BSKENV_OPNAV_SNAP_*); no parameter block.
+ *
+ * bskenv_snapshot_width: W, a constant of the batch kind (h is not read).  bskenv_snapshot: the records of m envs, envs_dev =
+ * their indices (int64[m], device memory) or NULL for the whole batch in index order (m == n).  bskenv_restore: writes m
+ * records into the envs named by envs_dev (NULL: the whole batch, m == n) -- state, stored ICs, parameter block (where a pool
+ * is loaded: the record's, which is the batch block for a row -1 record) and IC-pool row -- and, when obs_dev is given
+ * (double[n][5], opNav [n][4]), the observation of each restored env: the one its source returned last (for an env fresh
+ * from a reset or an auto-reset, the initial observation of its stored ICs).  Episode statistics are not touched.
+ * Handle settings are not part of a record, and a restore may cross them: force-model upgrades (bskenv_set_gravity_degree2),
+ * ephemeris tables, the organisation, the loaded pools themselves, first_env_index and the seed.
+ *
+ * A record is an env's state, not its random-stream identity: a restored LEO env's next reset draws from the DESTINATION's
+ * (seed, global env index, episode), with the episode counter from the record; a restored opNav env's sensor noise continues
+ * under the destination's (noise_seed, global env index, episode).  So a restore into the same global index of a handle with
+ * the same seed reproduces the source bit for bit, through auto-resets too; a LEO restore into another index reproduces it
+ * until that env's next reset; an opNav restore into another index does so only with the noise off (nav_noise = 0,
+ * pixel_noise_std = 0).
+ *
+ * Both calls check their indices, and restore its records, in a device kernel before anything is written, then read one
+ * check word back and SYNCHRONISE THE CALLER'S STREAM (snapshot only with explicit indices).  BSKENV_EINVAL, with nothing
+ * written and bskenv_last_error naming the first offending record position, for: a record of another batch kind, format
+ * version or width; another fingerprint; an index outside [0, n); an index named twice (restore); a LEO record with a pool
+ * row >= 0 for a handle without a loaded parameter pool; a null pointer where one is required, m < 1, or envs_dev = NULL
+ * with m != n; and (LEO) a host-buffer step in flight. */
+#define BSKENV_SNAPSHOT_VERSION 1
+#define BSKENV_SNAPSHOT_KIND_LEO 1
+#define BSKENV_SNAPSHOT_KIND_OPNAV 2
+#define BSKENV_SNAP_S 4
+#define BSKENV_SNAP_I 93
+#define BSKENV_SNAP_ICS 115
+#define BSKENV_SNAP_PARAMS 134
+#define BSKENV_SNAP_ICROW 171
+#define BSKENV_SNAPSHOT_W 172
+#define BSKENV_OPNAV_SNAP_S 4
+#define BSKENV_OPNAV_SNAP_I 87
+#define BSKENV_OPNAV_SNAP_ICS 101
+#define BSKENV_OPNAV_SNAP_ICROW 113
+#define BSKENV_OPNAV_SNAPSHOT_W 114
+int bskenv_snapshot_width(const bskenv_handle *h);
+int bskenv_snapshot(bskenv_handle *h, int64_t m, const int64_t *envs_dev /* [m] or NULL */, double *rec_dev /* [m][W] */,
+                    void *stream);
+int bskenv_restore(bskenv_handle *h, int64_t m, const int64_t *envs_dev /* [m] or NULL */, const double *rec_dev /* [m][W] */,
+                   double *obs_dev /* [n][5] or NULL */, void *stream);
 
 /* Episode statistics of this shard since the last call (sum of returns, sum of lengths, episodes
  * finished, finished by wheel / power / decay / max-length): int64/double[8] in `stats_host`.
@@ -354,6 +415,13 @@ int bskenv_opnav_state_dims(const bskenv_opnav_handle *h, int32_t *n_double_fiel
 int bskenv_opnav_get_state(bskenv_opnav_handle *h, double *dstate_dev, int64_t *istate_dev, void *stream);
 int bskenv_opnav_set_state(bskenv_opnav_handle *h, const double *dstate_dev, const int64_t *istate_dev, void *stream);
 int bskenv_opnav_state_field(const char *name, int32_t *is_int);
+/* Per-env state snapshots of the opNav batch: record layout, semantics and refusals as bskenv_snapshot / bskenv_restore
+ * (W = BSKENV_OPNAV_SNAPSHOT_W, obs_dev double[n][4]: the last observation, zeros for an env fresh from a reset). */
+int bskenv_opnav_snapshot_width(const bskenv_opnav_handle *h);
+int bskenv_opnav_snapshot(bskenv_opnav_handle *h, int64_t m, const int64_t *envs_dev /* [m] or NULL */,
+                          double *rec_dev /* [m][W] */, void *stream);
+int bskenv_opnav_restore(bskenv_opnav_handle *h, int64_t m, const int64_t *envs_dev /* [m] or NULL */,
+                         const double *rec_dev /* [m][W] */, double *obs_dev /* [n][4] or NULL */, void *stream);
 /* [sum of returns, sum of lengths, episodes finished, by max_length, by numModes, env-steps, measurement updates,
  *  rejected filter updates] since the last call */
 int bskenv_opnav_episode_stats(bskenv_opnav_handle *h, double *stats_host);
